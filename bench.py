@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the PG-MORL hot path (BASELINE.json metric: MOPG env-steps/s; configs[1]).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config c2|...]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config c2|...] [--dump-outputs DIR]
 
 One "step" = one MOPG iteration of the population shard on one batch of synthetic trajectories: rollout inference
 (K1) + vector GAE / advantage (K2) + PPO update of E epochs x B minibatches with Adam (K3). Every GEN_ITERS-th step
@@ -35,6 +35,7 @@ import subprocess
 import sys
 import threading
 import time
+import zlib
 
 import numpy as np
 
@@ -518,6 +519,24 @@ def measured_traffic(kernel):
     return e["dram_bytes"], e.get("csv")
 
 
+DUMP_BYTES = 60 << 20       # data of all dumped arrays together; with the .npy headers the directory stays under 64 MB
+
+
+def dump_outputs(out_dir, arrays):
+    """Write `arrays` (name -> numpy array) as out_dir/<name>.npy in float32 / float64. When they hold more than DUMP_BYTES,
+    every array is cut to the same fraction of its elements: a flat sample at sorted indices drawn from a generator seeded
+    by the array's name, so that two runs with the same arguments write the same sample."""
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {k: a if a.dtype in (np.float32, np.float64) else a.astype(np.float64) for k, a in arrays.items()}
+    frac = min(1.0, DUMP_BYTES / sum(a.nbytes for a in arrays.values()))
+    for name, a in arrays.items():
+        if frac < 1.0:
+            flat = a.reshape(-1)
+            rng = np.random.default_rng(zlib.crc32(name.encode()))
+            a = flat[np.sort(rng.choice(flat.size, int(flat.size * frac), replace=False))]
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -532,7 +551,13 @@ def main():
     ap.add_argument("--no-boundary", action="store_true", help="leave the generation boundary out of the timed loops")
     ap.add_argument("--quarter-sample", action="store_true",
                     help="reference arm: T/4 steps per iteration (same minibatch size) instead of the full-size iteration")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one computed for rank 0's tasks (updated policies and "
+                         "Adam state, rollout values / actions / log-probs, returns, advantages, losses, task weights) as "
+                         "DIR/<name>.npy, at most 64 MB in all (a fixed seeded sample of larger outputs)")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
     if args.impl == "reference":
         # CPU-only arm: hide the GPUs before torch is imported (fork-based worker pools cannot follow the CUDA
         # autograd threads torch starts when a device is visible)
@@ -702,6 +727,10 @@ def main():
     t1 = time.perf_counter()
     clk = clocks.stop(t0, t1)
     bnd_timed = list(bnd_log)
+    if args.dump_outputs and rank == 0:
+        # taken here: the generation and stage-time runs below move the population state on
+        dump_outputs(args.dump_outputs, {k: getattr(pop, k).cpu().numpy() for k in (
+            "params", "adam_m", "adam_v", "adam_step", "value", "action", "logp", "returns", "adv", "losses", "weights")})
     # one whole generation as a unit: GEN_ITERS e2e steps + the boundary, wall clock (skipped steps never happen: the
     # boundary fires on the last of the GEN_ITERS steps)
     gen = None

@@ -99,15 +99,17 @@ def _fake_mopg(args, task_batch, device, iteration, num_updates, start_time=None
     return out
 
 
-def _run(save_dir, method):
-    morl.initialize_warm_up_batch = _fake_warm_up
-    morl.mopg_population_update = _fake_mopg
+def _run(save_dir, method, patch=setattr):
+    """`patch` installs the stand-ins; the test's own process passes monkeypatch.setattr so that the real device stages
+    are back for the tests that run after it."""
+    patch(morl, "initialize_warm_up_batch", _fake_warm_up)
+    patch(morl, "mopg_population_update", _fake_mopg)
     if not torch.cuda.is_available():
         # no CPU fallback exists in the product: the archive's dominance filter is K5. On a machine without a GPU this
         # test (host protocol only) lets the ORACLE stand in for that one kernel.
         from oracle import selection_oracle as so
         from pgmorl_b200 import ep as ep_mod
-        ep_mod.get_ep_indices = lambda objs: list(so.get_ep_indices(np.asarray(objs, dtype=np.float64)))
+        patch(ep_mod, "get_ep_indices", lambda objs: list(so.get_ep_indices(np.asarray(objs, dtype=np.float64))))
     return morl.run(_args(save_dir, method), device="cpu")
 
 
@@ -148,13 +150,13 @@ import pytest
 
 
 @pytest.mark.parametrize("method", ["prediction-guided", "moead", "ra", "random"])
-def test_sharded_run_equals_single_process_run(tmp_path, method):
+def test_sharded_run_equals_single_process_run(tmp_path, monkeypatch, method):
     if method == "prediction-guided":
         pytest.importorskip("torch")
         if not torch.cuda.is_available():
             pytest.skip("prediction-guided selection launches K4 / K5 (the sharded GPU test covers it)")
     one, two = str(tmp_path / "w1"), str(tmp_path / "w2")
-    _run(one, method)
+    _run(one, method, monkeypatch.setattr)
     mp.spawn(_worker, args=(2, _free_port(), two, method), nprocs=2, join=True)
     migrated = int(open(os.path.join(two, "migrated.count")).read())
     os.remove(os.path.join(two, "migrated.count"))
