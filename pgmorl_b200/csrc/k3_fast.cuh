@@ -74,7 +74,7 @@ __host__ __device__ inline int k3_fast_stage_floats(int OP, int KH) {
     return (f.nrs1 - 1) * (H * OP + H) + (f.nrsH - 1) * KH * (H + 4);
 }
 
-template <int TM>
+template <int TM, int KU>
 __device__ __forceinline__ void layer_fwd_fast(const float *__restrict__ in, int ldi, const float *__restrict__ W,
                                                int ldw, const float *__restrict__ bias, int K,
                                                float *__restrict__ out, int tr, int tc) {
@@ -84,7 +84,8 @@ __device__ __forceinline__ void layer_fwd_fast(const float *__restrict__ in, int
     for (int i = 0; i < TM; ++i) acc[i][0] = acc[i][1] = acc[i][2] = acc[i][3] = 0ull;
     const float *ip = in + tr * ldi;
     const float *wp = W + 4 * tc * ldw;
-#pragma unroll 2
+    // KU k-blocks unrolled: with two warps per scheduler only independent loads of later k-blocks hide the LDS latency
+#pragma unroll(KU)
     for (int k = 0; k < K; k += 4) {
         ulonglong2 av[TM], b[4];
 #pragma unroll
@@ -294,10 +295,10 @@ __global__ void __launch_bounds__(NTHREADS, 1) k3_ppo_fast_kernel(const K3Args a
             PGM_TR(1)
 
             // ---------------- forward ----------------
-            layer_fwd_fast<TM>(x, RSS, n.W1, L.ldw1, n.b1, OP, h1, tr, tc);
+            layer_fwd_fast<TM, (TM == 2 ? 4 : 2)>(x, RSS, n.W1, L.ldw1, n.b1, OP, h1, tr, tc);
             if (more) gather_issue((ci + 1) & 1);  // async copies overlap layer 2 .. backward
             __syncthreads();
-            layer_fwd_fast<TM>(h1, LDH, n.W2, LDH, n.b2, H, h2, tr, tc);
+            layer_fwd_fast<TM, (TM == 2 ? H / 4 : 2)>(h1, LDH, n.W2, LDH, n.b2, H, h2, tr, tc);
             __syncthreads();
 
             // ---------------- head + per-element loss terms: item = (head row aa, batch row r) ----------------
@@ -305,7 +306,7 @@ __global__ void __launch_bounds__(NTHREADS, 1) k3_ppo_fast_kernel(const K3Args a
                 const int aa = i / RC, r = i - aa * RC;
                 const float *hp = h2 + r * LDH, *wp = n.Wh + aa * LDH;
                 u64 ac0 = 0ull, ac1 = 0ull;
-#pragma unroll 4
+#pragma unroll
                 for (int k = 0; k < H; k += 4) {
                     const ulonglong2 hv = lds2x64(hp + k), wv = lds2x64(wp + k);
                     ac0 = ffma2(hv.x, wv.x, ac0); ac1 = ffma2(hv.y, wv.y, ac1);
@@ -389,7 +390,7 @@ __global__ void __launch_bounds__(NTHREADS, 1) k3_ppo_fast_kernel(const K3Args a
             // ---------------- dW2, db2, dz1 -> d1 ----------------
             {
                 const int tj = tid & 15, tk = tid >> 4;
-#pragma unroll 4
+#pragma unroll 8
                 for (int r = 0; r < RC; ++r) {
                     const float4 dv = lds4(dz + r * LDH + 4 * tj);
                     const ulonglong2 hv = lds2x64(h1 + r * LDH + 4 * tk);
@@ -409,7 +410,7 @@ __global__ void __launch_bounds__(NTHREADS, 1) k3_ppo_fast_kernel(const K3Args a
                 u64 acc[TM][2];
 #pragma unroll
                 for (int i = 0; i < TM; ++i) acc[i][0] = acc[i][1] = 0ull;
-#pragma unroll 2
+#pragma unroll(TM == 2 ? 4 : 2)
                 for (int j = 0; j < H; j += 4) {
                     float4 av[TM];
                     ulonglong2 bv[4];
@@ -454,7 +455,7 @@ __global__ void __launch_bounds__(NTHREADS, 1) k3_ppo_fast_kernel(const K3Args a
 
             // ---------------- phase C: dW1/db1 on slots [0, nW1), dWh/dbh/dls on the rest ----------------
             if (isW1) {
-#pragma unroll 4
+#pragma unroll 8
                 for (int r = r1lo; r < r1hi; ++r) {
                     const float4 dv = lds4(d1 + r * LDH + 4 * l16);
                     const ulonglong2 xv = lds2x64(x + r * RSS + 4 * kg1);
@@ -469,7 +470,7 @@ __global__ void __launch_bounds__(NTHREADS, 1) k3_ppo_fast_kernel(const K3Args a
                 for (int ia = 0; ia < 4; ++ia) {
                     const int aa = aslot + ia * fp.nA;
                     if (aa < KH) {
-#pragma unroll 4
+#pragma unroll 8
                         for (int r = rhlo; r < rhhi; ++r) {
                             const float sv = ho[r * ldo + aa] * dlpS[r];
                             const ulonglong2 hv = lds2x64(h2 + r * LDH + 4 * l16);
