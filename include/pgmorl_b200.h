@@ -93,22 +93,40 @@ int pgm_policy_step_f32(const float *params, const int32_t *ctl, const float *ob
                         size_t logp_task_stride, float *act_out, int P, int N, int O, int A, int M, void *stream);
 
 /* ---------------------------------------------------------------------------
- * K2  vector-reward GAE + scalarised, normalised advantage.
- * Replaces RolloutStorage.compute_returns, branch use_gae && use_proper_time_limits
- * (a2c/storage.py:83-94) and the PPO.update preamble (a2c/algo/ppo.py:43-56) with
- * WeightedSumScalarization.evaluate (morl/scalarization_methods.py:28-29).
+ * K2  vector-reward returns + scalarised, normalised advantage.
+ * Replaces RolloutStorage.compute_returns (a2c/storage.py:77-116) and the PPO.update preamble
+ * (a2c/algo/ppo.py:43-56) with WeightedSumScalarization.evaluate (morl/scalarization_methods.py:28-29).
  *
  *   rewards [P,T,N,M]  value [P,T+1,N,M]  masks,bad_masks [P,T+1,N]
  *   weights [P,M]  obj_var [P,M] or NULL (NULL => no un-normalisation)
  *   returns [P,T,N,M] out     adv [P,T,N] out (skipped when weights==NULL or adv==NULL)
+ *
+ * pgm_returns_adv_f32: the branch of compute_returns is `mode`, an OR of
+ *   PGM_RET_GAE                 use_gae: generalised advantage estimation with lambda = lam
+ *                               (otherwise n-step discounted returns; lam is ignored)
+ *   PGM_RET_PROPER_TIME_LIMITS  use_proper_time_limits: bad_masks cut the recursion at time-limit ends
+ *                               (otherwise bad_masks is read by no branch)
+ *   boot [P,N,M] or NULL: the bootstrap value of the n-step branches (returns[-1] = next_value); NULL = value row T.
+ *   The GAE branches bootstrap from value row T and ignore boot. The advantage is returns - value[:T] in every branch.
+ * pgm_gae_adv_f32 = pgm_returns_adv_f32 with mode PGM_RET_GAE | PGM_RET_PROPER_TIME_LIMITS and boot NULL
+ *   (storage.py:83-94, the branch PG-MORL runs).
  */
+enum {
+    PGM_RET_GAE = 1,
+    PGM_RET_PROPER_TIME_LIMITS = 2
+};
+
+int pgm_returns_adv_f32(const float *rewards, const float *value, const float *boot, const float *masks,
+                        const float *bad_masks, const float *weights, const float *obj_var, float gamma, float lam,
+                        int mode, float *returns, float *adv, int P, int T, int N, int M, void *stream);
+
 int pgm_gae_adv_f32(const float *rewards, const float *value, const float *masks,
                     const float *bad_masks, const float *weights, const float *obj_var,
                     float gamma, float lam, float *returns, float *adv, int P, int T, int N, int M,
                     void *stream);
 
 /* ---------------------------------------------------------------------------
- * K3  PPO update: E epochs x B minibatches of clipped surrogate + clipped vector
+ * K3  PPO update: E epochs x B minibatches of clipped surrogate + (clipped) vector
  * value loss (- ecoef*entropy), backward, global grad-norm clip, Adam -- all tasks
  * in one launch, each task's chain of E*B dependent steps run by one thread-block
  * cluster. Replaces PPO.update (a2c/algo/ppo.py:62-115), feed_forward_generator
@@ -126,10 +144,15 @@ int pgm_gae_adv_f32(const float *rewards, const float *value, const float *masks
  *            shapes (17,6,2) and (11,3,3); 0 = choose from P, the shape and the SM count (tensor cores from 8 tasks on).
  *            Tensor-core operand ranges: |obs| < 65 504 (unscaled fp16 pairs), |parameter| < 255.9, |backward signal| < 16;
  *            beyond them the task's outputs become inf / NaN (non-saturating conversions), never a silently clamped result.
- *            OR-able flags 0x100 / 0x200 / 0x400 / 0x800 / 0x1000 / 0x2000 select the step tail of the FFMA cluster kernel
- *            (A/B and tests; bit-identical results; default = 0x2000, csrc/k3_ppo.cu).
+ *            OR-able flags 0x100 / 0x200 / 0x400 / 0x800 / 0x1000 / 0x2000 / 0x4000 select the step tail of the FFMA cluster
+ *            kernel (A/B and tests; bit-identical results; default = 0x2000, csrc/k3_ppo.cu).
+ *            OR-able flag PGM_PPO_VALUE_UNCLIPPED (every kernel family): the value loss is 0.5 * mean((V - R)^2)
+ *            (use_clipped_value_loss=False, a2c/algo/ppo.py:86-94 else branch) instead of the clipped
+ *            0.5 * mean(max((V - R)^2, (V_clip - R)^2)); losses[:,0] reports the loss that was minimised.
  *   S and B must satisfy S % B < S / B (the reference's BatchSampler(drop_last=True) then yields exactly B minibatches).
  */
+#define PGM_PPO_VALUE_UNCLIPPED 0x10000
+
 typedef struct {
     double clip_param;      /* 0.2  a2c/algo/ppo.py:83-84  */
     double value_loss_coef; /* 0.5  */

@@ -40,6 +40,7 @@ SIGNATURES = {
     "pgm_policy_forward_f32": (_I, [_P, _P, _P, _I, _P, _P, _P, _I, _I, _I, _I, _I, _I, _I, _P]),
     "pgm_policy_step_f32": (_I, [_P, _P, _P, _P, _I, _P, _Z, _P, _Z, _P, _Z, _P, _Z, _P, _I, _I, _I, _I, _I, _P]),
     "pgm_gae_adv_f32": (_I, [_P, _P, _P, _P, _P, _P, _F, _F, _P, _P, _I, _I, _I, _I, _P]),
+    "pgm_returns_adv_f32": (_I, [_P, _P, _P, _P, _P, _P, _P, _F, _F, _I, _P, _P, _I, _I, _I, _I, _P]),
     "pgm_ppo_workspace_bytes": (_Z, [_I, _I, _I, _I, _I, _I]),
     "pgm_ppo_update_f32": (_I, [_P, _P, _P, _P, _P, _P, _Z, _P, _P, _P, _Z, _P, _P, _P, _I, _I, _I,
                                 C.POINTER(PpoHyper), _P, _P, _Z, _I, _I, _I, _I, _I, _I, _P]),

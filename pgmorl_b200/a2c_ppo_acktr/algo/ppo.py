@@ -61,8 +61,6 @@ class PPO():
     def __init__(self, actor_critic, clip_param, ppo_epoch, num_mini_batch, value_loss_coef, entropy_coef, lr=None,
                  eps=None, max_grad_norm=None, use_clipped_value_loss=True, obj_weights=None, scalarization_func=None,
                  cluster=0):
-        if not use_clipped_value_loss:
-            raise NotImplementedError("PPO: PG-MORL uses the clipped value loss (ppo.py:86-94)")
         self.actor_critic = actor_critic
         self.clip_param, self.ppo_epoch, self.num_mini_batch = clip_param, ppo_epoch, num_mini_batch
         self.value_loss_coef, self.entropy_coef, self.max_grad_norm = value_loss_coef, entropy_coef, max_grad_norm
@@ -90,10 +88,11 @@ class PPO():
         w = torch.as_tensor(np.asarray(scal.weights, dtype=np.float64), dtype=torch.float32, device=dev)[None]
         ov = None if obj_var is None else torch.as_tensor(np.asarray(obj_var, dtype=np.float64) * np.ones(M),
                                                           dtype=torch.float32, device=dev)[None]
-        # advantage from the returns already in storage (ppo.py:43-56): K2 recomputes returns and normalises
-        ret, adv = K.gae_adv(rollouts.rewards[None], rollouts.value_preds[None], rollouts.masks.view(1, T + 1, N),
-                             rollouts.bad_masks.view(1, T + 1, N), self._gamma(rollouts), self._lam(rollouts),
-                             weights=w, obj_var=ov)
+        # advantage from the returns already in storage (ppo.py:43-56): K2 recomputes returns (same branch and bootstrap
+        # as compute_returns) and normalises
+        ret, adv = K.returns_adv(rollouts.rewards[None], rollouts.value_preds[None], rollouts.masks.view(1, T + 1, N),
+                                 rollouts.bad_masks.view(1, T + 1, N), self._gamma(rollouts), self._lam(rollouts),
+                                 weights=w, obj_var=ov, **rollouts.return_branch())
         perm = torch.stack([torch.randperm(S) for _ in range(self.ppo_epoch)]).to(torch.int32).to(dev)[None].contiguous()
         step = torch.tensor([opt.step_count], dtype=torch.int32, device=dev)
         lr = torch.tensor([opt.param_groups[0]["lr"]], dtype=torch.float64, device=dev)
@@ -103,7 +102,8 @@ class PPO():
         losses = K.ppo_update(params, m, v, step, lr, rollouts.obs.view(1, (T + 1) * N, d.obs),
                               rollouts.actions.view(1, S, d.act), rollouts.action_log_probs.view(1, S),
                               rollouts.value_preds.view(1, (T + 1) * N, M), ret.view(1, S, M), adv.view(1, S), perm,
-                              self.num_mini_batch, d, hyper=hyper, cluster=self.cluster)
+                              self.num_mini_batch, d, hyper=hyper, cluster=self.cluster,
+                              clipped_value_loss=self.use_clipped_value_loss)
         opt.step_count = int(step.item())
         vl, al, ent = losses[0].tolist()
         return vl, al, ent

@@ -1,5 +1,5 @@
 """RolloutStorage with the reference's buffers and methods (a2c_ppo_acktr/storage.py:9-154), resident in HBM as
-float32. compute_returns (GAE with proper time limits, the branch PG-MORL uses: storage.py:83-94) is a K2 launch."""
+float32. compute_returns (all four branches of storage.py:77-116) is a K2 launch."""
 import torch
 
 from .. import kernels as K
@@ -47,15 +47,25 @@ class RolloutStorage(object):
         self.bad_masks[0].copy_(self.bad_masks[-1])
 
     def compute_returns(self, next_value, use_gae, gamma, gae_lambda, use_proper_time_limits=True):
-        if not (use_gae and use_proper_time_limits):
-            raise NotImplementedError("compute_returns: PG-MORL runs use_gae with proper time limits "
-                                      "(morl/run.py:56-70); the other branches of storage.py:77-116 are not ported")
-        self.gamma, self.gae_lambda = gamma, gae_lambda      # PPO.update re-derives the advantage with the same values
-        self.value_preds[-1].copy_(torch.as_tensor(next_value).to(self.obs.device, torch.float32))
+        # PPO.update re-derives the advantage with the same branch and values (return_branch())
+        self.gamma, self.gae_lambda = gamma, gae_lambda
+        self.use_gae, self.use_proper_time_limits = bool(use_gae), bool(use_proper_time_limits)
+        nv = torch.as_tensor(next_value).to(self.obs.device, torch.float32)
+        if use_gae:
+            self.value_preds[-1].copy_(nv)
+        else:
+            self.returns[-1].copy_(nv)        # the n-step branches bootstrap from returns[-1]; value_preds[-1] is left alone
         T, N, M = self.rewards.shape
-        ret, _ = K.gae_adv(self.rewards[None], self.value_preds[None], self.masks.view(1, T + 1, N),
-                           self.bad_masks.view(1, T + 1, N), gamma, gae_lambda)
+        ret, _ = K.returns_adv(self.rewards[None], self.value_preds[None], self.masks.view(1, T + 1, N),
+                               self.bad_masks.view(1, T + 1, N), gamma, gae_lambda, **self.return_branch())
         self.returns[:-1].copy_(ret[0])
+
+    def return_branch(self):
+        """Keyword arguments of kernels.returns_adv for the branch the last compute_returns took (default: GAE with
+        proper time limits, morl/run.py:56-70)."""
+        use_gae = getattr(self, "use_gae", True)
+        return dict(use_gae=use_gae, use_proper_time_limits=getattr(self, "use_proper_time_limits", True),
+                    boot=None if use_gae else self.returns[-1][None])
 
     def feed_forward_generator(self, advantages, num_mini_batch=None, mini_batch_size=None):
         """Same minibatches as storage.py:118-154 (torch.randperm on the global CPU generator); the device PPO

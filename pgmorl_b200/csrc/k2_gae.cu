@@ -1,14 +1,18 @@
-// K2 -- vector-reward GAE + weight-scalarised, normalised advantage.
+// K2 -- vector-reward returns + weight-scalarised, normalised advantage.
 //
-// Replaces RolloutStorage.compute_returns (a2c/storage.py:83-94: use_gae and
+// Replaces RolloutStorage.compute_returns (a2c/storage.py:77-116, all four branches of use_gae x
 // use_proper_time_limits) and the PPO.update preamble (a2c/algo/ppo.py:43-56) with
 // WeightedSumScalarization.evaluate (morl/scalarization_methods.py:28-29).
 //
-// The reference's recurrence, per env column n and objective m, going backwards in t:
-//     delta_t = r_t + gamma * V_{t+1} * mask_{t+1} - V_t
-//     g_t     = (delta_t + gamma*lam*mask_{t+1} * g_{t+1}) * bad_{t+1}
-//     ret_t   = g_t + V_t
-// is the affine map g_t = a_t * g_{t+1} + d_t with a_t = gamma*lam*mask*bad, d_t = delta_t*bad.
+// Every branch of the reference, per env column n and objective m, going backwards in t, is the
+// affine map g_t = a_t * g_{t+1} + d_t (m = mask_{t+1}, b = bad_{t+1}, delta_t = r_t + gamma*V_{t+1}*m - V_t):
+//     MODE                     a_t           d_t                   g at t = T   ret_t     raw advantage
+//     GAE | PROPER_TIME_LIMITS gamma*lam*m*b delta_t * b           0            g + V_t   g
+//     PROPER_TIME_LIMITS       gamma*m*b     r_t*b + (1 - b)*V_t   bootstrap    g         g - V_t
+//     GAE                      gamma*lam*m   delta_t               0            g + V_t   g
+//     (none: n-step returns)   gamma*m       r_t                   bootstrap    g         g - V_t
+// The bootstrap is `boot` [P,N,M], or value row T when boot is NULL. MODE is a template parameter, so the
+// first row compiles to exactly the instructions it had before the other branches existed.
 // One CTA per task, one warp per env column: the warp walks T in blocks of 32 steps (lane = step,
 // so global loads of a block are contiguous across the CTA's warps), composes the 32 affine maps
 // with a shuffle scan and chains blocks through a carried g. The scalarised raw advantage
@@ -22,12 +26,30 @@ namespace pgm {
 
 constexpr int K2_MAXM = 8;
 
-template <int M>
+template <int MODE>
+__device__ __forceinline__ float k2_boot(const float *__restrict__ boot, const float *__restrict__ value, int task, int T,
+                                         int N, int M, int n, int m) {
+    if (MODE & PGM_RET_GAE) return 0.f;
+    return boot ? __ldg(boot + ((size_t)task * N + n) * M + m) : __ldg(value + ((size_t)T * N + n) * M + m);
+}
+
+// d_t of step t for one objective (table above); mk, bd = mask / bad mask of slot t+1, v = V_t, vnp -> V_{t+1}
+template <int MODE>
+__device__ __forceinline__ float k2_d(float r, float v, const float *__restrict__ vnp, float gamma, float mk, float bd) {
+    if (MODE == (PGM_RET_GAE | PGM_RET_PROPER_TIME_LIMITS)) return (r + gamma * __ldg(vnp) * mk - v) * bd;
+    if (MODE == PGM_RET_GAE) return r + gamma * __ldg(vnp) * mk - v;
+    if (MODE == PGM_RET_PROPER_TIME_LIMITS) return fmaf(r, bd, (1.f - bd) * v);
+    return r;
+}
+
+template <int M, int MODE>
 __global__ void __launch_bounds__(1024) k2_gae_kernel(const float *__restrict__ rewards, const float *__restrict__ value,
+                                                      const float *__restrict__ boot,
                                                       const float *__restrict__ masks, const float *__restrict__ bad_masks,
                                                       const float *__restrict__ weights, const float *__restrict__ obj_var,
                                                       float gamma, float lam, float *__restrict__ returns,
                                                       float *__restrict__ adv, int T, int N) {
+    constexpr bool GAE = (MODE & PGM_RET_GAE) != 0, PTL = (MODE & PGM_RET_PROPER_TIME_LIMITS) != 0;
     __shared__ float red[34];
     const int task = blockIdx.x;
     const int lane = threadIdx.x & 31, n = threadIdx.x >> 5;   // warp n <-> env column n
@@ -45,10 +67,10 @@ __global__ void __launch_bounds__(1024) k2_gae_kernel(const float *__restrict__ 
         float s = obj_var ? sqrtf(__ldg(obj_var + task * M + m) + 1e-8f) : 1.f;
         ws[m] = do_adv ? __ldg(weights + task * M + m) * s : 0.f;
     }
-    const float gl = gamma * lam;
+    const float gl = GAE ? gamma * lam : gamma;
     float carry[M];
 #pragma unroll
-    for (int m = 0; m < M; ++m) carry[m] = 0.f;
+    for (int m = 0; m < M; ++m) carry[m] = k2_boot<MODE>(boot, value, task, T, N, M, n, m);
     float psum = 0.f;
 
     const int nblk = (T + 31) / 32;
@@ -60,14 +82,13 @@ __global__ void __launch_bounds__(1024) k2_gae_kernel(const float *__restrict__ 
         for (int m = 0; m < M; ++m) { d[m] = 0.f; v[m] = 0.f; }
         if (ok) {
             const float mk = __ldg(masks + (size_t)(t + 1) * N + n);
-            const float bd = __ldg(bad_masks + (size_t)(t + 1) * N + n);
-            a = gl * mk * bd;
+            const float bd = PTL ? __ldg(bad_masks + (size_t)(t + 1) * N + n) : 1.f;
+            a = PTL ? gl * mk * bd : gl * mk;
 #pragma unroll
             for (int m = 0; m < M; ++m) {
                 const float r = __ldg(rewards + ((size_t)t * N + n) * M + m);
                 v[m] = __ldg(value + ((size_t)t * N + n) * M + m);
-                const float vn = __ldg(value + ((size_t)(t + 1) * N + n) * M + m);
-                d[m] = (r + gamma * vn * mk - v[m]) * bd;
+                d[m] = k2_d<MODE>(r, v[m], value + ((size_t)(t + 1) * N + n) * M + m, gamma, mk, bd);
             }
         }
         // suffix composition over lanes: after the scan, g_t = d + a * carry where (a, d) is the
@@ -88,11 +109,11 @@ __global__ void __launch_bounds__(1024) k2_gae_kernel(const float *__restrict__ 
 #pragma unroll
         for (int m = 0; m < M; ++m) {
             g[m] = fmaf(a, carry[m], d[m]);
-            s = fmaf(ws[m], g[m], s);
+            s = fmaf(ws[m], GAE ? g[m] : g[m] - v[m], s);
         }
         if (ok) {
 #pragma unroll
-            for (int m = 0; m < M; ++m) returns[((size_t)t * N + n) * M + m] = g[m] + v[m];
+            for (int m = 0; m < M; ++m) returns[((size_t)t * N + n) * M + m] = GAE ? g[m] + v[m] : g[m];
             if (do_adv) { adv[(size_t)t * N + n] = s; psum += s; }
         }
 #pragma unroll
@@ -117,12 +138,14 @@ __global__ void __launch_bounds__(1024) k2_gae_kernel(const float *__restrict__ 
 // unknown right-hand carry is scaled by (g_t = g_loc_t + A_t * G_in), both in shared memory. Phase 2: N*M threads chain the
 // NSEG segment maps (a handful of steps). Phase 3: every warp finishes its segment. The dependent chain shrinks from T/32
 // to T/(32 NSEG) + NSEG rounds.
-template <int M>
+template <int M, int MODE>
 __global__ void __launch_bounds__(1024) k2_gae_seg_kernel(const float *__restrict__ rewards, const float *__restrict__ value,
+                                                          const float *__restrict__ boot,
                                                           const float *__restrict__ masks, const float *__restrict__ bad_masks,
                                                           const float *__restrict__ weights, const float *__restrict__ obj_var,
                                                           float gamma, float lam, float *__restrict__ returns,
                                                           float *__restrict__ adv, int T, int N, int NSEG, int SEG) {
+    constexpr bool GAE = (MODE & PGM_RET_GAE) != 0, PTL = (MODE & PGM_RET_PROPER_TIME_LIMITS) != 0;
     extern __shared__ float sm[];                 // A[T*N] | Gloc[M][T*N]
     __shared__ float red[34];
     __shared__ float segA[32], segG[32][M], segIn[32][M];     // per warp (= column, segment)
@@ -146,7 +169,7 @@ __global__ void __launch_bounds__(1024) k2_gae_seg_kernel(const float *__restric
         float s = obj_var ? sqrtf(__ldg(obj_var + task * M + m) + 1e-8f) : 1.f;
         ws[m] = do_adv ? __ldg(weights + task * M + m) * s : 0.f;
     }
-    const float gl = gamma * lam;
+    const float gl = GAE ? gamma * lam : gamma;
     const int t0 = sg * SEG, t1 = min(T, t0 + SEG);          // my segment [t0, t1)
 
     // ---- phase 1: local solution of my segment (carry 0 from the right) ----
@@ -162,14 +185,13 @@ __global__ void __launch_bounds__(1024) k2_gae_seg_kernel(const float *__restric
             for (int m = 0; m < M; ++m) d[m] = 0.f;
             if (ok) {
                 const float mk = __ldg(masks + (size_t)(t + 1) * N + n);
-                const float bd = __ldg(bad_masks + (size_t)(t + 1) * N + n);
-                a = gl * mk * bd;
+                const float bd = PTL ? __ldg(bad_masks + (size_t)(t + 1) * N + n) : 1.f;
+                a = PTL ? gl * mk * bd : gl * mk;
 #pragma unroll
                 for (int m = 0; m < M; ++m) {
                     const float r = __ldg(rewards + ((size_t)t * N + n) * M + m);
                     const float v = __ldg(value + ((size_t)t * N + n) * M + m);
-                    const float vn = __ldg(value + ((size_t)(t + 1) * N + n) * M + m);
-                    d[m] = (r + gamma * vn * mk - v) * bd;
+                    d[m] = k2_d<MODE>(r, v, value + ((size_t)(t + 1) * N + n) * M + m, gamma, mk, bd);
                 }
             }
 #pragma unroll
@@ -204,10 +226,11 @@ __global__ void __launch_bounds__(1024) k2_gae_seg_kernel(const float *__restric
         }
     }
     __syncthreads();
-    // ---- phase 2: chain the segment maps from the right: G_in(sg) = g at the first step of segment sg + 1 ----
+    // ---- phase 2: chain the segment maps from the right: G_in(sg) = g at the first step of segment sg + 1; the last
+    //      segment's right-hand carry is 0 (GAE) or the bootstrap (n-step) ----
     if (threadIdx.x < N * M) {
         const int nn = threadIdx.x / M, m = threadIdx.x % M;
-        float G = 0.f;
+        float G = k2_boot<MODE>(boot, value, task, T, N, M, nn, m);
         for (int q = NSEG - 1; q >= 0; --q) {
             const int ww = q * N + nn;
             segIn[ww][m] = G;
@@ -227,8 +250,9 @@ __global__ void __launch_bounds__(1024) k2_gae_seg_kernel(const float *__restric
 #pragma unroll
             for (int m = 0; m < M; ++m) {
                 const float g = fmaf(At, gin[m], Gsh[(size_t)m * S + (size_t)t * N + n]);
-                returns[((size_t)t * N + n) * M + m] = g + __ldg(value + ((size_t)t * N + n) * M + m);
-                s = fmaf(ws[m], g, s);
+                const float v = __ldg(value + ((size_t)t * N + n) * M + m);
+                returns[((size_t)t * N + n) * M + m] = GAE ? g + v : g;
+                s = fmaf(ws[m], GAE ? g : g - v, s);
             }
             if (do_adv) { Ash[(size_t)t * N + n] = s; psum += s; }      // raw advantage stays on chip for the normalisation
         }
@@ -247,14 +271,10 @@ __global__ void __launch_bounds__(1024) k2_gae_seg_kernel(const float *__restric
 
 using namespace pgm;
 
-extern "C" int pgm_gae_adv_f32(const float *rewards, const float *value, const float *masks, const float *bad_masks,
-                               const float *weights, const float *obj_var, float gamma, float lam, float *returns,
-                               float *adv, int P, int T, int N, int M, void *stream) {
-    PGM_REQUIRE(rewards && value && masks && bad_masks && returns, "pgm_gae_adv_f32: null pointer");
-    PGM_REQUIRE(P > 0 && T > 0 && N > 0 && N <= 32, "pgm_gae_adv_f32: need 1 <= N <= 32 env columns (got %d)", N);
-    PGM_REQUIRE(M >= 1 && M <= K2_MAXM, "pgm_gae_adv_f32: obj_num %d unsupported", M);
-    PGM_REQUIRE(!(weights && adv) || (long long)T * N >= 2, "pgm_gae_adv_f32: need >= 2 samples to normalise");
-    cudaStream_t st = (cudaStream_t)stream;
+template <int MODE>
+static int k2_launch(const float *rewards, const float *value, const float *boot, const float *masks, const float *bad_masks,
+                     const float *weights, const float *obj_var, float gamma, float lam, float *returns, float *adv, int P,
+                     int T, int N, int M, cudaStream_t st) {
     // small populations: 32 warps per task, the time axis cut into 32 / N segments (k2_gae_seg_kernel); needs the task's
     // (1 + M) * T * N floats of scratch in shared memory. Large populations already fill the GPU with one warp per column.
     const size_t seg_smem = (size_t)(1 + M) * T * N * sizeof(float);
@@ -262,17 +282,65 @@ extern "C" int pgm_gae_adv_f32(const float *rewards, const float *value, const f
         const int NSEG = 32 / N;
         const int SEG = ((T + NSEG - 1) / NSEG + 31) / 32 * 32;
 #define PGM_K2S(MM) case MM: \
-            PGM_CUDA(cudaFuncSetAttribute(k2_gae_seg_kernel<MM>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)seg_smem)); \
-            k2_gae_seg_kernel<MM><<<P, 1024, seg_smem, st>>>(rewards, value, masks, bad_masks, weights, obj_var, gamma, lam, returns, adv, T, N, NSEG, SEG); break;
+            PGM_CUDA(cudaFuncSetAttribute(k2_gae_seg_kernel<MM, MODE>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)seg_smem)); \
+            k2_gae_seg_kernel<MM, MODE><<<P, 1024, seg_smem, st>>>(rewards, value, boot, masks, bad_masks, weights, obj_var, gamma, lam, returns, adv, T, N, NSEG, SEG); break;
         switch (M) { PGM_K2S(1) PGM_K2S(2) PGM_K2S(3) PGM_K2S(4) }
 #undef PGM_K2S
         PGM_CUDA(cudaGetLastError());
         return PGM_OK;
     }
     dim3 grid(P), block(32 * N);
-#define PGM_K2(MM) case MM: k2_gae_kernel<MM><<<grid, block, 0, st>>>(rewards, value, masks, bad_masks, weights, obj_var, gamma, lam, returns, adv, T, N); break;
+#define PGM_K2(MM) case MM: k2_gae_kernel<MM, MODE><<<grid, block, 0, st>>>(rewards, value, boot, masks, bad_masks, weights, obj_var, gamma, lam, returns, adv, T, N); break;
     switch (M) { PGM_K2(1) PGM_K2(2) PGM_K2(3) PGM_K2(4) PGM_K2(5) PGM_K2(6) PGM_K2(7) PGM_K2(8) }
 #undef PGM_K2
     PGM_CUDA(cudaGetLastError());
     return PGM_OK;
+}
+
+// argument checks of both entry points (messages name the function the caller called)
+static int k2_check(const char *fn, const float *rewards, const float *value, const float *masks, const float *bad_masks,
+                    const float *weights, int mode, const float *returns, const float *adv, int P, int T, int N, int M) {
+    PGM_REQUIRE(rewards && value && masks && bad_masks && returns, "%s: null pointer", fn);
+    PGM_REQUIRE(P > 0 && T > 0 && N > 0 && N <= 32, "%s: need 1 <= N <= 32 env columns (got %d)", fn, N);
+    PGM_REQUIRE(M >= 1 && M <= K2_MAXM, "%s: obj_num %d unsupported", fn, M);
+    PGM_REQUIRE(!(weights && adv) || (long long)T * N >= 2, "%s: need >= 2 samples to normalise", fn);
+    PGM_REQUIRE((mode & ~(PGM_RET_GAE | PGM_RET_PROPER_TIME_LIMITS)) == 0, "%s: unknown mode bits 0x%x", fn, mode);
+    return PGM_OK;
+}
+
+static int k2_run(int mode, const float *rewards, const float *value, const float *boot, const float *masks,
+                  const float *bad_masks, const float *weights, const float *obj_var, float gamma, float lam, float *returns,
+                  float *adv, int P, int T, int N, int M, void *stream) {
+    cudaStream_t st = (cudaStream_t)stream;
+    switch (mode) {
+        case PGM_RET_GAE | PGM_RET_PROPER_TIME_LIMITS:
+            return k2_launch<PGM_RET_GAE | PGM_RET_PROPER_TIME_LIMITS>(rewards, value, boot, masks, bad_masks, weights, obj_var,
+                                                                         gamma, lam, returns, adv, P, T, N, M, st);
+        case PGM_RET_GAE:
+            return k2_launch<PGM_RET_GAE>(rewards, value, boot, masks, bad_masks, weights, obj_var, gamma, lam, returns, adv, P,
+                                          T, N, M, st);
+        case PGM_RET_PROPER_TIME_LIMITS:
+            return k2_launch<PGM_RET_PROPER_TIME_LIMITS>(rewards, value, boot, masks, bad_masks, weights, obj_var, gamma, lam,
+                                                         returns, adv, P, T, N, M, st);
+        default:
+            return k2_launch<0>(rewards, value, boot, masks, bad_masks, weights, obj_var, gamma, lam, returns, adv, P, T, N, M, st);
+    }
+}
+
+extern "C" int pgm_returns_adv_f32(const float *rewards, const float *value, const float *boot, const float *masks,
+                                   const float *bad_masks, const float *weights, const float *obj_var, float gamma, float lam,
+                                   int mode, float *returns, float *adv, int P, int T, int N, int M, void *stream) {
+    if (int rc = k2_check("pgm_returns_adv_f32", rewards, value, masks, bad_masks, weights, mode, returns, adv, P, T, N, M))
+        return rc;
+    return k2_run(mode, rewards, value, boot, masks, bad_masks, weights, obj_var, gamma, lam, returns, adv, P, T, N, M, stream);
+}
+
+extern "C" int pgm_gae_adv_f32(const float *rewards, const float *value, const float *masks, const float *bad_masks,
+                               const float *weights, const float *obj_var, float gamma, float lam, float *returns,
+                               float *adv, int P, int T, int N, int M, void *stream) {
+    const int mode = PGM_RET_GAE | PGM_RET_PROPER_TIME_LIMITS;
+    if (int rc = k2_check("pgm_gae_adv_f32", rewards, value, masks, bad_masks, weights, mode, returns, adv, P, T, N, M))
+        return rc;
+    return k2_run(mode, rewards, value, nullptr, masks, bad_masks, weights, obj_var, gamma, lam, returns, adv, P, T, N, M,
+                  stream);
 }

@@ -131,7 +131,7 @@ __device__ __forceinline__ void layer_fwd_fast(const float *__restrict__ in, int
 // TAIL = 6  : as TAIL = 5, and the slices that hold only dW2 (5 of 8 at Walker2d dims, 70 % of the bytes) leave EARLY: dW2 is
 //             final after the {dW2, dz1} phase of the step's last chunk, so its tiles are written to the image there and the
 //             bulk copies of the W2-only slices fly under phase C, the row-split combine and the rest of the image write.
-template <int C, int TM, int TAIL>
+template <int C, int TM, int TAIL, bool VU = false>
 __global__ void __launch_bounds__(NTHREADS, 1) k3_ppo_fast_kernel(const K3Args a) {
     constexpr bool RA = TAIL == 1, MC = TAIL >= 2, GL = TAIL == 3, BP = TAIL >= 4, NB = TAIL >= 5, EP = TAIL == 6;
     constexpr int RC = 16 * TM;
@@ -328,7 +328,8 @@ __global__ void __launch_bounds__(NTHREADS, 1) k3_ppo_fast_kernel(const K3Args a
                     const float dlt = V - vo;
                     const float vcl = vo + fminf(fmaxf(dlt, -clip), clip);
                     const float ea = V - R, eb = vcl - R;
-                    const float la = ea * ea, lb = eb * eb;
+                    // unclipped value loss (VU): lb = -1 < 0 <= la, so max(la, lb) = la and wa = 1, gradient 2 * ea exactly
+                    const float la = ea * ea, lb = VU ? -1.f : eb * eb;
                     const float wa = la > lb ? 1.f : (la == lb ? 0.5f : 0.f);
                     const float pas = (dlt >= -clip && dlt <= clip) ? 1.f : 0.f;
                     if (valid) loss_val += fmaxf(la, lb);

@@ -1,8 +1,9 @@
 // K3 -- PPO update for the whole population shard in ONE launch.
 //
 // Replaces PPO.update's minibatch loop (a2c/algo/ppo.py:62-107): evaluate_actions,
-// clipped surrogate, clipped vector value loss, autograd backward, clip_grad_norm_ and
-// Adam.step, plus the sampler of a2c/storage.py:118-154 (consumes the host permutation).
+// clipped surrogate, clipped (use_clipped_value_loss) or plain vector value loss, autograd
+// backward, clip_grad_norm_ and Adam.step, plus the sampler of a2c/storage.py:118-154
+// (consumes the host permutation).
 //
 // Parallel decomposition. A task is a chain of E*B dependent optimiser steps, so the only
 // parallelism inside a step is over the minibatch rows and over the two independent networks
@@ -128,11 +129,12 @@ __device__ __forceinline__ float fast_sqrt(float x) { float r; asm("sqrt.approx.
 
 // C: CTAs per task; TM: rows per thread per chunk (chunk = 16*TM rows);
 // KG1: 4-column groups of dW1 per thread (OP <= 64*KG1); NA: head rows per thread (A,M <= 16*NA);
-// DB: double-buffered record gather.
+// DB: double-buffered record gather; VU: unclipped value loss (every kernel family takes it as a template parameter, so the
+// clipped instantiations are the code they were before the option existed).
 // Generic path (any supported dims, incl. wide observations and C == 1): each CTA updates a 1/G
 // slice of its half in global memory and all CTAs reload the parameters (three barriers per step).
 // Small networks on C >= 2 take the fast path in k3_fast.cuh instead.
-template <int C, int TM, int KG1, int NA, bool DB>
+template <int C, int TM, int KG1, int NA, bool DB, bool VU = false>
 __global__ void __launch_bounds__(NTHREADS, 1) k3_ppo_kernel(const K3Args a) {
     constexpr int RC = 16 * TM;
     constexpr int NHALF = (C == 1) ? 2 : 1;
@@ -291,7 +293,8 @@ __global__ void __launch_bounds__(NTHREADS, 1) k3_ppo_kernel(const K3Args a) {
                             const float d = V - vo;
                             const float vcl = vo + fminf(fmaxf(d, -clip), clip);
                             const float ea = V - R, eb = vcl - R;
-                            const float la = ea * ea, lb = eb * eb;
+                            // unclipped value loss (VU): lb = -1 < 0 <= la, so max(la, lb) = la and wa = 1, gradient 2 * ea exactly
+                            const float la = ea * ea, lb = VU ? -1.f : eb * eb;
                             const float wa = la > lb ? 1.f : (la == lb ? 0.5f : 0.f);
                             const float pas = (d >= -clip && d <= clip) ? 1.f : 0.f;
                             if (valid) loss_val += fmaxf(la, lb);
@@ -556,6 +559,7 @@ namespace pgm {
 struct K3Plan {
     int C, G, TM, KG1, NA, RC, Rg, RSG, RSS, NHP;
     bool DB, fast, tc, tcw;
+    bool vu;      // unclipped value loss (PGM_PPO_VALUE_UNCLIPPED): the VU = true instantiation of the chosen kernel
     int tail;     // fast path step tail (k3_fast.cuh): 0 three cluster barriers, 1 redundant Adam, 2 TMA multicast broadcast
     int rs;
     int stage_floats;
@@ -637,7 +641,7 @@ constexpr int K3_CLUSTER_TAILBP = 0x1000;  // tail 4
 constexpr int K3_CLUSTER_TAILNB = 0x2000;  // tail 5
 constexpr int K3_CLUSTER_TAILEP = 0x4000;  // tail 6
 constexpr int K3_CLUSTER_FLAGS = K3_CLUSTER_TAIL2 | K3_CLUSTER_TAILMC | K3_CLUSTER_TAILGL | K3_CLUSTER_TAIL0 | K3_CLUSTER_TAILBP |
-                                 K3_CLUSTER_TAILNB | K3_CLUSTER_TAILEP;
+                                 K3_CLUSTER_TAILNB | K3_CLUSTER_TAILEP | PGM_PPO_VALUE_UNCLIPPED;
 
 static int k3_plan(K3Plan &pl, int P, int S, int mb, int O, int A, int M, int cluster, int sms) {
     NetLayout L(O, A, M);
@@ -645,6 +649,7 @@ static int k3_plan(K3Plan &pl, int P, int S, int mb, int O, int A, int M, int cl
     const bool tailgl = (cluster & K3_CLUSTER_TAILGL) != 0, tail0 = (cluster & K3_CLUSTER_TAIL0) != 0;
     const bool tailbp = (cluster & K3_CLUSTER_TAILBP) != 0, tailnb = (cluster & K3_CLUSTER_TAILNB) != 0;
     const bool tailep = (cluster & K3_CLUSTER_TAILEP) != 0;
+    pl.vu = (cluster & PGM_PPO_VALUE_UNCLIPPED) != 0;
     cluster &= ~K3_CLUSTER_FLAGS;
     pl.tc = false; pl.tcw = false; pl.tail = 0; pl.off_mv = 0;
     // wide observations (Humanoid): the streamed tensor-core kernel; row split over as many CTAs per half as fill the SMs
@@ -782,39 +787,39 @@ static int k3_launch_k(Kern kern, int C, const K3Args &a, const K3Plan &pl, int 
     return PGM_OK;
 }
 
-template <int C>
+template <int C, bool VU>
 static int k3_launch_c(const K3Args &a, const K3Plan &pl, int P, cudaStream_t st) {
     if constexpr (C > 1) {
         if (pl.fast) {
             if (pl.tail == 1)
-                return pl.TM == 2 ? k3_launch_k(k3_ppo_fast_kernel<C, 2, 1>, C, a, pl, P, st)
-                                  : k3_launch_k(k3_ppo_fast_kernel<C, 4, 1>, C, a, pl, P, st);
+                return pl.TM == 2 ? k3_launch_k(k3_ppo_fast_kernel<C, 2, 1, VU>, C, a, pl, P, st)
+                                  : k3_launch_k(k3_ppo_fast_kernel<C, 4, 1, VU>, C, a, pl, P, st);
             if (pl.tail == 2)
-                return pl.TM == 2 ? k3_launch_k(k3_ppo_fast_kernel<C, 2, 2>, C, a, pl, P, st)
-                                  : k3_launch_k(k3_ppo_fast_kernel<C, 4, 2>, C, a, pl, P, st);
+                return pl.TM == 2 ? k3_launch_k(k3_ppo_fast_kernel<C, 2, 2, VU>, C, a, pl, P, st)
+                                  : k3_launch_k(k3_ppo_fast_kernel<C, 4, 2, VU>, C, a, pl, P, st);
             if (pl.tail == 3)
-                return pl.TM == 2 ? k3_launch_k(k3_ppo_fast_kernel<C, 2, 3>, C, a, pl, P, st)
-                                  : k3_launch_k(k3_ppo_fast_kernel<C, 4, 3>, C, a, pl, P, st);
+                return pl.TM == 2 ? k3_launch_k(k3_ppo_fast_kernel<C, 2, 3, VU>, C, a, pl, P, st)
+                                  : k3_launch_k(k3_ppo_fast_kernel<C, 4, 3, VU>, C, a, pl, P, st);
             if (pl.tail == 4)
-                return pl.TM == 2 ? k3_launch_k(k3_ppo_fast_kernel<C, 2, 4>, C, a, pl, P, st)
-                                  : k3_launch_k(k3_ppo_fast_kernel<C, 4, 4>, C, a, pl, P, st);
+                return pl.TM == 2 ? k3_launch_k(k3_ppo_fast_kernel<C, 2, 4, VU>, C, a, pl, P, st)
+                                  : k3_launch_k(k3_ppo_fast_kernel<C, 4, 4, VU>, C, a, pl, P, st);
             if (pl.tail == 5)
-                return pl.TM == 2 ? k3_launch_k(k3_ppo_fast_kernel<C, 2, 5>, C, a, pl, P, st)
-                                  : k3_launch_k(k3_ppo_fast_kernel<C, 4, 5>, C, a, pl, P, st);
+                return pl.TM == 2 ? k3_launch_k(k3_ppo_fast_kernel<C, 2, 5, VU>, C, a, pl, P, st)
+                                  : k3_launch_k(k3_ppo_fast_kernel<C, 4, 5, VU>, C, a, pl, P, st);
             if (pl.tail == 6)
-                return pl.TM == 2 ? k3_launch_k(k3_ppo_fast_kernel<C, 2, 6>, C, a, pl, P, st)
-                                  : k3_launch_k(k3_ppo_fast_kernel<C, 4, 6>, C, a, pl, P, st);
+                return pl.TM == 2 ? k3_launch_k(k3_ppo_fast_kernel<C, 2, 6, VU>, C, a, pl, P, st)
+                                  : k3_launch_k(k3_ppo_fast_kernel<C, 4, 6, VU>, C, a, pl, P, st);
 
-            return pl.TM == 2 ? k3_launch_k(k3_ppo_fast_kernel<C, 2, 0>, C, a, pl, P, st)
-                              : k3_launch_k(k3_ppo_fast_kernel<C, 4, 0>, C, a, pl, P, st);
+            return pl.TM == 2 ? k3_launch_k(k3_ppo_fast_kernel<C, 2, 0, VU>, C, a, pl, P, st)
+                              : k3_launch_k(k3_ppo_fast_kernel<C, 4, 0, VU>, C, a, pl, P, st);
         }
-        if (pl.KG1 == 6) return k3_launch_k(k3_ppo_kernel<C, 2, 6, 2, false>, C, a, pl, P, st);
-        return pl.TM == 2 ? k3_launch_k(k3_ppo_kernel<C, 2, 1, 1, true>, C, a, pl, P, st)
-                          : k3_launch_k(k3_ppo_kernel<C, 4, 1, 1, true>, C, a, pl, P, st);
+        if (pl.KG1 == 6) return k3_launch_k(k3_ppo_kernel<C, 2, 6, 2, false, VU>, C, a, pl, P, st);
+        return pl.TM == 2 ? k3_launch_k(k3_ppo_kernel<C, 2, 1, 1, true, VU>, C, a, pl, P, st)
+                          : k3_launch_k(k3_ppo_kernel<C, 4, 1, 1, true, VU>, C, a, pl, P, st);
     } else {
-        if (pl.KG1 == 6) return k3_launch_k(k3_ppo_kernel<1, 2, 6, 2, false>, 1, a, pl, P, st);
-        return pl.TM == 2 ? k3_launch_k(k3_ppo_kernel<1, 2, 1, 1, false>, 1, a, pl, P, st)
-                          : k3_launch_k(k3_ppo_kernel<1, 4, 1, 1, false>, 1, a, pl, P, st);
+        if (pl.KG1 == 6) return k3_launch_k(k3_ppo_kernel<1, 2, 6, 2, false, VU>, 1, a, pl, P, st);
+        return pl.TM == 2 ? k3_launch_k(k3_ppo_kernel<1, 2, 1, 1, false, VU>, 1, a, pl, P, st)
+                          : k3_launch_k(k3_ppo_kernel<1, 4, 1, 1, false, VU>, 1, a, pl, P, st);
     }
 }
 
@@ -831,22 +836,30 @@ static int k3_launch_w(Kern kern, const K3Args &a, const TwExtra &x, const K3Pla
     return PGM_OK;
 }
 
+template <bool VU>
 static int k3_launch(const K3Args &a, const K3Plan &pl, int P, cudaStream_t st) {
     if (pl.tc) {
-        if (a.L.O == 17) return pl.rs == 2 ? k3_launch_k(k3_tc_kernel<17, 6, 2, 2>, pl.C, a, pl, P, st)
-                                           : k3_launch_k(k3_tc_kernel<17, 6, 2, 1>, pl.C, a, pl, P, st);
-        return pl.rs == 2 ? k3_launch_k(k3_tc_kernel<11, 3, 3, 2>, pl.C, a, pl, P, st)
-                          : k3_launch_k(k3_tc_kernel<11, 3, 3, 1>, pl.C, a, pl, P, st);
+        if (a.L.O == 17) return pl.rs == 2 ? k3_launch_k(k3_tc_kernel<17, 6, 2, 2, VU>, pl.C, a, pl, P, st)
+                                           : k3_launch_k(k3_tc_kernel<17, 6, 2, 1, VU>, pl.C, a, pl, P, st);
+        return pl.rs == 2 ? k3_launch_k(k3_tc_kernel<11, 3, 3, 2, VU>, pl.C, a, pl, P, st)
+                          : k3_launch_k(k3_tc_kernel<11, 3, 3, 1, VU>, pl.C, a, pl, P, st);
     }
     switch (pl.C) {
-        case 1: return k3_launch_c<1>(a, pl, P, st);
-        case 2: return k3_launch_c<2>(a, pl, P, st);
-        case 4: return k3_launch_c<4>(a, pl, P, st);
-        case 8: return k3_launch_c<8>(a, pl, P, st);
-        case 16: return k3_launch_c<16>(a, pl, P, st);
+        case 1: return k3_launch_c<1, VU>(a, pl, P, st);
+        case 2: return k3_launch_c<2, VU>(a, pl, P, st);
+        case 4: return k3_launch_c<4, VU>(a, pl, P, st);
+        case 8: return k3_launch_c<8, VU>(a, pl, P, st);
+        case 16: return k3_launch_c<16, VU>(a, pl, P, st);
     }
     set_error("ppo: bad cluster %d", pl.C);
     return PGM_ERR_ARG;
+}
+
+template <bool VU>
+static int k3_launch_tcw(const K3Args &a, const TwExtra &x, const K3Plan &pl, int P, cudaStream_t st) {
+    if (pl.rs == 4) return k3_launch_w(k3_tcw_kernel<376, 17, 2, 4, VU>, a, x, pl, P, st);
+    if (pl.rs == 2) return k3_launch_w(k3_tcw_kernel<376, 17, 2, 2, VU>, a, x, pl, P, st);
+    return k3_launch_w(k3_tcw_kernel<376, 17, 2, 1, VU>, a, x, pl, P, st);
 }
 
 static int sm_count(int &sms) {
@@ -932,9 +945,7 @@ static int ppo_common(float *params, float *adam_m, float *adam_v, int32_t *adam
         PGM_CUDA(cudaGetLastError());
         // features O+1 .. 383 of the last W1 block image are never written by the kernel: they must be zero, not stale bytes
         PGM_CUDA(cudaMemsetAsync(ws + pl.off_w1img, 0, (size_t)P * 2 * TW_NB * 8192 * sizeof(__half), st));
-        if (pl.rs == 4) return k3_launch_w(k3_tcw_kernel<376, 17, 2, 4>, a, x, pl, P, st);
-        if (pl.rs == 2) return k3_launch_w(k3_tcw_kernel<376, 17, 2, 2>, a, x, pl, P, st);
-        return k3_launch_w(k3_tcw_kernel<376, 17, 2, 1>, a, x, pl, P, st);
+        return pl.vu ? k3_launch_tcw<true>(a, x, pl, P, st) : k3_launch_tcw<false>(a, x, pl, P, st);
     }
     {
         const size_t total = (size_t)P * S * pl.RSG;
@@ -946,7 +957,7 @@ static int ppo_common(float *params, float *adam_m, float *adam_v, int32_t *adam
     }
     // padding entries of the gradient slots are never written by the kernel: keep them zero
     PGM_CUDA(cudaMemsetAsync(ws + pl.off_gpart, 0, (size_t)P * 2 * (pl.G + 1) * pl.NHP * sizeof(float), st));
-    return k3_launch(a, pl, P, st);
+    return pl.vu ? k3_launch<true>(a, pl, P, st) : k3_launch<false>(a, pl, P, st);
 }
 
 extern "C" int pgm_ppo_update_f32(float *params, float *adam_m, float *adam_v, int32_t *adam_step, const double *lr,

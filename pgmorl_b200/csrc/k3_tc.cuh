@@ -68,7 +68,7 @@ constexpr uint32_t TC_D1 = 0, TC_D2 = 64, TC_ACC = 128, TC_GSTRIDE = 192, TC_GW2
 #define TCT(i)
 #endif
 
-template <int O, int A, int M, int RS>      // RS = CTAs per network half (row split): 1 or 2
+template <int O, int A, int M, int RS, bool VU = false>      // RS = CTAs per network half (row split): 1 or 2
 __global__ void __launch_bounds__(TC_THREADS, 1) k3_tc_kernel(const K3Args a) {
     constexpr int OP = (O + 3) / 4 * 4;
     constexpr int NK1 = (O + 1 + 15) / 16;           // K steps of layer 1: x, ones column at index O, zero padding
@@ -458,7 +458,8 @@ __global__ void __launch_bounds__(TC_THREADS, 1) k3_tc_kernel(const K3Args a) {
                             const float dlt = V - vo;
                             const float vcl = vo + fminf(fmaxf(dlt, -clip), clip);
                             const float ea = V - R, eb = vcl - R;
-                            const float la = ea * ea, lb = eb * eb;
+                            // unclipped value loss (VU): lb = -1 < 0 <= la, so max(la, lb) = la and wa = 1, gradient 2 * ea exactly
+                            const float la = ea * ea, lb = VU ? -1.f : eb * eb;
                             const float wa = la > lb ? 1.f : (la == lb ? 0.5f : 0.f);
                             const float pas = (dlt >= -clip && dlt <= clip) ? 1.f : 0.f;
                             if (row_valid) { loss_val += fmaxf(la, lb); go = vscale * (wa * 2.f * ea + (1.f - wa) * 2.f * eb * pas); }

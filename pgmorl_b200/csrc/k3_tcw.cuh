@@ -110,7 +110,7 @@ struct TwExtra {          // wide-path buffers inside the workspace
     float *pmv;           // [P][2 halves][master | m | v][NHP]
 };
 
-template <int O, int A, int M, int RS>
+template <int O, int A, int M, int RS, bool VU = false>
 __global__ void __launch_bounds__(TC_THREADS, 1) k3_tcw_kernel(const K3Args a, const TwExtra x) {
     constexpr int NHP = tw_nhp(O, A);
     constexpr int KHP = 24;                              // head outputs handled per row (A <= 24)
@@ -506,7 +506,8 @@ __global__ void __launch_bounds__(TC_THREADS, 1) k3_tcw_kernel(const K3Args a, c
                         const float dlt = V - vo;
                         const float vcl = vo + fminf(fmaxf(dlt, -clip), clip);
                         const float ea = V - R, eb = vcl - R;
-                        const float la = ea * ea, lb = eb * eb;
+                        // unclipped value loss (VU): lb = -1 < 0 <= la, so max(la, lb) = la and wa = 1, gradient 2 * ea exactly
+                        const float la = ea * ea, lb = VU ? -1.f : eb * eb;
                         const float wa = la > lb ? 1.f : (la == lb ? 0.5f : 0.f);
                         const float pas = (dlt >= -clip && dlt <= clip) ? 1.f : 0.f;
                         if (row_valid) { loss_val += fmaxf(la, lb); go = vscale * (wa * 2.f * ea + (1.f - wa) * 2.f * eb * pas); }

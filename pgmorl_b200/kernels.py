@@ -9,6 +9,8 @@ from ._nvtx import rng as _nvtx
 from .layout import NetDims
 
 ACT_SAMPLE, ACT_DETERMINISTIC, ACT_EVALUATE = 0, 1, 2
+RET_GAE, RET_PROPER_TIME_LIMITS = 1, 2        # mode bits of pgm_returns_adv_f32
+PPO_VALUE_UNCLIPPED = 0x10000                 # flag OR-ed into K3's `cluster`: value loss without the clip
 
 
 def _stream():
@@ -86,6 +88,30 @@ def gae_adv(rewards, value, masks, bad_masks, gamma, lam, weights=None, obj_var=
     return returns, adv
 
 
+def returns_adv(rewards, value, masks, bad_masks, gamma, lam, use_gae=True, use_proper_time_limits=True, weights=None,
+                obj_var=None, boot=None, out=None):
+    """K2 with the branch of RolloutStorage.compute_returns chosen by use_gae / use_proper_time_limits (storage.py:77-116).
+    Shapes as gae_adv; boot [P,N,M] = bootstrap value of the n-step branches (None: value row T; the GAE branches always
+    bootstrap from value row T). Returns (returns [P,T,N,M], adv [P,T,N] or None); adv = normalised scalarisation of
+    returns - value[:T]."""
+    for n, t in (("rewards", rewards), ("value", value), ("masks", masks), ("bad_masks", bad_masks),
+                 ("weights", weights), ("obj_var", obj_var), ("boot", boot)):
+        _f32c(t, n)
+    P, T, N, M = rewards.shape
+    assert value.shape == (P, T + 1, N, M) and masks.shape == (P, T + 1, N) and bad_masks.shape == (P, T + 1, N)
+    assert boot is None or boot.shape == (P, N, M)
+    if out is not None:
+        returns, adv = out
+    else:
+        returns = torch.empty_like(rewards)
+        adv = torch.empty(P, T, N, device=rewards.device, dtype=torch.float32) if weights is not None else None
+    mode = (RET_GAE if use_gae else 0) | (RET_PROPER_TIME_LIMITS if use_proper_time_limits else 0)
+    check(lib().pgm_returns_adv_f32(ptr(rewards), ptr(value), ptr(boot), ptr(masks), ptr(bad_masks), ptr(weights),
+                                    ptr(obj_var), float(gamma), float(lam), mode, ptr(returns), ptr(adv), P, T, N, M,
+                                    _stream()))
+    return returns, adv
+
+
 def ppo_workspace(P, S, dims: NetDims, device, cluster=0):
     n = lib().pgm_ppo_workspace_bytes(P, S, dims.obs, dims.act, dims.obj, cluster)
     return torch.empty(n + 256, dtype=torch.uint8, device=device)
@@ -97,10 +123,12 @@ def _aligned(ws):
 
 
 def ppo_update(params, adam_m, adam_v, adam_step, lr, obs, action, logp_old, value_old, returns, adv, perm,
-               num_mini_batch, dims: NetDims, hyper: PpoHyper = None, workspace=None, cluster=0, losses=None):
+               num_mini_batch, dims: NetDims, hyper: PpoHyper = None, workspace=None, cluster=0, losses=None,
+               clipped_value_loss=True):
     """K3. In place on params/adam_m/adam_v [P,n_par] and adam_step [P] int32.
     obs [P,>=S,O] / value_old [P,>=S,M] may carry the extra T+1 slot (only the first S rows are read);
     action [P,S,A]; logp_old, adv [P,S]; returns [P,S,M]; perm int32 [P or 1,E,S]; lr float64 [P].
+    clipped_value_loss=False: value loss 0.5 * mean((V - R)^2) (PPO(use_clipped_value_loss=False), ppo.py:86-94).
     Returns losses [P,3] = (value_loss, action_loss, entropy) averaged over the E*B updates."""
     P, S, A = action.shape
     for n, t in (("params", params), ("adam_m", adam_m), ("adam_v", adam_v), ("obs", obs), ("action", action),
@@ -120,14 +148,15 @@ def ppo_update(params, adam_m, adam_v, adam_step, lr, obs, action, logp_old, val
     check(lib().pgm_ppo_update_f32(
         ptr(params), ptr(adam_m), ptr(adam_v), ptr(adam_step), ptr(lr), ptr(obs), obs.stride(0), ptr(action),
         ptr(logp_old), ptr(value_old), value_old.stride(0), ptr(returns), ptr(adv), ptr(perm),
-        int(perm.shape[0] == 1 and P > 1), E, num_mini_batch, C.byref(hyper), ptr(losses), wp, wn, cluster,
-        P, S, dims.obs, dims.act, dims.obj, _stream()))
+        int(perm.shape[0] == 1 and P > 1), E, num_mini_batch, C.byref(hyper), ptr(losses), wp, wn,
+        cluster if clipped_value_loss else cluster | PPO_VALUE_UNCLIPPED, P, S, dims.obs, dims.act, dims.obj, _stream()))
     return losses
 
 
 def ppo_grad(params, obs, action, logp_old, value_old, returns, adv, idx, dims: NetDims, hyper=None,
-             cluster=0):
-    """Verification aid: un-clipped gradient [P,n_par] and losses [P,3] of one minibatch `idx` (int32 [mb])."""
+             cluster=0, clipped_value_loss=True):
+    """Verification aid: gradient [P,n_par] (before the grad-norm clip) and losses [P,3] of one minibatch `idx`
+    (int32 [mb]); clipped_value_loss as in ppo_update."""
     P, S, A = action.shape
     hyper = hyper or PpoHyper()
     ws = ppo_workspace(P, S, dims, params.device, cluster)
@@ -136,7 +165,8 @@ def ppo_grad(params, obs, action, logp_old, value_old, returns, adv, idx, dims: 
     losses = torch.empty(P, 3, device=params.device, dtype=torch.float32)
     check(lib().pgm_ppo_grad_f32(ptr(params), ptr(obs), obs.stride(0), ptr(action), ptr(logp_old), ptr(value_old),
                                  value_old.stride(0), ptr(returns), ptr(adv), ptr(idx), idx.numel(),
-                                 C.byref(hyper), ptr(grad), ptr(losses), wp, wn, cluster, P, S, dims.obs, dims.act,
+                                 C.byref(hyper), ptr(grad), ptr(losses), wp, wn,
+                                 cluster if clipped_value_loss else cluster | PPO_VALUE_UNCLIPPED, P, S, dims.obs, dims.act,
                                  dims.obj, _stream()))
     return grad, losses
 

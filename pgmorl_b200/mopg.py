@@ -199,19 +199,23 @@ def MOPG_worker(args, task_id, task, device, iteration, num_updates, start_time,
 _POP_CACHE = {}
 
 
-def _population(dims, P, args, hyper, dev, cluster):
-    """The device-resident population shard of this (shape, size, schedule): rollout buffers, K3 workspace, pinned staging
-    and the captured per-step graphs are allocated ONCE and reused by every generation (SURVEY 8(f1))."""
+def _population(dims, P, args, hyper, dev, cluster, clipped_value_loss=True):
+    """The device-resident population shard of this (shape, size, schedule, PPO options): rollout buffers, K3 workspace,
+    pinned staging and the captured per-step graphs are allocated ONCE and reused by every generation (SURVEY 8(f1)).
+    The return branch is args.use_gae / args.use_proper_time_limits (default: GAE with proper time limits, as the
+    reference's run.py:56-70 sets them)."""
     from .rollout import StepPipe
+    use_gae, use_ptl = bool(getattr(args, "use_gae", True)), bool(getattr(args, "use_proper_time_limits", True))
     key = (dims, P, args.num_steps, args.num_processes, args.ppo_epoch, args.num_mini_batch, args.gamma, args.gae_lambda,
-           str(dev), cluster)
+           str(dev), cluster, use_gae, use_ptl, bool(clipped_value_loss))
     hit = _POP_CACHE.get(key)
     if hit is None:
         if len(_POP_CACHE) >= 4:                       # a run alternates between at most a few shard sizes
             _POP_CACHE.pop(next(iter(_POP_CACHE)))
         pop = PopulationMOPG(dims, P, args.num_steps, args.num_processes, ppo_epoch=args.ppo_epoch,
                              num_mini_batch=args.num_mini_batch, gamma=args.gamma, gae_lambda=args.gae_lambda,
-                             hyper=hyper, device=dev, cluster=cluster)
+                             hyper=hyper, device=dev, cluster=cluster, use_gae=use_gae, use_proper_time_limits=use_ptl,
+                             clipped_value_loss=bool(clipped_value_loss))
         hit = _POP_CACHE[key] = {"pop": pop, "pipe": StepPipe(pop), "raw": None}
     hit["pop"].hyper = hyper
     return hit
@@ -314,7 +318,7 @@ def mopg_population_update(args, task_batch, device, iteration, num_updates, sta
     g0 = ag0.optimizer.param_groups[0]
     hyper = PpoHyper(ag0.clip_param, ag0.value_loss_coef, ag0.entropy_coef, ag0.max_grad_norm, g0["betas"][0],
                      g0["betas"][1], g0["eps"])
-    cache = _population(dims, P, args, hyper, dev, cluster)
+    cache = _population(dims, P, args, hyper, dev, cluster, ag0.use_clipped_value_loss)
     pop, pipe = cache["pop"], cache["pipe"]
     envs_all = []
     raw_mode = _HOOKS["make_raw_vec_envs"] is not None

@@ -22,10 +22,15 @@ from .layout import NetDims
 
 class PopulationMOPG:
     def __init__(self, dims: NetDims, P, T, N, ppo_epoch=10, num_mini_batch=32, gamma=0.995, gae_lambda=0.95,
-                 hyper: PpoHyper = None, device="cuda", cluster=0, shared_rng=True):
+                 hyper: PpoHyper = None, device="cuda", cluster=0, shared_rng=True, use_gae=True,
+                 use_proper_time_limits=True, clipped_value_loss=True):
         self.dims, self.P, self.T, self.N = dims, P, T, N
         self.E, self.B = ppo_epoch, num_mini_batch
         self.gamma, self.lam = gamma, gae_lambda
+        # branch of compute_returns (storage.py:77-116; the n-step branches bootstrap from value row T, where K1 puts the
+        # value of the last observation) and PPO's use_clipped_value_loss
+        self.use_gae, self.use_proper_time_limits = use_gae, use_proper_time_limits
+        self.clipped_value_loss = clipped_value_loss
         self.hyper = hyper or PpoHyper()
         self.device = torch.device(device)
         self.cluster = cluster
@@ -88,14 +93,23 @@ class PopulationMOPG:
             K.policy_forward(self.params, self.obs, d, eps=self.eps, rows_a=self.S,
                              out=(self.value, self.action, self.logp))
         with _nvtx("mopg.k2_gae_adv"):
-            K.gae_adv(self.rewards, self.value.view(P, T + 1, N, d.obj), self.masks, self.bad_masks, self.gamma,
-                      self.lam, weights=self.weights, obj_var=self.obj_var, out=(self.returns, self.adv))
+            self._returns_adv()
         with _nvtx("mopg.k3_ppo_update"):
-            K.ppo_update(self.params, self.adam_m, self.adam_v, self.adam_step, self.lr, self.obs, self.action,
-                         self.logp, self.value, self.returns.view(P, self.S, d.obj), self.adv.view(P, self.S),
-                         self.perm, self.B, d, hyper=self.hyper, workspace=self.workspace, cluster=self.cluster,
-                         losses=self.losses)
+            self._ppo_update()
         return self.losses
+
+    def _returns_adv(self):
+        T, N, P, d = self.T, self.N, self.P, self.dims
+        K.returns_adv(self.rewards, self.value.view(P, T + 1, N, d.obj), self.masks, self.bad_masks, self.gamma, self.lam,
+                      use_gae=self.use_gae, use_proper_time_limits=self.use_proper_time_limits, weights=self.weights,
+                      obj_var=self.obj_var, out=(self.returns, self.adv))
+
+    def _ppo_update(self):
+        P, d = self.P, self.dims
+        K.ppo_update(self.params, self.adam_m, self.adam_v, self.adam_step, self.lr, self.obs, self.action,
+                     self.logp, self.value, self.returns.view(P, self.S, d.obj), self.adv.view(P, self.S),
+                     self.perm, self.B, d, hyper=self.hyper, workspace=self.workspace, cluster=self.cluster,
+                     losses=self.losses, clipped_value_loss=self.clipped_value_loss)
 
     GPU_LAUNCHES_PER_STEP = 4   # K1 forward, K2 GAE/adv, K3 record pack, K3 PPO
 
@@ -154,13 +168,8 @@ class PopulationMOPG:
 
     def update_only(self):
         """K2 + K3 on the rollout already in the buffers."""
-        T, N, P, d = self.T, self.N, self.P, self.dims
-        K.gae_adv(self.rewards, self.value.view(P, T + 1, N, d.obj), self.masks, self.bad_masks, self.gamma,
-                  self.lam, weights=self.weights, obj_var=self.obj_var, out=(self.returns, self.adv))
-        K.ppo_update(self.params, self.adam_m, self.adam_v, self.adam_step, self.lr, self.obs, self.action,
-                     self.logp, self.value, self.returns.view(P, self.S, d.obj), self.adv.view(P, self.S),
-                     self.perm, self.B, d, hyper=self.hyper, workspace=self.workspace, cluster=self.cluster,
-                     losses=self.losses)
+        self._returns_adv()
+        self._ppo_update()
         return self.losses
 
     def upload(self, obs, rewards, masks, bad_masks, eps, perm):
