@@ -139,9 +139,11 @@ int pgm_gae_adv_f32(const float *rewards, const float *value, const float *masks
  *   perm [P or 1, E, S] int32 : minibatch b of epoch e = perm[e, b*mb:(b+1)*mb], mb = S / B
  *   losses [P,3] out: mean over E*B updates of (value_loss, action_loss, entropy)
  *   workspace: >= pgm_ppo_workspace_bytes(...) bytes, 256-byte aligned
- *   cluster: 1,2,4,8,16 = CTAs per task of the FP32 FFMA kernels; 32 / 64 = the tensor-core kernel (tcgen05 UMMA on FP16
- *            operand pairs, FP32 accumulate, FP32-level accuracy) with 2 / 4 CTAs per task, built for the (O,A,M)
- *            shapes (17,6,2) and (11,3,3); 0 = choose from P, the shape and the SM count (tensor cores from 8 tasks on).
+ *   cluster: 1,2,4,8,16 = CTAs per task of the FP32 FFMA kernels (O <= 384, A <= 32, M <= 16 at 2..16; cluster 1 keeps
+ *            both halves in one CTA and refuses shapes whose halves need more than 227 KB together, e.g. Humanoid's);
+ *            32 / 64 = the tensor-core kernel (tcgen05 UMMA on FP16 operand pairs, FP32 accumulate, FP32-level
+ *            accuracy) with 2 / 4 CTAs per task, built for the (O,A,M) shapes (17,6,2) and (11,3,3); 0 = choose
+ *            from P, the shape and the SM count (tensor cores from 8 tasks on).
  *            Tensor-core operand ranges: |obs| < 65 504 (unscaled fp16 pairs), |parameter| < 255.9, |backward signal| < 16;
  *            beyond them the task's outputs become inf / NaN (non-saturating conversions), never a silently clamped result.
  *            OR-able flags 0x100 / 0x200 / 0x400 / 0x800 / 0x1000 / 0x2000 / 0x4000 select the step tail of the FFMA cluster

@@ -183,10 +183,13 @@ def ppo_grad(net, x, action, logp_old, v_old, ret, adv, clip=0.2, vcoef=0.5, eco
     return g, (value_loss, action_loss, ent)
 
 
-def clip_and_adam(p, g, m, v, step, lr, max_grad_norm=0.5, beta1=0.9, beta2=0.999, eps=1e-5):
+def clip_and_adam(p, g, m, v, step, lr, max_grad_norm=0.5, beta1=0.9, beta2=0.999, eps=1e-5, norms=None):
     """clip_grad_norm_ (coef = min(1, max/(norm+1e-6)), always multiplied) then one Adam
-    step in torch's _single_tensor_adam arithmetic. In place on p, m, v; returns step+1."""
+    step in torch's _single_tensor_adam arithmetic. In place on p, m, v; returns step+1.
+    `norms`, if a list, receives the gradient norm before clipping."""
     total = math.sqrt(float((g * g).sum()))
+    if norms is not None:
+        norms.append(total)
     coef = min(1.0, max_grad_norm / (total + 1e-6))
     g = g * coef
     step += 1
@@ -202,9 +205,10 @@ def clip_and_adam(p, g, m, v, step, lr, max_grad_norm=0.5, beta1=0.9, beta2=0.99
 
 def ppo_update(flat, m, v, step, lr, dims, obs, action, logp, value, returns, adv, perm,
                num_mini_batch, clip=0.2, vcoef=0.5, ecoef=0.0, max_grad_norm=0.5,
-               adam_eps=1e-5):
+               adam_eps=1e-5, beta1=0.9, beta2=0.999, norms=None):
     """algo/ppo.py:62-115. obs [T+1,N,O] etc.; perm int [E, T*N]. In place on flat/m/v.
-    Returns (step, (value_loss, action_loss, entropy) averaged over E*B updates)."""
+    Returns (step, (value_loss, action_loss, entropy) averaged over E*B updates).
+    `norms`, if a list, receives each step's gradient norm before clipping."""
     O, A, M = dims
     net = Net(flat, O, A, M)
     T, N = action.shape[0], action.shape[1]
@@ -221,7 +225,7 @@ def ppo_update(flat, m, v, step, lr, dims, obs, action, logp, value, returns, ad
             idx = perm[e, b * mb:(b + 1) * mb]
             g, losses = ppo_grad(net, X[idx], ACT[idx], LP[idx], VO[idx], RET[idx], ADV[idx],
                                  clip, vcoef, ecoef)
-            step = clip_and_adam(flat, g, m, v, step, lr, max_grad_norm, eps=adam_eps)
+            step = clip_and_adam(flat, g, m, v, step, lr, max_grad_norm, beta1, beta2, adam_eps, norms)
             sums += losses
     return step, tuple(sums / (perm.shape[0] * num_mini_batch))
 

@@ -747,16 +747,23 @@ static int k3_plan(K3Plan &pl, int P, int S, int mb, int O, int A, int M, int cl
         // step tail: default from K3_DEFAULT_TAIL; others on request (cluster flags, or PGM_K3_TAIL=0|1|2 in the
         // environment for whole-program A/B runs)
         static const int env_tail = [] { const char *e = getenv("PGM_K3_TAIL"); return (e && e[0] >= '0' && e[0] <= '6') ? e[0] - '0' : -1; }();
-        pl.tail = tail0 ? 0 : (tail2 ? 1 : (tailmc ? 2 : (tailgl ? 3 : (tailbp ? 4 : (tailnb ? 5 : (tailep ? 6 : (env_tail >= 0 ? env_tail : K3_DEFAULT_TAIL)))))));
-        if (pl.tail == 1 && !(pl.G >= 2 && k3_fast_smem_bytes(L, pl.TM, pl.RSS, pl.NHP, pl.stage_floats, pl.G, true) <= 227 * 1024))
-            pl.tail = 0;
-        if (pl.tail >= 2 && pl.G < 2) pl.tail = 0;
-        if (pl.tail >= 4 && k3_fast_smem_bytes(L, pl.TM, pl.RSS, pl.NHP, pl.stage_floats, pl.G, false, false, true) > 227 * 1024)
-            pl.tail = 2;
-        pl.smem = k3_fast_smem_bytes(L, pl.TM, pl.RSS, pl.NHP, pl.stage_floats, pl.G, pl.tail == 1, pl.tail == 3, pl.tail >= 4);
-    } else {
-        pl.smem = k3_smem_bytes(L, C, pl.TM, pl.DB, pl.RSS);
+        const int want = tail0 ? 0 : (tail2 ? 1 : (tailmc ? 2 : (tailgl ? 3 : (tailbp ? 4 : (tailnb ? 5 : (tailep ? 6 : (env_tail >= 0 ? env_tail : K3_DEFAULT_TAIL)))))));
+        // one CTA per half (C = 2) keeps a whole half resident: with TM = 4 that exceeds 227 KB at wider shapes (Ant,
+        // (27,8,2): 237 664 B). Fall back to TM = 2, then to the generic double-buffered kernel below.
+        for (;;) {
+            pl.tail = want;
+            if (pl.tail == 1 && !(pl.G >= 2 && k3_fast_smem_bytes(L, pl.TM, pl.RSS, pl.NHP, pl.stage_floats, pl.G, true) <= 227 * 1024))
+                pl.tail = 0;
+            if (pl.tail >= 2 && pl.G < 2) pl.tail = 0;
+            if (pl.tail >= 4 && k3_fast_smem_bytes(L, pl.TM, pl.RSS, pl.NHP, pl.stage_floats, pl.G, false, false, true) > 227 * 1024)
+                pl.tail = 2;
+            pl.smem = k3_fast_smem_bytes(L, pl.TM, pl.RSS, pl.NHP, pl.stage_floats, pl.G, pl.tail == 1, pl.tail == 3, pl.tail >= 4);
+            if (pl.smem <= 227 * 1024 || pl.TM == 2) break;
+            pl.TM = 2; pl.RC = 32; pl.Rg = round_up(rows, pl.RC);
+        }
+        if (pl.smem > 227 * 1024) { pl.fast = false; pl.stage_floats = 0; pl.tail = 0; }
     }
+    if (!pl.fast) pl.smem = k3_smem_bytes(L, C, pl.TM, pl.DB, pl.RSS);
     PGM_REQUIRE(pl.smem <= 227 * 1024, "ppo: configuration needs %zu B of shared memory (O=%d, cluster=%d)", pl.smem, O, C);
     size_t off = 0;
     auto seg = [&](size_t bytes) { size_t o = off; off += (bytes + 255) / 256 * 256; return o; };

@@ -52,10 +52,14 @@ def param_layout(d):
     return out, off
 
 
-# Named environment shapes from the reference's launch scripts (SURVEY.md section 8).
+# Named environment shapes from the reference's launch scripts (SURVEY.md section 8). Ant's 27 observations are qpos[2:]
+# and qvel of the reference's environments/ant.py, without contact forces.
 ENV_SHAPES = {
     "walker2d": NetDims(17, 6, 2),
     "halfcheetah": NetDims(17, 6, 2),
+    "hopper2": NetDims(11, 3, 2),
     "hopper3": NetDims(11, 3, 3),
+    "ant": NetDims(27, 8, 2),
+    "swimmer": NetDims(8, 2, 2),
     "humanoid": NetDims(376, 17, 2),
 }

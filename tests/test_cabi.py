@@ -49,6 +49,20 @@ def test_n_par_matches_python_layout(library):
     for d in ENV_SHAPES.values():
         assert library.pgm_n_par(d.obs, d.act, d.obj) == d.n_par
     assert library.pgm_n_par(17, 6, 2) == 11150 and library.pgm_n_par(376, 17, 2) == 57828
+    # Hopper-v2, Ant, Swimmer (the reference's other launch scripts)
+    assert library.pgm_n_par(11, 3, 2) == 10184 and library.pgm_n_par(27, 8, 2) == 12562 and library.pgm_n_par(8, 2, 2) == 9734
+
+
+def test_offsets_of_the_other_reference_shapes(library):
+    """Hopper-v2, Ant and Swimmer: offsets of the 13 tensors, written out (critic head and actor head start right after
+    the two 64-wide halves; their sizes follow M and A)."""
+    import ctypes
+    want = {(11, 3, 2): [0, 704, 768, 4864, 4928, 5632, 5696, 9792, 9856, 9984, 9986, 10178, 10181],
+            (27, 8, 2): [0, 1728, 1792, 5888, 5952, 7680, 7744, 11840, 11904, 12032, 12034, 12546, 12554],
+            (8, 2, 2): [0, 512, 576, 4672, 4736, 5248, 5312, 9408, 9472, 9600, 9602, 9730, 9732]}
+    for (O, A, M), offs in want.items():
+        out = (ctypes.c_int * 13)()
+        assert library.pgm_param_offsets(O, A, M, out) == 0 and list(out) == offs
 
 
 def test_tensor_offsets_match_python_layout(library):

@@ -15,7 +15,12 @@ from tests.helpers import rel_err
 
 pytestmark = pytest.mark.gpu
 
-DIMS = {"walker": NetDims(17, 6, 2), "hopper3": NetDims(11, 3, 3), "humanoid": NetDims(376, 17, 2)}
+DIMS = {"walker": NetDims(17, 6, 2), "hopper3": NetDims(11, 3, 3), "humanoid": NetDims(376, 17, 2),
+        "hopper2": NetDims(11, 3, 2), "ant": NetDims(27, 8, 2), "swimmer": NetDims(8, 2, 2),
+        # test-only shapes at the edges of the K3 planner (tests/test_gpu_shapes.py)
+        "s16_16_2": NetDims(16, 16, 2), "s48_16_16": NetDims(48, 16, 16), "s45_16_3": NetDims(45, 16, 3),
+        "s60_6_2": NetDims(60, 6, 2), "s64_4_4": NetDims(64, 4, 4), "s33_17_2": NetDims(33, 17, 2)}
+TC_SHAPES = ("walker", "hopper3", "humanoid")      # shapes with tensor-core K3 kernels (cluster 32 / 64 / 128)
 
 
 def dev(x, dtype=torch.float32):
@@ -49,7 +54,11 @@ def make_case(d, P, T, N, seed):
                                          # >= 1024 rows: the tensor-core forward (csrc/k1_tc.cuh), ragged last tile
                                          ("walker", 2, 301, 4), ("hopper3", 3, 613, 2),
                                          # Humanoid, >= 1024 rows: the wide tensor-core forward (csrc/k1_tcw.cuh)
-                                         ("humanoid", 2, 150, 8), ("humanoid", 20, 140, 8)])
+                                         ("humanoid", 2, 150, 8), ("humanoid", 20, 140, 8),
+                                         # shapes without a tensor-core forward at >= 1024 rows: the FFMA kernel, several
+                                         # chunks per CTA (8 x 2049 x 4 rows at Ant dims), ragged last chunk
+                                         ("ant", 8, 2048, 4), ("hopper2", 2, 300, 4), ("swimmer", 3, 613, 2),
+                                         ("s48_16_16", 2, 260, 4)])
 @pytest.mark.parametrize("shared_eps", [True, False])
 def test_k1_rollout_matches_oracle(name, P, T, N, shared_eps):
     from pgmorl_b200 import kernels as K
@@ -68,7 +77,8 @@ def test_k1_rollout_matches_oracle(name, P, T, N, shared_eps):
         assert rel_err(logp[p].cpu().numpy().reshape(T, N), ref[p]["logp"]) < 2e-5
 
 
-@pytest.mark.parametrize("name,T", [("walker", 40), ("walker", 300), ("humanoid", 300)])    # 300 x 4 rows: tensor-core forwards
+@pytest.mark.parametrize("name,T", [("walker", 40), ("walker", 300), ("humanoid", 300),    # 300 x 4 rows: tensor-core forwards
+                                    ("ant", 300), ("swimmer", 40)])
 def test_k1_modes(name, T):
     from pgmorl_b200 import kernels as K
     d = DIMS[name]
@@ -185,10 +195,14 @@ def _ppo_inputs(d, P, T, N, seed):
 
 # 32 / 64 / 128 = tensor-core paths (tcgen05): 2 / 4 / 8 CTAs per task; csrc/k3_tc.cuh (Walker2d, Hopper-v3 shapes),
 # csrc/k3_tcw.cuh (Humanoid: layer 1 streamed in 64-feature blocks)
-@pytest.mark.parametrize("cluster", [1, 2, 4, 8, 16, 32, 64, 128])
+@pytest.mark.parametrize("cluster", [1, 2, 4, 8, 16, 32, 64, 128, 0])
 @pytest.mark.parametrize("name,P,T,N,mb", [("walker", 2, 64, 4, 256), ("walker", 1, 30, 4, 100),
                                             ("hopper3", 2, 48, 2, 64), ("humanoid", 1, 32, 8, 96),
-                                            ("humanoid", 2, 64, 8, 512), ("humanoid", 1, 40, 8, 300)])
+                                            ("humanoid", 2, 64, 8, 512), ("humanoid", 1, 40, 8, 300),
+                                            ("hopper2", 2, 64, 4, 256), ("ant", 2, 64, 4, 256), ("swimmer", 2, 64, 4, 256),
+                                            ("s16_16_2", 2, 64, 4, 256), ("s48_16_16", 2, 64, 4, 256),
+                                            ("s45_16_3", 2, 64, 4, 256), ("s60_6_2", 2, 64, 4, 256),
+                                            ("s64_4_4", 2, 64, 4, 256), ("s33_17_2", 2, 64, 4, 256)])
 def test_k3_gradient_matches_oracle(name, P, T, N, mb, cluster):
     from pgmorl_b200 import kernels as K
     d = DIMS[name]
@@ -198,6 +212,8 @@ def test_k3_gradient_matches_oracle(name, P, T, N, mb, cluster):
         pytest.skip("8 CTAs per task exist on the wide-observation tensor-core path only")
     if name == "humanoid" and cluster == 16:
         pytest.skip("16-CTA clusters are a plan of the small-network FFMA kernel only")
+    if name not in TC_SHAPES and cluster in (32, 64):
+        pytest.skip("the tensor-core kernels are instantiated for the Walker2d, Hopper-v3 and Humanoid shapes only")
     cur, pk, perm = _ppo_inputs(d, P, T, N, seed=11)
     S = T * N
     idx = np.random.RandomState(0).permutation(S)[:mb]
@@ -217,17 +233,26 @@ def test_k3_gradient_matches_oracle(name, P, T, N, mb, cluster):
 
 
 @pytest.mark.parametrize("cluster", [0, 1, 2, 4, 8, 16, 32, 64])
-@pytest.mark.parametrize("name,P,T,N,B", [("walker", 3, 64, 4, 4), ("hopper3", 2, 48, 2, 3), ("walker", 2, 160, 4, 2)])
+@pytest.mark.parametrize("name,P,T,N,B", [("walker", 3, 64, 4, 4), ("hopper3", 2, 48, 2, 3), ("walker", 2, 160, 4, 2),
+                                          ("hopper2", 2, 64, 4, 2), ("ant", 3, 64, 4, 2), ("swimmer", 2, 64, 4, 2),
+                                          ("s16_16_2", 2, 64, 4, 2), ("s45_16_3", 2, 128, 4, 2), ("s60_6_2", 2, 64, 4, 2),
+                                          ("s33_17_2", 2, 64, 4, 2),
+                                          # 40 tasks: the auto plan keeps two CTAs per task (Ant: TM = 2 fallback)
+                                          ("ant", 40, 32, 4, 1)])
 def test_k3_update_matches_oracle(name, P, T, N, B, cluster):
     from pgmorl_b200 import kernels as K
     d = DIMS[name]
+    if name not in TC_SHAPES and cluster in (32, 64):
+        pytest.skip("the tensor-core kernels are instantiated for the Walker2d, Hopper-v3 and Humanoid shapes only")
+    if P > 3 and cluster != 0:
+        pytest.skip("the large population runs the auto plan only")
     cur, pk, perm = _ppo_inputs(d, P, T, N, seed=13)
     S = T * N
     rng = np.random.RandomState(2)
     m0 = rng.randn(P, d.n_par) * 1e-3
     v0 = rng.rand(P, d.n_par) * 1e-5
-    step0 = np.array([0, 7, 640][:P], dtype=np.int32)
-    lr = np.array([3e-4, 2.5e-4, 1e-4][:P])
+    step0 = np.resize(np.array([0, 7, 640], dtype=np.int32), P)
+    lr = np.resize(np.array([3e-4, 2.5e-4, 1e-4]), P)
     gp, gm, gv = dev(cur), dev(m0), dev(v0)
     gstep = dev(step0, torch.int32)
     losses = K.ppo_update(gp, gm, gv, gstep, dev(lr, torch.float64), dev(pk["obs"]), dev(pk["action"]),
@@ -297,7 +322,10 @@ TAILEP = 0x4000   # TAILNB + the W2-only gradient slices are pushed right after 
 
 
 @pytest.mark.parametrize("cluster", [4, 8, 16])
-@pytest.mark.parametrize("name,P,T,N,B", [("walker", 3, 64, 4, 4), ("hopper3", 2, 48, 2, 3), ("walker", 2, 512, 4, 8)])
+@pytest.mark.parametrize("name,P,T,N,B", [("walker", 3, 64, 4, 4), ("hopper3", 2, 48, 2, 3), ("walker", 2, 512, 4, 8),
+                                          # phase-C plans of the fast kernel the named shapes above do not reach
+                                          ("hopper2", 2, 64, 4, 1), ("ant", 2, 64, 4, 1), ("swimmer", 2, 64, 4, 1),
+                                          ("s16_16_2", 2, 64, 4, 1), ("s48_16_16", 2, 64, 4, 1)])
 def test_k3_step_tails_bit_identical(name, P, T, N, B, cluster):
     """The alternative step tails (two-barrier tail with whole-half Adam in every CTA; TMA multicast parameter broadcast)
     perform the same operations in the same order as the three-barrier sliced tail: parameters, moments and losses are
@@ -415,12 +443,13 @@ def test_population_iterations_match_reference_goldens(name):
             assert rel_err(losses[p], z[pre + "losses"]) < 1e-3
 
 
-@pytest.mark.parametrize("cluster", [8, 32, 64])
-def test_k3_per_task_permutations_equal_shared(cluster):
+@pytest.mark.parametrize("name,cluster", [pytest.param("walker", c, id=str(c)) for c in (8, 32, 64)] +
+                         [("ant", 2), ("ant", 16), ("s45_16_3", 8), ("s33_17_2", 4), ("swimmer", 1)])
+def test_k3_per_task_permutations_equal_shared(name, cluster):
     """perm given per task ([P,E,S]) with identical rows must reproduce the shared-permutation ([1,E,S]) result bit for bit
     (the reference seeds every worker alike, mopg.py:96, but the C ABI accepts per-task streams)."""
     from pgmorl_b200 import kernels as K
-    d = DIMS["walker"]
+    d = DIMS[name]
     P, T, N, B = 3, 96, 4, 2                       # mb = 192: two row tiles on the tensor-core path, the second one ragged
     cur, pk, perm = _ppo_inputs(d, P, T, N, seed=17)
     res = []

@@ -15,11 +15,9 @@ from oracle import mopg_oracle as orc
 from pgmorl_b200 import synthetic
 from pgmorl_b200.layout import NetDims
 from tests.helpers import rel_err
-from tests.test_gpu_kernels import TAIL0, TAIL2, TAILBP, TAILEP, TAILGL, TAILMC, TAILNB, make_case
+from tests.test_gpu_kernels import DIMS, TAIL0, TAIL2, TAILBP, TAILEP, TAILGL, TAILMC, TAILNB, make_case
 
 pytestmark = pytest.mark.gpu
-
-DIMS = {"walker": NetDims(17, 6, 2), "hopper3": NetDims(11, 3, 3), "humanoid": NetDims(376, 17, 2)}
 
 
 def dev(x, dtype=torch.float32):
@@ -89,7 +87,8 @@ def _unclipped_inputs(d, P, T, N, seed):
 
 
 K3_CASES = [("walker", c) for c in (1, 2, 4, 8, 16, 32, 64)] + [("hopper3", c) for c in (1, 2, 4, 8, 16, 32, 64)] + \
-           [("humanoid", c) for c in (8, 32, 64, 128)]
+           [("humanoid", c) for c in (8, 32, 64, 128)] + \
+           [("s45_16_3", c) for c in (2, 4, 8)] + [("s60_6_2", 16), ("ant", 2), ("s33_17_2", 1)]   # generic DB, TM = 2 fallback, big
 
 
 @pytest.mark.parametrize("name,cluster", K3_CASES)
