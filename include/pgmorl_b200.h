@@ -246,6 +246,11 @@ int pgm_ep_filter_f64(const double *objs, int n, int M, int32_t *keep_idx, int32
  *           Pareto-filter, then closed forms on the front sorted by objective 0.
  *   M == 3: utils.compute_hypervolume (InnerHyperVolume, morl/hypervolume.py:41-153, round(hv,4))
  *           and utils.compute_sparsity (morl/utils.py:87-100) of the given front (all coords >= 0).
+ *   M == 4: the same two functions (hypervolume.py:41-153 with its stored volumes / areas and area-reuse
+ *           flags, utils.py:87-100); points with a negative coordinate are left out of the hypervolume as
+ *           hypervolume.py:55-61 does. At most 2 202 points (the scorer's 93 bytes of shared memory per
+ *           point within 200 KB), else an error.
+ *   M >= 5 or M < 2: error.
  * workspace >= pgm_select_workspace_bytes(n, 1, M, 1). */
 int pgm_front_metrics_f64(const double *pts, int n, int M, double *out, void *workspace,
                           size_t workspace_bytes, void *stream);
@@ -260,7 +265,12 @@ int pgm_front_metrics_f64(const double *pts, int n, int M, double *out, void *wo
  * virtual front, written to front_out [E+num_tasks, M] (both optional / may be NULL).
  * 3 objectives: every candidate of a round is scored on top of the round's shared base front (sorted lists, slice areas
  * and the head of the hypervolume sum are built once per round in the workspace); the per-candidate scratch of
- * 97 * (E + num_tasks + 1) bytes must fit 200 KB of shared memory (archive fronts up to ~2 100 points), else an error. */
+ * 97 * (E + num_tasks + 1) bytes must fit 200 KB of shared memory (archive fronts up to ~2 100 points), else an error.
+ * 4 objectives (update_ep utils.py:42-65, hypervolume.py:41-153, compute_sparsity utils.py:87-100): one CTA per
+ * candidate replays the reference's 4-D dimension sweep, stored level-2 volumes / areas and area-reuse flags included;
+ * the per-candidate scratch of 93 * (E + num_tasks + 1) bytes must fit 200 KB of shared memory
+ * (E + num_tasks + 1 <= 2 202), else an error. M >= 5: error.
+ * pgm_select_workspace_bytes covers M = 2, 3 and 4. */
 size_t pgm_select_workspace_bytes(int E, int C, int M, int num_tasks);
 int pgm_select_greedy_f64(const double *ep, int E, const double *cand, int C, int M, double alpha,
                           int num_tasks, int32_t *best_ids, double *hv, double *sparsity,

@@ -583,9 +583,279 @@ __device__ inline void update_front_3d_block(const double *f, int n, const doubl
     __syncthreads();
 }
 
+// ---- 4 objectives ---------------------------------------------------------------------------------
+// update_ep (utils.py:42-65) at 4 objectives by all threads of one CTA; the same steps as update_front_3d_block.
+__device__ inline void update_front_4d_block(const double *f, int n, const double *p, double *out, int *count_out, int *flags,
+                                             int *wtot) {
+    __shared__ int s_on, s_pos;
+    const int tid = threadIdx.x, nt = blockDim.x;
+    const double p0 = p[0], p1 = p[1], p2 = p[2], p3 = p[3];
+    if (p0 < 0.0 || p1 < 0.0 || p2 < 0.0 || p3 < 0.0) {
+        for (int i = tid; i < 4 * n; i += nt) out[i] = f[i];
+        if (tid == 0) *count_out = n;
+        __syncthreads();
+        return;
+    }
+    if (tid == 0) { s_on = 1; s_pos = INT_MAX; }
+    __syncthreads();
+    for (int i = tid; i < n; i += nt) {
+        const double *q = f + 4 * i;
+        if (q[0] >= p0 - 1e-5 && q[1] >= p1 - 1e-5 && q[2] >= p2 - 1e-5 && q[3] >= p3 - 1e-5 &&
+            (q[0] > p0 + 1e-5 || q[1] > p1 + 1e-5 || q[2] > p2 + 1e-5 || q[3] > p3 + 1e-5))
+            s_on = 0;                                            // benign race: every writer stores 0
+        flags[i] = (p0 >= q[0] && p1 >= q[1] && p2 >= q[2] && p3 >= q[3]) ? 0 : 1;
+    }
+    __syncthreads();
+    const int m = block_excl_scan(flags, n, wtot);
+    const bool on = s_on != 0;
+    if (on)
+        for (int i = tid; i < n; i += nt) {
+            const double *q = f + 4 * i;
+            if (!(p0 >= q[0] && p1 >= q[1] && p2 >= q[2] && p3 >= q[3]) && p0 < q[0]) atomicMin(&s_pos, flags[i]);
+        }
+    __syncthreads();
+    const int pos = min(s_pos, m);
+    for (int i = tid; i < n; i += nt) {
+        const double *q = f + 4 * i;
+        if (p0 >= q[0] && p1 >= q[1] && p2 >= q[2] && p3 >= q[3]) continue;
+        const int dst = flags[i] + ((on && flags[i] >= pos) ? 1 : 0);
+        out[4 * dst] = q[0]; out[4 * dst + 1] = q[1]; out[4 * dst + 2] = q[2]; out[4 * dst + 3] = q[3];
+    }
+    if (tid == 0) {
+        if (on) { out[4 * pos] = p0; out[4 * pos + 1] = p1; out[4 * pos + 2] = p2; out[4 * pos + 3] = p3; }
+        *count_out = m + (on ? 1 : 0);
+    }
+    __syncthreads();
+}
+
+// 2-D area (hvRecursive at dimIndex 1, hypervolume.py:92-105) of the points of the 4-D sweep that are in list 1 while
+// slice (k, t) is computed: objective-3 rank <= k and objective-2 rank <= t. hx, hy, h2, h3: coordinates 0 and 1 and
+// the ranks 2 and 3 of the points in list-1 order.
+__device__ __forceinline__ double slice_area_4d(const double *hx, const double *hy, const int *h2, const int *h3, int n,
+                                                int k, int t) {
+    double h = 0.0, acc = 0.0, prevy = 0.0;
+    bool first = true;
+#pragma unroll 4
+    for (int u = 0; u < n; ++u) {
+        const double x = hx[u], y = hy[u];
+        if (h3[u] > k || h2[u] > t) continue;
+        if (first) { h = x; prevy = y; first = false; }
+        else {
+            acc = dadd(acc, dmul(h, dsub(prevy, y)));
+            if (x < h) h = x;
+            prevy = y;
+        }
+    }
+    return dadd(acc, dmul(h, prevy));
+}
+
+// One CTA per candidate: L = update_ep(front, p); hv = round4(InnerHyperVolume(L)); sp = compute_sparsity(L), at 4
+// objectives (use_cand = 0: L = the front itself, for pgm_front_metrics_f64).
+//
+// The hypervolume is hvRecursive (hypervolume.py:106-153) from dimIndex 3, restated without the linked lists but with
+// the same float64 operations in the same order (tests/hv_ref.py keeps the lists; the two are compared bit for bit):
+//  * The FPL lists only ever hold the points of the preProcess order that are currently inserted, in that order. At
+//    level 3 the points enter in list-3 order; while point k of list 3 is processed, list 2 holds the points of
+//    objective-3 rank <= k, and while the level-2 call processes the point at list-2 position t, list 1 holds those
+//    of objective-2 rank <= t as well. So each level-1 call is slice_area_4d(k, t).
+//  * Level 2 keeps the reference's state across calls: bounds[2] (lowered by every level-3 reinsert, set by every
+//    level-2 reinsert), the stored volume[2] / area[2] of every point, and the ignore flags. A call first walks down
+//    from the top of list 2 as the removal loop does, resumes its volume from the stored state of the point below the
+//    first one it keeps, and takes area[2] from the predecessor for points whose flag is 2 or 3 ("ignore >= 2")
+//    instead of calling level 1. Only the flags below 2 are ever reset, and none exist, so flags persist.
+//  * bounds[0] and bounds[1] never rise above -1e308 and no level reads them; level 3 runs once, so its flag reset and
+//    its own reuse branch never fire (a point's flag is 0 when level 3 reaches it: it was outside every earlier list).
+// The level-1 calls of one level-2 call depend only on the point set, so they run in parallel (one thread per slice);
+// the walk that strings them together -- volume chain, area reuse, flags -- is serial on thread 0.
+//
+// Dynamic shared memory (score4d_smem): 8 * nmax doubles, 7 * nmax ints, nmax flag bytes.
+__global__ void __launch_bounds__(256) k5_score4d_kernel(SelState st, int buf, const double *__restrict__ cand, int C,
+                                                         double *__restrict__ hv, double *__restrict__ sp, int nmax,
+                                                         int use_cand) {
+    extern __shared__ __align__(16) unsigned char smraw[];
+    const int c = blockIdx.x, tid = threadIdx.x, nt = blockDim.x;
+    if (use_cand) {
+        if (*st.done || !st.mask[c]) {
+            if (tid == 0) { hv[c] = 0.0; sp[c] = 0.0; }
+            return;
+        }
+    }
+    double *c0 = reinterpret_cast<double *>(smraw), *c1 = c0 + nmax, *c2 = c1 + nmax, *c3 = c2 + nmax;
+    double *hx = c3 + nmax, *hy = hx + nmax, *area2 = hy + nmax, *vol2 = area2 + nmax;
+    int *pos = reinterpret_cast<int *>(vol2 + nmax), *r2 = pos + nmax, *r3 = r2 + nmax, *l2 = r3 + nmax, *l3 = l2 + nmax,
+        *h2 = l3 + nmax, *h3 = h2 + nmax;
+    unsigned char *flag = reinterpret_cast<unsigned char *>(h3 + nmax);
+    double *cd[4] = {c0, c1, c2, c3};
+    __shared__ int s_on_ep, s_n, s_ins, s_qt, s_qp, s_len;
+
+    const double *f = st.front[buf];
+    const int n0 = st.count[buf];
+    double p[4] = {0.0, 0.0, 0.0, 0.0};
+    bool p_valid = false;
+    if (use_cand) {
+        p[0] = cand[4 * c]; p[1] = cand[4 * c + 1]; p[2] = cand[4 * c + 2]; p[3] = cand[4 * c + 3];
+        p_valid = p[0] >= 0.0 && p[1] >= 0.0 && p[2] >= 0.0 && p[3] >= 0.0;
+    }
+    if (tid == 0) { s_on_ep = 1; s_ins = 0; }
+    __syncthreads();
+    // ---- update_ep: keep flags (pos[i] = 1 if kept), on_ep, insertion index ----
+    for (int i = tid; i < n0; i += nt) {
+        const double *q = f + 4 * i;
+        bool keep = true;
+        if (p_valid) {
+            keep = !(p[0] >= q[0] && p[1] >= q[1] && p[2] >= q[2] && p[3] >= q[3]);
+            if (q[0] >= p[0] - 1e-5 && q[1] >= p[1] - 1e-5 && q[2] >= p[2] - 1e-5 && q[3] >= p[3] - 1e-5 &&
+                (q[0] > p[0] + 1e-5 || q[1] > p[1] + 1e-5 || q[2] > p[2] + 1e-5 || q[3] > p[3] + 1e-5))
+                s_on_ep = 0;                                     // benign race: every writer stores 0
+        }
+        pos[i] = keep ? 1 : 0;
+    }
+    __syncthreads();
+    if (tid == 0) {
+        const bool ins = p_valid && s_on_ep;
+        int m = 0, ip = -1;
+        for (int i = 0; i < n0; ++i) {
+            if (pos[i]) {
+                if (ins && ip < 0 && p[0] < f[4 * i]) { ip = m; ++m; }   // p goes before the first kept q with p0 < q0
+                pos[i] = m; ++m;
+            } else pos[i] = -1;
+        }
+        if (ins && ip < 0) { ip = m; ++m; }
+        s_n = m; s_ins = ins ? ip : -1;
+    }
+    __syncthreads();
+    const int n = s_n, ins = s_ins;
+    for (int i = tid; i < n0; i += nt)
+        if (pos[i] >= 0) {
+#pragma unroll
+            for (int d = 0; d < 4; ++d) cd[d][pos[i]] = -f[4 * i + d];
+        }
+    if (tid == 0 && ins >= 0) {
+#pragma unroll
+        for (int d = 0; d < 4; ++d) cd[d][ins] = -p[d];
+    }
+    __syncthreads();
+    if (n == 0) {
+        if (tid == 0) { hv[c] = 0.0; sp[c] = 0.0; }
+        return;
+    }
+    // ---- utils.compute_sparsity: per dimension the ascending values (hx as scratch), one running sum on thread 0 ----
+    double s = 0.0;
+#pragma unroll
+    for (int d = 0; d < 4; ++d) {
+        const double *v = cd[d];
+        for (int i = tid; i < n; i += nt) {
+            const double vi = -v[i];
+            int r = 0;
+            for (int j = 0; j < n; ++j) { const double vj = -v[j]; r += (vj < vi || (vj == vi && j < i)) ? 1 : 0; }
+            hx[r] = vi;
+        }
+        __syncthreads();
+        if (tid == 0)
+            for (int i = 1; i < n; ++i) { const double g = dsub(hx[i], hx[i - 1]); s = dadd(s, dmul(g, g)); }
+        __syncthreads();
+    }
+    // ---- the points that weakly dominate the reference point (hypervolume.py:55-61), compacted in order ----
+    if (tid == 0) {
+        sp[c] = n >= 2 ? s / (double)(n - 1) : 0.0;
+        int m = 0;
+        for (int i = 0; i < n; ++i)
+            if (c0[i] <= 0.0 && c1[i] <= 0.0 && c2[i] <= 0.0 && c3[i] <= 0.0) {
+                c0[m] = c0[i]; c1[m] = c1[i]; c2[m] = c2[i]; c3[m] = c3[i]; ++m;
+            }
+        s_n = m;
+    }
+    __syncthreads();
+    const int nh = s_n;
+    if (nh == 0) {
+        if (tid == 0) hv[c] = 0.0;
+        return;
+    }
+    // ---- preProcess (hypervolume.py:156-164): successive stable sorts by objectives 0, 1, 2, 3 ----
+    for (int i = tid; i < nh; i += nt) {
+        const double xi = c0[i], yi = c1[i], zi = c2[i], wi = c3[i];
+        int ry = 0, rz = 0, rw = 0;
+        for (int j = 0; j < nh; ++j) {
+            const double xj = c0[j], yj = c1[j], zj = c2[j], wj = c3[j];
+            const bool xlt = xj < xi || (xj == xi && j < i);                    // key (x, input position)
+            const bool ylt = yj < yi || (yj == yi && xlt);                       // key (y, x, input position)
+            const bool zlt = zj < zi || (zj == zi && ylt);                       // key (z, y, x, input position)
+            const bool wlt = wj < wi || (wj == wi && zlt);                       // key (w, z, y, x, input position)
+            ry += ylt; rz += zlt; rw += wlt;
+        }
+        r2[i] = rz; r3[i] = rw; l2[rz] = i; l3[rw] = i;
+        hx[ry] = xi; hy[ry] = yi; h2[ry] = rz; h3[ry] = rw;
+        flag[i] = 0; area2[i] = 0.0; vol2[i] = 0.0;
+    }
+    __syncthreads();
+    // ---- the sweep; thread 0 holds bounds[2], the level-3 volume and the previous level-3 area ----
+    double B = -1.0e308, hv3 = 0.0, a3prev = 0.0;
+    for (int k = 0; k < nh; ++k) {
+        if (tid == 0) {
+            const int pk = l3[k];
+            if (k > 0) {
+                hv3 = dadd(hv3, dmul(a3prev, dsub(c3[pk], c3[l3[k - 1]])));
+                if (B > c2[pk]) B = c2[pk];                                     // reinsert(p, 3, bounds)
+            }
+            // level-2 removal loop: from the top of list 2 down while q > bound or its predecessor >= bound
+            int t = nh - 1;
+            while (r3[l2[t]] > k) --t;
+            int tp = t - 1;
+            while (tp >= 0 && r3[l2[tp]] > k) --tp;
+            int len = k + 1;
+            while (len > 1 && (c2[l2[t]] > B || c2[l2[tp]] >= B)) {
+                t = tp;
+                --tp;
+                while (tp >= 0 && r3[l2[tp]] > k) --tp;
+                --len;
+            }
+            s_qt = t; s_qp = tp; s_len = len;
+        }
+        __syncthreads();
+        // level-1 calls of this level-2 call, for the points that will not take their predecessor's area
+        for (int t = s_qt + tid; t < nh; t += nt) {
+            const int j = l2[t];
+            if (r3[j] <= k && flag[j] < 2) area2[j] = slice_area_4d(hx, hy, h2, h3, nh, k, t);
+        }
+        __syncthreads();
+        if (tid == 0) {
+            const int qt = s_qt, qp = s_qp;
+            int q = l2[qt];
+            double hvol = 0.0;
+            if (s_len > 1) {
+                const int pq = l2[qp];
+                hvol = dadd(vol2[pq], dmul(area2[pq], dsub(c2[q], c2[pq])));
+            }
+            vol2[q] = hvol;
+            double aprev = qp >= 0 ? area2[l2[qp]] : 0.0;                      // the sentinel's area is 0
+            if (flag[q] >= 2) area2[q] = aprev;
+            else if (area2[q] <= aprev) flag[q] = 2;
+            for (int t = qt + 1; t < nh; ++t) {
+                const int pt = l2[t];
+                if (r3[pt] > k) continue;
+                hvol = dadd(hvol, dmul(area2[q], dsub(c2[pt], c2[q])));
+                B = c2[pt];                                                      // bounds[dimIndex] = pCargoDimIndex
+                aprev = area2[q];
+                q = pt;
+                vol2[q] = hvol;
+                if (flag[q] >= 2) area2[q] = aprev;
+                else if (area2[q] <= aprev) flag[q] = 2;
+            }
+            hvol = dsub(hvol, dmul(area2[q], c2[q]));
+            // level 3: area[3] of point k; ignore = 3 when it did not grow (read by the later level-2 calls)
+            if (hvol <= a3prev) flag[l3[k]] = 3;
+            a3prev = hvol;
+        }
+    }
+    if (tid == 0) {
+        hv3 = dsub(hv3, dmul(a3prev, c3[l3[nh - 1]]));
+        hv[c] = round4(hv3);
+    }
+}
+
 // ---- arg-max + virtual EP update: single CTA ---------------------------------------------------------
 // 3 objectives: dynamic shared memory of base3d_smem(nmax) bytes (first used as nmax ints by the front update); the new
-// front's base data for the next round's scorer is built here.
+// front's base data for the next round's scorer is built here. 4 objectives: nmax ints for the front update.
 template <int M>
 __global__ void __launch_bounds__(1024) k5_pick_kernel(SelState st, int buf, const double *__restrict__ cand, int C,
                                                        const double *__restrict__ hv, const double *__restrict__ sp,
@@ -633,6 +903,9 @@ __global__ void __launch_bounds__(1024) k5_pick_kernel(SelState st, int buf, con
                                   reinterpret_cast<int *>(pick_smem), wtot);
             base3d_build(st.front[buf ^ 1], st.count[buf ^ 1], nmax, st.b3, pick_smem);
         }
+        if (M == 4 && s_bi >= 0)
+            update_front_4d_block(st.front[buf], st.count[buf], cand + 4 * s_bi, st.front[buf ^ 1], &st.count[buf ^ 1],
+                                  reinterpret_cast<int *>(pick_smem), wtot);
     } else if (tid == 0) *best_out = -1;
     if (s_copy) {      // no pick this round: carry the front over so the buffers keep alternating
         const int n = st.count[buf];
@@ -698,6 +971,9 @@ static size_t sel_carve(SelState &st, char *ws, int E, int C, int M, int num_tas
 
 static size_t score3d_smem(int nmax) { return (size_t)nmax * (4 * sizeof(double) + 5 * sizeof(int)); }
 static size_t score3d_inc_smem(int nmax) { return (size_t)nmax * (9 * sizeof(double) + 6 * sizeof(int) + 1) + 16; }
+static size_t score4d_smem(int nmax) { return (size_t)nmax * (8 * sizeof(double) + 7 * sizeof(int) + 1); }
+// Largest front (points of L = update_ep(front, p)) the 4-D scorer's shared-memory layout holds: 2 202 points.
+constexpr size_t SCORE4D_SMEM_MAX = 200 * 1024;
 
 }  // namespace pgm
 
@@ -731,7 +1007,7 @@ extern "C" int pgm_select_greedy_f64(const double *ep, int E, const double *cand
                                      int num_tasks, int32_t *best_ids, double *hv, double *sparsity, double *front_out,
                                      int32_t *n_front, void *workspace, size_t workspace_bytes, void *stream) {
     PGM_REQUIRE((ep || E == 0) && (cand || C == 0) && best_ids && hv && sparsity && workspace, "pgm_select_greedy_f64: null pointer");
-    PGM_REQUIRE(M == 2 || M == 3, "pgm_select_greedy_f64: exact hypervolume is implemented for 2 and 3 objectives (got %d)", M);
+    PGM_REQUIRE(M >= 2 && M <= 4, "pgm_select_greedy_f64: exact hypervolume is implemented for 2 to 4 objectives (got %d)", M);
     PGM_REQUIRE(E >= 0 && C >= 0 && num_tasks >= 1, "pgm_select_greedy_f64: bad sizes E=%d C=%d num_tasks=%d", E, C, num_tasks);
     PGM_REQUIRE(((uintptr_t)workspace & 255) == 0, "pgm_select_greedy_f64: workspace must be 256-byte aligned");
     SelState st;
@@ -746,6 +1022,12 @@ extern "C" int pgm_select_greedy_f64(const double *ep, int E, const double *cand
         PGM_CUDA(cudaFuncSetAttribute(k5_base3d_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smemb));
         PGM_CUDA(cudaFuncSetAttribute(k5_pick_kernel<3>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smemb));
     }
+    const size_t smem4 = score4d_smem(nmax), smemp4 = (size_t)nmax * sizeof(int);
+    if (M == 4) {
+        PGM_REQUIRE(smem4 <= SCORE4D_SMEM_MAX, "pgm_select_greedy_f64: front of %d points exceeds the 4-D scorer's shared memory "
+                    "(at most %d points: archive + num_tasks + 1)", nmax, (int)(SCORE4D_SMEM_MAX / score4d_smem(1)));
+        PGM_CUDA(cudaFuncSetAttribute(k5_score4d_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem4));
+    }
     {
         const int nthr = (E * M > C ? E * M : C) + 1;
         k5_init_kernel<<<(nthr + 255) / 256, 256, 0, s>>>(st, ep, E, M, C);
@@ -756,10 +1038,12 @@ extern "C" int pgm_select_greedy_f64(const double *ep, int E, const double *cand
         double *hv_r = hv + (size_t)r * C, *sp_r = sparsity + (size_t)r * C;
         if (C > 0) {
             if (M == 2) k5_score2d_kernel<<<(C + 127) / 128, 128, 0, s>>>(st, buf, cand, C, hv_r, sp_r);
-            else k5_score3d_inc_kernel<<<C, S3_THREADS, smem3, s>>>(st, buf, cand, C, hv_r, sp_r, nmax);
+            else if (M == 3) k5_score3d_inc_kernel<<<C, S3_THREADS, smem3, s>>>(st, buf, cand, C, hv_r, sp_r, nmax);
+            else k5_score4d_kernel<<<C, 256, smem4, s>>>(st, buf, cand, C, hv_r, sp_r, nmax, 1);
         }
         if (M == 2) k5_pick_kernel<2><<<1, 1024, 0, s>>>(st, buf, cand, C, hv_r, sp_r, alpha, best_ids + r, nmax);
-        else k5_pick_kernel<3><<<1, 1024, smemb, s>>>(st, buf, cand, C, hv_r, sp_r, alpha, best_ids + r, nmax);
+        else if (M == 3) k5_pick_kernel<3><<<1, 1024, smemb, s>>>(st, buf, cand, C, hv_r, sp_r, alpha, best_ids + r, nmax);
+        else k5_pick_kernel<4><<<1, 1024, smemp4, s>>>(st, buf, cand, C, hv_r, sp_r, alpha, best_ids + r, nmax);
     }
     k5_finish_kernel<<<8, 256, 0, s>>>(st, num_tasks & 1, M, front_out, n_front);
     PGM_CUDA(cudaGetLastError());
@@ -769,7 +1053,7 @@ extern "C" int pgm_select_greedy_f64(const double *ep, int E, const double *cand
 extern "C" int pgm_front_metrics_f64(const double *pts, int n, int M, double *out, void *workspace,
                                      size_t workspace_bytes, void *stream) {
     PGM_REQUIRE(out && workspace && (pts || n == 0), "pgm_front_metrics_f64: null pointer");
-    PGM_REQUIRE(M == 2 || M == 3, "pgm_front_metrics_f64: implemented for 2 and 3 objectives (got %d)", M);
+    PGM_REQUIRE(M >= 2 && M <= 4, "pgm_front_metrics_f64: implemented for 2 to 4 objectives (got %d)", M);
     PGM_REQUIRE(((uintptr_t)workspace & 255) == 0, "pgm_front_metrics_f64: workspace must be 256-byte aligned");
     cudaStream_t s = (cudaStream_t)stream;
     SelState st;
@@ -785,6 +1069,13 @@ extern "C" int pgm_front_metrics_f64(const double *pts, int n, int M, double *ou
         k5_dominance_kernel<2><<<blocks, 256, 0, s>>>(pts, n, (int *)(keep_idx + n));
         k5_rank_kernel<2><<<blocks, 256, 0, s>>>(pts, n, (int *)(keep_idx + n), keep_idx, n_keep);
         k5_metrics2d_kernel<<<1, 32, 0, s>>>(pts, keep_idx, n_keep, out);
+    } else if (M == 4) {
+        const size_t smem4 = score4d_smem(n);
+        PGM_REQUIRE(smem4 <= SCORE4D_SMEM_MAX, "pgm_front_metrics_f64: %d points exceed the 4-D scorer's shared memory (at most %d)",
+                    n, (int)(SCORE4D_SMEM_MAX / score4d_smem(1)));
+        PGM_CUDA(cudaFuncSetAttribute(k5_score4d_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem4));
+        k5_init_kernel<<<(n * M + 256) / 256, 256, 0, s>>>(st, pts, n, M, 0);
+        k5_score4d_kernel<<<1, 256, smem4, s>>>(st, 0, nullptr, 1, out, out + 1, n, 0);
     } else {
         const int nmax = n + 2;
         const size_t smem3 = score3d_smem(nmax);

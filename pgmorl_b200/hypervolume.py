@@ -1,12 +1,15 @@
 """Exact hypervolume indicator with the reference's interface (morl/hypervolume.py:23-74).
 
 The reference implements variant 3 of the Fonseca-Paquete-Lopez-Ibanez dimension sweep with linked
-lists; for the 2 and 3 objectives PG-MORL uses, it reduces to a sorted sweep / z-slices of 2-D areas.
-`compute` runs that on the GPU (csrc/k5_select.cu) in float64 with the reference's summation order
-and returns `round(hv, 4)` like hypervolume.py:74."""
+lists; for 2 and 3 objectives it reduces to a sorted sweep / z-slices of 2-D areas, and at 4 objectives
+the kernel replays the sweep's stored volumes, areas and area-reuse flags. `compute` runs it on the GPU
+(csrc/k5_select.cu) in float64 with the reference's operations and order and returns `round(hv, 4)`
+like hypervolume.py:74. The device kernels stop at 4 objectives (MAX_OBJECTIVES)."""
 import numpy as np
 
 from . import kernels as K
+
+MAX_OBJECTIVES = 4
 
 
 class InnerHyperVolume:
@@ -23,8 +26,8 @@ class InnerHyperVolume:
         if len(pts) == 0:
             return 0.0
         M = pts.shape[1]
-        if M == 3:
+        if M in (3, 4):
             return K.front_metrics(pts)[0]
         if M == 2:
             return round(K.front_metrics(pts)[0], 4)
-        raise NotImplementedError("InnerHyperVolume: device kernels cover 2 and 3 objectives")
+        raise NotImplementedError(f"InnerHyperVolume: device kernels cover 2 to {MAX_OBJECTIVES} objectives (got {M})")

@@ -204,7 +204,10 @@ def ep_filter(objs):
 
 
 def front_metrics(pts):
-    """(hypervolume, sparsity) of a point set: Population2d semantics for M=2, utils.* for M=3."""
+    """(hypervolume, sparsity) of a point set: Population2d semantics for M=2 (get_ep_indices first, hypervolume not
+    rounded); for M=3 and M=4 utils.compute_hypervolume (InnerHyperVolume, round(hv, 4)) and utils.compute_sparsity of
+    the points as given. M=4 leaves points with a negative coordinate out of the hypervolume, as InnerHyperVolume does;
+    M=3 expects none. At most 2 202 points at M=4 (the 4-D scorer's shared memory); more raise."""
     if len(pts) == 0:
         return 0.0, 0.0
     d = _dev_f64(pts)

@@ -34,11 +34,14 @@ def get_ep_indices(obj_batch_input):
 
 def update_ep(ep_objs_batch, new_objs):
     """Fold one point into a front with the reference's 1e-5 tolerances (utils.py:42-65); the front stays
-    ordered by objective 0. Runs the same device routine the 3-objective greedy selection uses."""
+    ordered by objective 0. Runs the same device routine the 3- and 4-objective greedy selection uses."""
+    from .hypervolume import MAX_OBJECTIVES
     new_objs = np.asarray(new_objs, dtype=np.float64)
     M = len(new_objs)
-    if M != 3:
-        raise NotImplementedError("update_ep: the reference calls it for 3 objectives only; so does the kernel")
+    if M > MAX_OBJECTIVES:
+        raise NotImplementedError(f"update_ep: the device kernels cover at most {MAX_OBJECTIVES} objectives (got {M})")
+    if M < 3:
+        raise NotImplementedError("update_ep: the reference calls it for 3 or more objectives only; so does the kernel")
     ep = np.asarray(ep_objs_batch, dtype=np.float64).reshape(-1, M)
     front = K.select_greedy(ep, new_objs[None, :], 0.0, 1)[3]      # one candidate, one round: it is folded in
     return [row.copy() for row in front]
@@ -68,11 +71,15 @@ def compute_hypervolume(ep_objs_batch):
 
 def compute_sparsity(ep_objs_batch):
     """Per-dimension sorted squared gaps / (n - 1) (utils.py:87-100)."""
+    from .hypervolume import MAX_OBJECTIVES
     if len(ep_objs_batch) < 2:
         return 0.0
     pts = np.asarray(ep_objs_batch, dtype=np.float64)
-    if pts.shape[1] != 3:
-        raise NotImplementedError("compute_sparsity: the device kernel covers 3 objectives (2 objectives use "
+    if pts.shape[1] > MAX_OBJECTIVES:
+        raise NotImplementedError(f"compute_sparsity: the device kernels cover at most {MAX_OBJECTIVES} objectives "
+                                  f"(got {pts.shape[1]})")
+    if pts.shape[1] not in (3, 4):
+        raise NotImplementedError("compute_sparsity: the device kernel covers 3 and 4 objectives (2 objectives use "
                                   "Population.compute_sparsity)")
     return K.front_metrics(pts)[1]
 
