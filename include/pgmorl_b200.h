@@ -18,7 +18,12 @@
  *     asynchronous w.r.t. the host unless stated;
  *   - return value 0 = success, otherwise an error code; pgm_last_error()
  *     gives the message of the last failure on the calling thread.
- *   - hidden width is fixed at 64 (a2c/model.py:202 default, warm_up.py:34-38).
+ *   - hidden width: 64 (a2c/model.py:202 default, warm_up.py:34-38) in every entry point without a `hidden`
+ *     argument; the *_h entry points take it explicitly and accept 32, 64 and 128 (MLPBase(hidden_size=...)).
+ *     Any other width is an error. Width 64 runs the same kernels as the entry points without `hidden`; 32 and 128 run
+ *     the FP32 FFMA kernels only (K1's FFMA forward, K3's generic cluster kernel at 2..16 CTAs per task).
+ *     Shared memory bounds the observation width: at 128 one network half of Walker2d's shape is about 80 KB and
+ *     Humanoid (O = 376, 194 KB for W1 alone) fits neither K1 nor K3; at 32 every named shape fits, Humanoid included.
  */
 #ifndef PGMORL_B200_H
 #define PGMORL_B200_H
@@ -50,12 +55,15 @@ enum {
 int pgm_abi_version(void);
 const char *pgm_last_error(void);
 
-/* number of parameters of one policy (actor 64-64 + critic 64-64 + heads + logstd) */
+/* number of parameters of one policy (actor H-H + critic H-H + heads + logstd; H = 64, or `hidden` for the _h form,
+ * which returns -1 and sets pgm_last_error() for a width other than 32, 64, 128) */
 int pgm_n_par(int obs_dim, int act_dim, int obj_num);
+int pgm_n_par_h(int obs_dim, int act_dim, int obj_num, int hidden);
 /* offsets (in elements) of the 13 parameter tensors of one policy inside its flat vector, in the reference's
  * named_parameters() order: base.actor.0.{weight,bias}, base.actor.2.{weight,bias}, base.critic.0.{...}, base.critic.2.{...},
  * base.critic_linear.{weight,bias}, dist.fc_mean.{weight,bias}, dist.logstd._bias (a2c/model.py:201-256) */
 int pgm_param_offsets(int obs_dim, int act_dim, int obj_num, int *out13);
+int pgm_param_offsets_h(int obs_dim, int act_dim, int obj_num, int hidden, int *out13);
 
 /* ---------------------------------------------------------------------------
  * K1  population-batched actor-critic forward.
@@ -71,10 +79,16 @@ int pgm_param_offsets(int obs_dim, int act_dim, int obj_num, int *out13);
  *   value   [P, rows_v, M]  out ;   logp [P, rows_a] out
  * Trajectory mode: rows_v=(T+1)*N, rows_a=T*N.  Per-step mode: rows_v=rows_a=N.
  * get_value: rows_a=0.
+ * pgm_policy_forward_h_f32: the same at hidden width `hidden` (32, 64, 128). The tensor-core forwards serve width 64;
+ * 32 and 128 run on the FP32 FFMA kernel, which refuses an observation width whose parameter image exceeds 227 KB of
+ * shared memory (Humanoid at 128).
  */
 int pgm_policy_forward_f32(const float *params, const float *obs, const float *eps, int eps_shared,
                            float *action, float *value, float *logp, int mode, int P, int rows_v,
                            int rows_a, int O, int A, int M, void *stream);
+int pgm_policy_forward_h_f32(const float *params, const float *obs, const float *eps, int eps_shared,
+                             float *action, float *value, float *logp, int mode, int P, int rows_v,
+                             int rows_a, int O, int A, int M, int hidden, void *stream);
 
 /* K1 in per-step mode for real environment loops (morl/mopg.py:103-135: one Policy.act per environment step): every
  * task's N current observations -> value / sampled action / log-prob written STRAIGHT INTO time slot t of the rollout
@@ -91,6 +105,11 @@ int pgm_policy_step_f32(const float *params, const int32_t *ctl, const float *ob
                         int eps_shared, float *obs_buf, size_t obs_task_stride, float *value_buf,
                         size_t value_task_stride, float *action_buf, size_t action_task_stride, float *logp_buf,
                         size_t logp_task_stride, float *act_out, int P, int N, int O, int A, int M, void *stream);
+int pgm_policy_step_h_f32(const float *params, const int32_t *ctl, const float *obs_stage, const float *eps,
+                          int eps_shared, float *obs_buf, size_t obs_task_stride, float *value_buf,
+                          size_t value_task_stride, float *action_buf, size_t action_task_stride, float *logp_buf,
+                          size_t logp_task_stride, float *act_out, int P, int N, int O, int A, int M, int hidden,
+                          void *stream);
 
 /* ---------------------------------------------------------------------------
  * K2  vector-reward returns + scalarised, normalised advantage.
@@ -152,6 +171,11 @@ int pgm_gae_adv_f32(const float *rewards, const float *value, const float *masks
  *            (use_clipped_value_loss=False, a2c/algo/ppo.py:86-94 else branch) instead of the clipped
  *            0.5 * mean(max((V - R)^2, (V_clip - R)^2)); losses[:,0] reports the loss that was minimised.
  *   S and B must satisfy S % B < S / B (the reference's BatchSampler(drop_last=True) then yields exactly B minibatches).
+ * The _h forms take the hidden width (32, 64, 128). At 32 and 128 only the generic FFMA cluster kernel exists: cluster
+ *   0 (auto, 2..16 CTAs per task), 2, 4, 8 or 16; cluster 1 and the tensor-core values 32 / 64 / 128 are refused with an
+ *   error naming the width. A shape whose network half exceeds 227 KB of shared memory is refused (Humanoid at 128);
+ *   at 128 the observation width is also limited to O <= 128 (the register tile of dW1), at 32 to O <= 384.
+ *   At 64 they are the functions without `hidden`.
  */
 #define PGM_PPO_VALUE_UNCLIPPED 0x10000
 
@@ -165,6 +189,8 @@ typedef struct {
 } pgm_ppo_hyper;
 
 size_t pgm_ppo_workspace_bytes(int P, int S, int O, int A, int M, int cluster);
+/* 0 for an unsupported hidden width */
+size_t pgm_ppo_workspace_bytes_h(int P, int S, int O, int A, int M, int cluster, int hidden);
 
 int pgm_ppo_update_f32(float *params, float *adam_m, float *adam_v, int32_t *adam_step,
                        const double *lr, const float *obs, size_t obs_task_stride,
@@ -174,6 +200,14 @@ int pgm_ppo_update_f32(float *params, float *adam_m, float *adam_v, int32_t *ada
                        const pgm_ppo_hyper *hyper_host, float *losses, void *workspace,
                        size_t workspace_bytes, int cluster, int P, int S, int O, int A, int M,
                        void *stream);
+int pgm_ppo_update_h_f32(float *params, float *adam_m, float *adam_v, int32_t *adam_step,
+                         const double *lr, const float *obs, size_t obs_task_stride,
+                         const float *action, const float *logp_old, const float *value_old,
+                         size_t value_task_stride, const float *returns, const float *adv,
+                         const int32_t *perm, int perm_shared, int E, int B,
+                         const pgm_ppo_hyper *hyper_host, float *losses, void *workspace,
+                         size_t workspace_bytes, int cluster, int P, int S, int O, int A, int M, int hidden,
+                         void *stream);
 
 /* Debug/verification aid: gradient of one minibatch (rows idx[0..mb)) of every task,
  * before clipping; grad [P, n_par], losses [P,3]. Same device code as pgm_ppo_update_f32. */
@@ -183,6 +217,12 @@ int pgm_ppo_grad_f32(const float *params, const float *obs, size_t obs_task_stri
                      const int32_t *idx, int mb, const pgm_ppo_hyper *hyper_host, float *grad,
                      float *losses, void *workspace, size_t workspace_bytes, int cluster, int P,
                      int S, int O, int A, int M, void *stream);
+int pgm_ppo_grad_h_f32(const float *params, const float *obs, size_t obs_task_stride,
+                       const float *action, const float *logp_old, const float *value_old,
+                       size_t value_task_stride, const float *returns, const float *adv,
+                       const int32_t *idx, int mb, const pgm_ppo_hyper *hyper_host, float *grad,
+                       float *losses, void *workspace, size_t workspace_bytes, int cluster, int P,
+                       int S, int O, int A, int M, int hidden, void *stream);
 
 /* ---------------------------------------------------------------------------
  * K4  batched fit of the hyperbolic prediction model (FLOAT64, one warp per fit).

@@ -37,8 +37,12 @@ SIGNATURES = {
     "pgm_last_error": (C.c_char_p, []),
     "pgm_n_par": (_I, [_I, _I, _I]),
     "pgm_param_offsets": (_I, [_I, _I, _I, _P]),
+    "pgm_n_par_h": (_I, [_I, _I, _I, _I]),
+    "pgm_param_offsets_h": (_I, [_I, _I, _I, _I, _P]),
     "pgm_policy_forward_f32": (_I, [_P, _P, _P, _I, _P, _P, _P, _I, _I, _I, _I, _I, _I, _I, _P]),
     "pgm_policy_step_f32": (_I, [_P, _P, _P, _P, _I, _P, _Z, _P, _Z, _P, _Z, _P, _Z, _P, _I, _I, _I, _I, _I, _P]),
+    "pgm_policy_forward_h_f32": (_I, [_P, _P, _P, _I, _P, _P, _P, _I, _I, _I, _I, _I, _I, _I, _I, _P]),
+    "pgm_policy_step_h_f32": (_I, [_P, _P, _P, _P, _I, _P, _Z, _P, _Z, _P, _Z, _P, _Z, _P, _I, _I, _I, _I, _I, _I, _P]),
     "pgm_gae_adv_f32": (_I, [_P, _P, _P, _P, _P, _P, _F, _F, _P, _P, _I, _I, _I, _I, _P]),
     "pgm_returns_adv_f32": (_I, [_P, _P, _P, _P, _P, _P, _P, _F, _F, _I, _P, _P, _I, _I, _I, _I, _P]),
     "pgm_ppo_workspace_bytes": (_Z, [_I, _I, _I, _I, _I, _I]),
@@ -56,6 +60,11 @@ SIGNATURES = {
     "pgm_vecnorm_rollout_step_f64": (_I, [_P] * 16 + [_P, _Z, _P, _Z, _P, _Z, _P, _Z] + [C.c_double] * 4 + [_I] * 5 + [_P]),
     "pgm_ppo_grad_f32": (_I, [_P, _P, _Z, _P, _P, _P, _Z, _P, _P, _P, _I, C.POINTER(PpoHyper), _P, _P, _P,
                               _Z, _I, _I, _I, _I, _I, _I, _P]),
+    "pgm_ppo_workspace_bytes_h": (_Z, [_I, _I, _I, _I, _I, _I, _I]),
+    "pgm_ppo_update_h_f32": (_I, [_P, _P, _P, _P, _P, _P, _Z, _P, _P, _P, _Z, _P, _P, _P, _I, _I, _I,
+                                  C.POINTER(PpoHyper), _P, _P, _Z, _I, _I, _I, _I, _I, _I, _I, _P]),
+    "pgm_ppo_grad_h_f32": (_I, [_P, _P, _Z, _P, _P, _P, _Z, _P, _P, _P, _I, C.POINTER(PpoHyper), _P, _P, _P,
+                                _Z, _I, _I, _I, _I, _I, _I, _I, _P]),
 }
 
 

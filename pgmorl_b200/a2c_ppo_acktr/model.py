@@ -2,7 +2,8 @@
 float32 CUDA vector (order: pgmorl_b200/layout.py) and whose forward passes are K1 launches.
 
 Only the configuration PG-MORL instantiates is supported (warm_up.py:34-40): 1-D observations, Box actions,
-MOMLPBase 64-64 tanh without LayerNorm, DiagGaussian with state-independent logstd. CNN / GRU / Categorical
+MOMLPBase H-H tanh without LayerNorm (H = base_kwargs['hidden_size'], default 64; 32, 64 and 128 run on the device),
+DiagGaussian with state-independent logstd. CNN / GRU / Categorical
 bases of the upstream class are never reached by morl/ and are not provided."""
 from collections import OrderedDict
 
@@ -13,6 +14,8 @@ from .. import kernels as K
 from ..layout import NetDims, param_layout
 from ..synthetic import init_policy_flat
 
+HIDDEN_SIZES = (32, 64, 128)     # hidden widths the K1 / K3 kernels are built for (include/pgmorl_b200.h)
+
 
 class Policy:
     def __init__(self, obs_shape, action_space, base=None, base_kwargs=None, obj_num=1, device="cuda", flat=None):
@@ -20,7 +23,11 @@ class Policy:
             raise NotImplementedError("Policy: only 1-D observations with Box actions (the MO-MuJoCo configuration)")
         if base_kwargs and base_kwargs.get("layernorm", False):
             raise NotImplementedError("Policy: layernorm=True is not part of the PG-MORL configuration (warm_up.py:37)")
-        self.dims = NetDims(int(obs_shape[0]), int(action_space.shape[0]), int(obj_num))
+        hidden = int((base_kwargs or {}).get("hidden_size", 64))
+        if hidden not in HIDDEN_SIZES:
+            raise NotImplementedError(f"Policy: hidden_size={hidden} is not supported; the kernels are built for "
+                                      f"hidden_size in {{32, 64, 128}}")
+        self.dims = NetDims(int(obs_shape[0]), int(action_space.shape[0]), int(obj_num), hidden)
         self.device = torch.device(device)
         if flat is None:
             flat = init_policy_flat(self.dims)          # draws from torch's global CPU generator like the reference

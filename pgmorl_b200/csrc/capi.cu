@@ -23,14 +23,26 @@ int cuda_fail(cudaError_t e, const char *what) {
 
 extern "C" int pgm_abi_version(void) { return PGM_ABI_VERSION; }
 extern "C" const char *pgm_last_error(void) { return pgm::g_err; }
-extern "C" int pgm_n_par(int O, int A, int M) { return pgm::NetLayout(O, A, M).n_par; }
+extern "C" int pgm_n_par_h(int O, int A, int M, int hidden) {
+    if (!pgm::hidden_supported(hidden)) {
+        pgm::set_error("pgm_n_par_h: hidden width %d is not one of {32, 64, 128}", hidden);
+        return -1;
+    }
+    return pgm::NetLayout(O, A, M, hidden).n_par;
+}
+extern "C" int pgm_n_par(int O, int A, int M) { return pgm_n_par_h(O, A, M, PGM_HIDDEN); }
 
 // Offsets of the 13 parameter tensors inside one flat vector, in named_parameters() order (pgmorl_b200/layout.py):
-// the kernels and the Python state_dict slicing must agree on them (tests/test_cabi.py).
-extern "C" int pgm_param_offsets(int O, int A, int M, int *out13) {
+// the kernels and the Python state_dict slicing must agree on them (tests/test_cabi.py, tests/test_oracle_hidden.py).
+extern "C" int pgm_param_offsets_h(int O, int A, int M, int hidden, int *out13) {
     if (!out13) return PGM_ERR_ARG;
-    const pgm::NetLayout L(O, A, M);
+    if (!pgm::hidden_supported(hidden)) {
+        pgm::set_error("pgm_param_offsets_h: hidden width %d is not one of {32, 64, 128}", hidden);
+        return PGM_ERR_ARG;
+    }
+    const pgm::NetLayout L(O, A, M, hidden);
     const int v[13] = {L.oW1a, L.ob1a, L.oW2a, L.ob2a, L.oW1c, L.ob1c, L.oW2c, L.ob2c, L.oWv, L.obv, L.oWmu, L.obmu, L.ols};
     for (int i = 0; i < 13; ++i) out13[i] = v[i];
     return PGM_OK;
 }
+extern "C" int pgm_param_offsets(int O, int A, int M, int *out13) { return pgm_param_offsets_h(O, A, M, PGM_HIDDEN, out13); }

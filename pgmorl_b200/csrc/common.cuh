@@ -8,10 +8,11 @@
 
 namespace pgm {
 
-constexpr int H = PGM_HIDDEN;   // hidden width (a2c/model.py:202)
+constexpr int H = PGM_HIDDEN;   // default hidden width (a2c/model.py:202); the FFMA kernels also take 32 and 128
 constexpr int LDH = H + 4;      // smem row stride of 64-wide tiles: 68 = 4*17 -> 8 consecutive rows
                                 // at the same column land in 8 distinct 16-byte bank groups
-constexpr int NTHREADS = 256;   // every MLP kernel uses 16x16 thread tiles
+__host__ __device__ inline bool hidden_supported(int hw) { return hw == 32 || hw == 64 || hw == 128; }
+constexpr int NTHREADS = 256;   // every MLP kernel uses 256-thread CTAs (16x16 tiles at hidden width 64, net.cuh)
 
 void set_error(const char *fmt, ...);
 int cuda_fail(cudaError_t e, const char *what);
@@ -46,17 +47,18 @@ struct NetLayout {
     int oW1a, ob1a, oW2a, ob2a, oW1c, ob1c, oW2c, ob2c, oWv, obv, oWmu, obmu, ols, n_par;
     int n_base;    // W1+b1+W2+b2 of one half
     __host__ __device__ NetLayout() {}
-    __host__ __device__ NetLayout(int O_, int A_, int M_) : O(O_), A(A_), M(M_) {
+    // hw = hidden width (32, 64 or 128)
+    __host__ __device__ NetLayout(int O_, int A_, int M_, int hw = H) : O(O_), A(A_), M(M_) {
         OP = round_up(O, 4);
         ldw1 = stride4odd(OP);
-        oW1a = 0; ob1a = oW1a + H * O; oW2a = ob1a + H; ob2a = oW2a + H * H;
-        oW1c = ob2a + H; ob1c = oW1c + H * O; oW2c = ob1c + H; ob2c = oW2c + H * H;
-        oWv = ob2c + H; obv = oWv + M * H; oWmu = obv + M; obmu = oWmu + A * H;
+        oW1a = 0; ob1a = oW1a + hw * O; oW2a = ob1a + hw; ob2a = oW2a + hw * hw;
+        oW1c = ob2a + hw; ob1c = oW1c + hw * O; oW2c = ob1c + hw; ob2c = oW2c + hw * hw;
+        oWv = ob2c + hw; obv = oWv + M * hw; oWmu = obv + M; obmu = oWmu + A * hw;
         ols = obmu + A; n_par = ols + A;
-        n_base = H * O + H + H * H + H;
+        n_base = hw * O + hw + hw * hw + hw;
     }
     // half 0 = actor (base at 0, head [Wmu bmu logstd] at oWmu), half 1 = critic (contiguous)
-    __host__ __device__ int half_size(int half) const { return n_base + (half == 0 ? A * H + 2 * A : M * H + M); }
+    __host__ __device__ int half_size(int half, int hw = H) const { return n_base + (half == 0 ? A * hw + 2 * A : M * hw + M); }
     __host__ __device__ int head_dim(int half) const { return half == 0 ? A : M; }
     __host__ __device__ int half_base(int half) const { return half == 0 ? oW1a : oW1c; }
     __host__ __device__ int half_head(int half) const { return half == 0 ? oWmu : oWv; }

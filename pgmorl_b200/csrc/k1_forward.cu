@@ -29,36 +29,38 @@ __host__ __device__ inline int k1_ldo(const NetLayout &L) { return (L.A > L.M ? 
 
 // SPLIT = false: both halves resident (small networks). SPLIT = true: one half resident at a time, the CTA walks
 // its chunks once per half (wide observations, e.g. Humanoid O = 376: one half's W1 alone is 97 KB).
-__host__ inline size_t k1_smem_bytes(const NetLayout &L, int TM, bool split) {
+__host__ inline size_t k1_smem_bytes(const NetLayout &L, int TM, bool split, int hw = H) {
     const int RC = 16 * TM;
-    const size_t h0 = halfnet_smem_floats(L, 0), h1 = halfnet_smem_floats(L, 1);
+    const size_t h0 = halfnet_smem_floats(L, 0, hw), h1 = halfnet_smem_floats(L, 1, hw);
     size_t f = split ? (h0 > h1 ? h0 : h1) : h0 + h1;
     f += (size_t)RC * L.ldw1;            // x
-    f += 2 * (size_t)RC * LDH;           // h1, h2
+    f += 2 * (size_t)RC * (hw + 4);      // h1, h2
     f += 2 * (size_t)RC * k1_ldo(L);     // mean, value
     return f * sizeof(float);
 }
 
-template <int TM, bool SPLIT>
-__global__ void __launch_bounds__(NTHREADS, SPLIT ? 1 : 2) k1_forward_kernel(const K1Args a) {
-    constexpr int RC = 16 * TM;
+// HW: hidden width (32, 64, 128; net.cuh RowTile). The body is shared by k1_forward_kernel (HW = 64) and
+// k1_forward_h_kernel (HW = 32, 128).
+template <int TM, bool SPLIT, int HW>
+__device__ __forceinline__ void k1_forward_body(const K1Args a) {
+    constexpr int RC = 16 * TM, LD = RowTile<HW>::LD;
     extern __shared__ __align__(16) float smem[];
     const NetLayout &L = a.L;
-    const int tid = threadIdx.x, tr = tid & 15, tc = tid >> 4;
+    const int tid = threadIdx.x, tr = tid & (RowTile<HW>::RT - 1), tc = tid >> RowTile<HW>::RT_LOG2;
     const int task = blockIdx.y;
     const int ldo = k1_ldo(L), ldx = L.ldw1;
 
     HalfNet actor, critic;
-    float *p = halfnet_carve(actor, smem, L, 0);
+    float *p = halfnet_carve<HW>(actor, smem, L, 0);
     if (SPLIT) {
-        float *pc = halfnet_carve(critic, smem, L, 1);      // same storage, used in a different pass
+        float *pc = halfnet_carve<HW>(critic, smem, L, 1);  // same storage, used in a different pass
         p = p > pc ? p : pc;
     } else {
-        p = halfnet_carve(critic, p, L, 1);
+        p = halfnet_carve<HW>(critic, p, L, 1);
     }
     float *x = p;  p += RC * ldx;
-    float *h1 = p; p += RC * LDH;
-    float *h2 = p; p += RC * LDH;
+    float *h1 = p; p += RC * LD;
+    float *h2 = p; p += RC * LD;
     float *mu = p; p += RC * ldo;
     float *vo = p;
 
@@ -84,9 +86,9 @@ __global__ void __launch_bounds__(NTHREADS, SPLIT ? 1 : 2) k1_forward_kernel(con
     for (int pass = 0; pass < (SPLIT ? 2 : 1); ++pass) {
         if (SPLIT && pass == 1 && (long long)c0 * RC >= rows_a) break;      // no action rows in this CTA's range
         __syncthreads();
-        if (!SPLIT) { halfnet_load<false>(actor, gp, L, 0); halfnet_load<false>(critic, gp, L, 1); }
-        else if (pass == 0) halfnet_load<false>(critic, gp, L, 1);
-        else halfnet_load<false>(actor, gp, L, 0);
+        if (!SPLIT) { halfnet_load<false, HW>(actor, gp, L, 0); halfnet_load<false, HW>(critic, gp, L, 1); }
+        else if (pass == 0) halfnet_load<false, HW>(critic, gp, L, 1);
+        else halfnet_load<false, HW>(actor, gp, L, 0);
         for (int i = tid; i < RC * ldx; i += NTHREADS) x[i] = 0.f;   // padded columns stay zero; loads touch k < O
         __syncthreads();
         for (int c = c0; c < c1; ++c) {
@@ -101,7 +103,7 @@ __global__ void __launch_bounds__(NTHREADS, SPLIT ? 1 : 2) k1_forward_kernel(con
             }
             __syncthreads();
             if (!SPLIT || pass == 0) {
-                half_forward<TM>(x, ldx, critic, L, h1, h2, vo, ldo, tr, tc);
+                half_forward<TM, HW>(x, ldx, critic, L, h1, h2, vo, ldo, tr, tc);
                 for (int i = tid; i < nrow * M; i += NTHREADS) {
                     int r = i / M, m = i - r * M;
                     value[(size_t)row0 * M + i] = vo[r * ldo + m];
@@ -109,7 +111,7 @@ __global__ void __launch_bounds__(NTHREADS, SPLIT ? 1 : 2) k1_forward_kernel(con
             }
             const int nact = min(nrow, rows_a - row0);   // rows of this chunk that carry an action
             if ((!SPLIT || pass == 1) && nact > 0) {        // uniform across the CTA
-                half_forward<TM>(x, ldx, actor, L, h1, h2, mu, ldo, tr, tc);
+                half_forward<TM, HW>(x, ldx, actor, L, h1, h2, mu, ldo, tr, tc);
                 // thread per (row, action dim): action + per-element log-density into mu[][] in place
                 for (int i = tid; i < nact * A; i += NTHREADS) {
                     int r = i / A, d = i - r * A;
@@ -137,6 +139,12 @@ __global__ void __launch_bounds__(NTHREADS, SPLIT ? 1 : 2) k1_forward_kernel(con
         }
     }
 }
+
+template <int TM, bool SPLIT>
+__global__ void __launch_bounds__(NTHREADS, SPLIT ? 1 : 2) k1_forward_kernel(const K1Args a) { k1_forward_body<TM, SPLIT, H>(a); }
+
+template <int TM, bool SPLIT, int HW>
+__global__ void __launch_bounds__(NTHREADS, SPLIT ? 1 : 2) k1_forward_h_kernel(const K1Args a) { k1_forward_body<TM, SPLIT, HW>(a); }
 
 }  // namespace pgm
 #include "k1_tc.cuh"
@@ -186,14 +194,15 @@ static int k1_tcw_launch(K1Args &a, int P, cudaStream_t st) {
     return PGM_OK;
 }
 
-static int k1_ffma_launch(K1Args &a, int P, int rows_v, int O, cudaStream_t stream);
+static int k1_ffma_launch(K1Args &a, int P, int rows_v, int O, int hidden, cudaStream_t stream);
 
-extern "C" int pgm_policy_forward_f32(const float *params, const float *obs, const float *eps, int eps_shared,
-                                      float *action, float *value, float *logp, int mode, int P, int rows_v,
-                                      int rows_a, int O, int A, int M, void *stream) {
+extern "C" int pgm_policy_forward_h_f32(const float *params, const float *obs, const float *eps, int eps_shared,
+                                        float *action, float *value, float *logp, int mode, int P, int rows_v,
+                                        int rows_a, int O, int A, int M, int hidden, void *stream) {
     PGM_REQUIRE(params && obs && value, "pgm_policy_forward_f32: null params/obs/value");
     PGM_REQUIRE(P > 0 && rows_v > 0 && rows_a >= 0 && rows_a <= rows_v, "pgm_policy_forward_f32: bad row counts");
     PGM_REQUIRE(O > 0 && A > 0 && M > 0 && A <= 64 && M <= 16, "pgm_policy_forward_f32: unsupported dims O=%d A=%d M=%d", O, A, M);
+    PGM_REQUIRE(hidden_supported(hidden), "pgm_policy_forward_f32: hidden width %d is not one of {32, 64, 128}", hidden);
     PGM_REQUIRE(mode >= 0 && mode <= 2, "pgm_policy_forward_f32: bad mode %d", mode);
     if (rows_a > 0) {
         PGM_REQUIRE(action && logp, "pgm_policy_forward_f32: rows_a>0 needs action and logp");
@@ -202,22 +211,42 @@ extern "C" int pgm_policy_forward_f32(const float *params, const float *obs, con
     K1Args a;
     a.params = params; a.obs = obs; a.eps = eps; a.action = action; a.value = value; a.logp = logp;
     a.eps_shared = eps_shared; a.mode = mode; a.P = P; a.rows_v = rows_v; a.rows_a = rows_a;
-    a.L = NetLayout(O, A, M);
+    a.L = NetLayout(O, A, M, hidden);
     a.obs_ts = a.val_ts = a.act_ts = a.logp_ts = 0; a.ctl = nullptr; a.obs_copy = nullptr; a.obs_copy_ts = 0; a.act_out = nullptr;
-    if (k1_tc_wanted(O, A, M, rows_v)) {
+    // the tensor-core forwards are built for hidden width 64; other widths run on the FFMA kernel
+    if (hidden == H && k1_tc_wanted(O, A, M, rows_v)) {
         if (O == 17) return k1_tc_launch(k1_tc_kernel<17, 6, 2>, a, P, O, (cudaStream_t)stream);
         return k1_tc_launch(k1_tc_kernel<11, 3, 3>, a, P, O, (cudaStream_t)stream);
     }
-    if (O == 376 && A == 17 && M == 2 && rows_v >= 1024) return k1_tcw_launch(a, P, (cudaStream_t)stream);
-    return k1_ffma_launch(a, P, rows_v, O, (cudaStream_t)stream);
+    if (hidden == H && O == 376 && A == 17 && M == 2 && rows_v >= 1024) return k1_tcw_launch(a, P, (cudaStream_t)stream);
+    return k1_ffma_launch(a, P, rows_v, O, hidden, (cudaStream_t)stream);
 }
 
-// FP32 FFMA kernel (per-step inference with a few rows, shapes without a tensor-core instantiation)
-static int k1_ffma_launch(K1Args &a, int P, int rows_v, int O, cudaStream_t stream) {
-    const bool split = k1_smem_bytes(a.L, 4, false) > 110 * 1024;       // keep two CTAs per SM for small networks
+extern "C" int pgm_policy_forward_f32(const float *params, const float *obs, const float *eps, int eps_shared,
+                                      float *action, float *value, float *logp, int mode, int P, int rows_v,
+                                      int rows_a, int O, int A, int M, void *stream) {
+    return pgm_policy_forward_h_f32(params, obs, eps, eps_shared, action, value, logp, mode, P, rows_v, rows_a, O, A, M, H,
+                                    stream);
+}
+
+template <typename Kern>
+static int k1_ffma_go(Kern kern, size_t &attr_done, const K1Args &a, dim3 grid, size_t smem, cudaStream_t stream) {
+    if (attr_done < smem) {                                              // raise the dynamic shared-memory limit once per size
+        PGM_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        attr_done = smem;
+    }
+    kern<<<grid, NTHREADS, smem, stream>>>(a);
+    return PGM_OK;
+}
+
+// FP32 FFMA kernel (per-step inference with a few rows, shapes without a tensor-core instantiation, hidden widths other
+// than 64)
+static int k1_ffma_launch(K1Args &a, int P, int rows_v, int O, int hidden, cudaStream_t stream) {
+    const bool split = k1_smem_bytes(a.L, 4, false, hidden) > 110 * 1024;   // keep two CTAs per SM for small networks
     const int TM = split ? 2 : 4, RC = 16 * TM;
-    const size_t smem = k1_smem_bytes(a.L, TM, split);
-    PGM_REQUIRE(smem <= 227 * 1024, "pgm_policy_forward_f32: obs dim %d needs %zu B shared memory", O, smem);
+    const size_t smem = k1_smem_bytes(a.L, TM, split, hidden);
+    PGM_REQUIRE(smem <= 227 * 1024, "pgm_policy_forward_f32: obs dim %d needs %zu B shared memory at hidden width %d", O, smem,
+                hidden);
     static int sms = 0;                                                  // queried once: this launcher sits in per-step loops
     if (sms == 0) {
         int dev = 0;
@@ -231,34 +260,32 @@ static int k1_ffma_launch(K1Args &a, int P, int rows_v, int O, cudaStream_t stre
     a.chunks_per_cta = (nchunks + ctas_per_task - 1) / ctas_per_task;
     ctas_per_task = (nchunks + a.chunks_per_cta - 1) / a.chunks_per_cta;
     dim3 grid(ctas_per_task, P);
-    static size_t attr_done[2] = {0, 0};                                 // raise the dynamic shared-memory limit once per size
-    if (split) {
-        if (attr_done[1] < smem) {
-            PGM_CUDA(cudaFuncSetAttribute(k1_forward_kernel<2, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-            attr_done[1] = smem;
-        }
-        k1_forward_kernel<2, true><<<grid, NTHREADS, smem, stream>>>(a);
-    } else {
-        if (attr_done[0] < smem) {
-            PGM_CUDA(cudaFuncSetAttribute(k1_forward_kernel<4, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-            attr_done[0] = smem;
-        }
-        k1_forward_kernel<4, false><<<grid, NTHREADS, smem, stream>>>(a);
-    }
+    static size_t attr_done[3][2] = {};                                  // [32 | 64 | 128][split]
+    size_t &done = attr_done[hidden == 32 ? 0 : (hidden == 64 ? 1 : 2)][split];
+    int rc;
+    if (hidden == 32) rc = split ? k1_ffma_go(k1_forward_h_kernel<2, true, 32>, done, a, grid, smem, stream)
+                                 : k1_ffma_go(k1_forward_h_kernel<4, false, 32>, done, a, grid, smem, stream);
+    else if (hidden == 128) rc = split ? k1_ffma_go(k1_forward_h_kernel<2, true, 128>, done, a, grid, smem, stream)
+                                       : k1_ffma_go(k1_forward_h_kernel<4, false, 128>, done, a, grid, smem, stream);
+    else rc = split ? k1_ffma_go(k1_forward_kernel<2, true>, done, a, grid, smem, stream)
+                    : k1_ffma_go(k1_forward_kernel<4, false>, done, a, grid, smem, stream);
+    if (rc) return rc;
     PGM_CUDA(cudaGetLastError());
     return PGM_OK;
 }
 
-extern "C" int pgm_policy_step_f32(const float *params, const int32_t *ctl, const float *obs_stage, const float *eps,
-                                   int eps_shared, float *obs_buf, size_t obs_task_stride, float *value_buf,
-                                   size_t value_task_stride, float *action_buf, size_t action_task_stride, float *logp_buf,
-                                   size_t logp_task_stride, float *act_out, int P, int N, int O, int A, int M, void *stream) {
+extern "C" int pgm_policy_step_h_f32(const float *params, const int32_t *ctl, const float *obs_stage, const float *eps,
+                                     int eps_shared, float *obs_buf, size_t obs_task_stride, float *value_buf,
+                                     size_t value_task_stride, float *action_buf, size_t action_task_stride, float *logp_buf,
+                                     size_t logp_task_stride, float *act_out, int P, int N, int O, int A, int M, int hidden,
+                                     void *stream) {
     PGM_REQUIRE(params && ctl && obs_buf && value_buf && action_buf && logp_buf && eps,
                 "pgm_policy_step_f32: null pointer argument");
     PGM_REQUIRE(P > 0 && N > 0 && O > 0 && A > 0 && M > 0 && A <= 64 && M <= 16, "pgm_policy_step_f32: unsupported sizes");
+    PGM_REQUIRE(hidden_supported(hidden), "pgm_policy_step_f32: hidden width %d is not one of {32, 64, 128}", hidden);
     K1Args a;
     a.params = params; a.eps = eps; a.eps_shared = eps_shared; a.mode = PGM_ACT_SAMPLE; a.P = P; a.rows_v = N; a.rows_a = N;
-    a.L = NetLayout(O, A, M);
+    a.L = NetLayout(O, A, M, hidden);
     a.ctl = ctl;
     if (obs_stage) {      // observations arrive in a dense staging block and are copied into their rollout slot by the kernel
         a.obs = obs_stage; a.obs_ts = 0; a.obs_copy = obs_buf; a.obs_copy_ts = obs_task_stride;
@@ -267,5 +294,14 @@ extern "C" int pgm_policy_step_f32(const float *params, const int32_t *ctl, cons
     }
     a.value = value_buf; a.val_ts = value_task_stride; a.action = action_buf; a.act_ts = action_task_stride;
     a.logp = logp_buf; a.logp_ts = logp_task_stride; a.act_out = act_out;
-    return k1_ffma_launch(a, P, N, O, (cudaStream_t)stream);
+    return k1_ffma_launch(a, P, N, O, hidden, (cudaStream_t)stream);
+}
+
+extern "C" int pgm_policy_step_f32(const float *params, const int32_t *ctl, const float *obs_stage, const float *eps,
+                                   int eps_shared, float *obs_buf, size_t obs_task_stride, float *value_buf,
+                                   size_t value_task_stride, float *action_buf, size_t action_task_stride, float *logp_buf,
+                                   size_t logp_task_stride, float *act_out, int P, int N, int O, int A, int M, void *stream) {
+    return pgm_policy_step_h_f32(params, ctl, obs_stage, eps, eps_shared, obs_buf, obs_task_stride, value_buf,
+                                 value_task_stride, action_buf, action_task_stride, logp_buf, logp_task_stride, act_out, P, N,
+                                 O, A, M, H, stream);
 }

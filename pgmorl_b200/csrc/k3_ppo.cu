@@ -109,18 +109,20 @@ __device__ __forceinline__ unsigned group_rank() {
 }
 
 // half-local flat parameter index -> offset inside the padded shared-memory image of the half
+template <int HW = H>
 __device__ __forceinline__ int half_img_off(const HalfNet &n, const NetLayout &L, int e) {
+    constexpr int LD = RowTile<HW>::LD, LOG2 = RowTile<HW>::LOG2;
     const int O = L.O;
-    if (e < H * O) { const int j = e / O; return j * L.ldw1 + (e - j * O); }
-    e -= H * O;
-    if (e < H) return (int)(n.b1 - n.W1) + e;
-    e -= H;
-    if (e < H * H) return (int)(n.W2 - n.W1) + (e >> 6) * LDH + (e & 63);
-    e -= H * H;
-    if (e < H) return (int)(n.b2 - n.W1) + e;
-    e -= H;
-    if (e < n.KH * H) return (int)(n.Wh - n.W1) + (e >> 6) * LDH + (e & 63);
-    e -= n.KH * H;
+    if (e < HW * O) { const int j = e / O; return j * L.ldw1 + (e - j * O); }
+    e -= HW * O;
+    if (e < HW) return (int)(n.b1 - n.W1) + e;
+    e -= HW;
+    if (e < HW * HW) return (int)(n.W2 - n.W1) + (e >> LOG2) * LD + (e & (HW - 1));
+    e -= HW * HW;
+    if (e < HW) return (int)(n.b2 - n.W1) + e;
+    e -= HW;
+    if (e < n.KH * HW) return (int)(n.Wh - n.W1) + (e >> LOG2) * LD + (e & (HW - 1));
+    e -= n.KH * HW;
     if (e < n.KH) return (int)(n.bh - n.W1) + e;
     return (int)(n.ls - n.W1) + (e - n.KH);
 }
@@ -131,21 +133,28 @@ __device__ __forceinline__ float fast_sqrt(float x) { float r; asm("sqrt.approx.
 // KG1: 4-column groups of dW1 per thread (OP <= 64*KG1); NA: head rows per thread (A,M <= 16*NA);
 // DB: double-buffered record gather; VU: unclipped value loss (every kernel family takes it as a template parameter, so the
 // clipped instantiations are the code they were before the option existed).
+// HW: hidden width (net.cuh RowTile). A thread's dW2 tile is CG x KQ2 quads by 4x4, its dW1 tile KG1 x CG; at HW = 32
+// the 32 k lanes cover OP <= 128 * KG1, at 64 and 128 the 16 k lanes cover OP <= 64 * KG1.
 // Generic path (any supported dims, incl. wide observations and C == 1): each CTA updates a 1/G
 // slice of its half in global memory and all CTAs reload the parameters (three barriers per step).
-// Small networks on C >= 2 take the fast path in k3_fast.cuh instead.
-template <int C, int TM, int KG1, int NA, bool DB, bool VU = false>
-__global__ void __launch_bounds__(NTHREADS, 1) k3_ppo_kernel(const K3Args a) {
+// Small networks on C >= 2 take the fast path in k3_fast.cuh instead (hidden width 64).
+// The body is shared by k3_ppo_kernel (HW = 64) and k3_ppo_h_kernel (HW = 32, 128).
+template <int C, int TM, int KG1, int NA, bool DB, bool VU, int HW>
+__device__ __forceinline__ void k3_ppo_body(const K3Args &a) {
+    using T = RowTile<HW>;
     constexpr int RC = 16 * TM;
+    constexpr int RT = T::RT, CT = T::CT, CG = T::CG, LD = T::LD, RPT = RC / RT;
+    constexpr int KQ2 = (HW / 4 + RT - 1) / RT;          // k quads of dW2 per thread
     constexpr int NHALF = (C == 1) ? 2 : 1;
     constexpr int G = (C == 1) ? 1 : C / 2;
     static_assert(!(DB && NHALF == 2), "double-buffered gather needs one half per CTA");
+    static_assert(RC % RT == 0, "chunk rows must be a multiple of the row lanes");
     extern __shared__ __align__(16) float smem[];
     __shared__ float red[34];
     __shared__ double sh_d[4];
 
     const NetLayout &L = a.L;
-    const int tid = threadIdx.x, tr = tid & 15, tc = tid >> 4;
+    const int tid = threadIdx.x, tr = tid & (RT - 1), tc = tid >> T::RT_LOG2;
     const int task = blockIdx.x / C;
     const unsigned rank = group_rank<C>();
     const int half0 = (C == 1) ? 0 : (int)(rank / G);
@@ -159,17 +168,17 @@ __global__ void __launch_bounds__(NTHREADS, 1) k3_ppo_kernel(const K3Args a) {
     HalfNet net[NHALF];
     float *p = smem;
 #pragma unroll
-    for (int hh = 0; hh < NHALF; ++hh) p = halfnet_carve(net[hh], p, L, half0 + hh);
-    float *h1 = p; p += RC * LDH;
-    float *h2 = p; p += RC * LDH;
-    float *dz = p; p += RC * LDH;
+    for (int hh = 0; hh < NHALF; ++hh) p = halfnet_carve<HW>(net[hh], p, L, half0 + hh);
+    float *h1 = p; p += RC * LD;
+    float *h2 = p; p += RC * LD;
+    float *dz = p; p += RC * LD;
     float *ho = p; p += round_up(RC * ldo, 4);
     float *els = p; p += round_up(RC * ldo, 4);
     float *recb = p;   // [DB ? 2 : 1][RC][RSS]
 
     float *gparams = a.params + (size_t)task * L.n_par;
 #pragma unroll
-    for (int hh = 0; hh < NHALF; ++hh) halfnet_load<false>(net[hh], gparams, L, half0 + hh);
+    for (int hh = 0; hh < NHALF; ++hh) halfnet_load<false, HW>(net[hh], gparams, L, half0 + hh);
 
     const float clip = (float)a.hy.clip_param;
     const float inv_mb = 1.f / (float)a.mb;
@@ -220,19 +229,26 @@ __global__ void __launch_bounds__(NTHREADS, 1) k3_ppo_kernel(const K3Args a) {
             const HalfNet &n = net[hh];
             const int KH = n.KH;
             // gradient accumulators (registers, persist over the chunks of this step)
-            float gW2[4][4], gb2[4], gW1[KG1][4][4], gb1[4], gWh[NA][4], gbh[NA], gls[NA];
+            float gW2[CG][KQ2][4][4], gb2[CG][4], gW1[KG1][CG][4][4], gb1[CG][4], gWh[NA][CG][4], gbh[NA], gls[NA];
+#pragma unroll
+            for (int jg = 0; jg < CG; ++jg)
 #pragma unroll
             for (int i = 0; i < 4; ++i) {
-                gb2[i] = 0.f; gb1[i] = 0.f;
+                gb2[jg][i] = 0.f; gb1[jg][i] = 0.f;
 #pragma unroll
                 for (int j = 0; j < 4; ++j) {
-                    gW2[i][j] = 0.f;
 #pragma unroll
-                    for (int q = 0; q < KG1; ++q) gW1[q][i][j] = 0.f;
+                    for (int kq = 0; kq < KQ2; ++kq) gW2[jg][kq][i][j] = 0.f;
+#pragma unroll
+                    for (int q = 0; q < KG1; ++q) gW1[q][jg][i][j] = 0.f;
                 }
             }
 #pragma unroll
-            for (int ia = 0; ia < NA; ++ia) { gbh[ia] = 0.f; gls[ia] = 0.f; gWh[ia][0] = gWh[ia][1] = gWh[ia][2] = gWh[ia][3] = 0.f; }
+            for (int ia = 0; ia < NA; ++ia) {
+                gbh[ia] = 0.f; gls[ia] = 0.f;
+#pragma unroll
+                for (int jg = 0; jg < CG; ++jg) gWh[ia][jg][0] = gWh[ia][jg][1] = gWh[ia][jg][2] = gWh[ia][jg][3] = 0.f;
+            }
 
             for (int c = 0; c < nchunk; ++c) {
                 const int ci = s * nchunk + c;
@@ -253,7 +269,7 @@ __global__ void __launch_bounds__(NTHREADS, 1) k3_ppo_kernel(const K3Args a) {
 
                 PGM_TR(1)
                 // ---------------- forward ----------------
-                half_forward<TM>(x, RSS, n, L, h1, h2, ho, ldo, tr, tc);
+                half_forward<TM, HW>(x, RSS, n, L, h1, h2, ho, ldo, tr, tc);
 
                 PGM_TR(2)
                 // ---------------- loss + d(loss)/d(head output), thread per row ----------------
@@ -307,40 +323,53 @@ __global__ void __launch_bounds__(NTHREADS, 1) k3_ppo_kernel(const K3Args a) {
                 PGM_TR(3)
                 // ---------------- phase A: head weight grads, dz2 ----------------
                 {
-                    const int kg = tid & 15, a0 = tid >> 4;
+                    const int kg = tid & (CT - 1), a0 = tid >> T::CT_LOG2;
 #pragma unroll
                     for (int ia = 0; ia < NA; ++ia) {
-                        const int aa = a0 + 16 * ia;
+                        const int aa = a0 + RT * ia;
                         if (aa < KH) {
 #pragma unroll 4
                             for (int r = 0; r < RC; ++r) {
                                 const float sv = ho[r * ldo + aa];
-                                const float4 hv = lds4(h2 + r * LDH + 4 * kg);
-                                gWh[ia][0] = fmaf(sv, hv.x, gWh[ia][0]); gWh[ia][1] = fmaf(sv, hv.y, gWh[ia][1]);
-                                gWh[ia][2] = fmaf(sv, hv.z, gWh[ia][2]); gWh[ia][3] = fmaf(sv, hv.w, gWh[ia][3]);
+#pragma unroll
+                                for (int jg = 0; jg < CG; ++jg) {
+                                    const float4 hv = lds4(h2 + r * LD + 4 * (kg + CT * jg));
+                                    float *gw = gWh[ia][jg];
+                                    gw[0] = fmaf(sv, hv.x, gw[0]); gw[1] = fmaf(sv, hv.y, gw[1]);
+                                    gw[2] = fmaf(sv, hv.z, gw[2]); gw[3] = fmaf(sv, hv.w, gw[3]);
+                                }
                                 if (kg == 0) gbh[ia] += sv;
                                 if (half == 0 && kg == 1) gls[ia] += els[r * ldo + aa];
                             }
                         }
                     }
-                    float acc[TM][4];
+                    float acc[RPT][CG][4];
 #pragma unroll
-                    for (int i = 0; i < TM; ++i) acc[i][0] = acc[i][1] = acc[i][2] = acc[i][3] = 0.f;
+                    for (int i = 0; i < RPT; ++i)
+#pragma unroll
+                        for (int jg = 0; jg < CG; ++jg) acc[i][jg][0] = acc[i][jg][1] = acc[i][jg][2] = acc[i][jg][3] = 0.f;
                     for (int aa = 0; aa < KH; ++aa) {
-                        const float4 w = lds4(n.Wh + aa * LDH + 4 * tc);
 #pragma unroll
-                        for (int i = 0; i < TM; ++i) {
-                            const float sv = ho[(tr + 16 * i) * ldo + aa];
-                            acc[i][0] = fmaf(sv, w.x, acc[i][0]); acc[i][1] = fmaf(sv, w.y, acc[i][1]);
-                            acc[i][2] = fmaf(sv, w.z, acc[i][2]); acc[i][3] = fmaf(sv, w.w, acc[i][3]);
+                        for (int jg = 0; jg < CG; ++jg) {
+                            const float4 w = lds4(n.Wh + aa * LD + 4 * (tc + CT * jg));
+#pragma unroll
+                            for (int i = 0; i < RPT; ++i) {
+                                const float sv = ho[(tr + RT * i) * ldo + aa];
+                                float *ac = acc[i][jg];
+                                ac[0] = fmaf(sv, w.x, ac[0]); ac[1] = fmaf(sv, w.y, ac[1]);
+                                ac[2] = fmaf(sv, w.z, ac[2]); ac[3] = fmaf(sv, w.w, ac[3]);
+                            }
                         }
                     }
 #pragma unroll
-                    for (int i = 0; i < TM; ++i) {
-                        const float4 hv = lds4(h2 + (tr + 16 * i) * LDH + 4 * tc);
-                        sts4(dz + (tr + 16 * i) * LDH + 4 * tc,
-                             make_float4(acc[i][0] * (1.f - hv.x * hv.x), acc[i][1] * (1.f - hv.y * hv.y),
-                                         acc[i][2] * (1.f - hv.z * hv.z), acc[i][3] * (1.f - hv.w * hv.w)));
+                    for (int i = 0; i < RPT; ++i)
+#pragma unroll
+                    for (int jg = 0; jg < CG; ++jg) {
+                        const int o = (tr + RT * i) * LD + 4 * (tc + CT * jg);
+                        const float4 hv = lds4(h2 + o);
+                        const float *ac = acc[i][jg];
+                        sts4(dz + o, make_float4(ac[0] * (1.f - hv.x * hv.x), ac[1] * (1.f - hv.y * hv.y),
+                                                 ac[2] * (1.f - hv.z * hv.z), ac[3] * (1.f - hv.w * hv.w)));
                     }
                 }
                 __syncthreads();
@@ -348,45 +377,63 @@ __global__ void __launch_bounds__(NTHREADS, 1) k3_ppo_kernel(const K3Args a) {
                 PGM_TR(4)
                 // ---------------- phase B: dW2, db2, dz1 (into the h2 buffer) ----------------
                 {
-                    const int tj = tid & 15, tk = tid >> 4;
+                    const int tj = tid & (CT - 1), tk = tid >> T::CT_LOG2;
 #pragma unroll 4
                     for (int r = 0; r < RC; ++r) {
-                        const float4 dv = lds4(dz + r * LDH + 4 * tj);
-                        const float4 hv = lds4(h1 + r * LDH + 4 * tk);
-                        const float dd[4] = {dv.x, dv.y, dv.z, dv.w};
 #pragma unroll
-                        for (int jj = 0; jj < 4; ++jj) {
-                            gW2[jj][0] = fmaf(dd[jj], hv.x, gW2[jj][0]); gW2[jj][1] = fmaf(dd[jj], hv.y, gW2[jj][1]);
-                            gW2[jj][2] = fmaf(dd[jj], hv.z, gW2[jj][2]); gW2[jj][3] = fmaf(dd[jj], hv.w, gW2[jj][3]);
+                        for (int jg = 0; jg < CG; ++jg) {
+                            const float4 dv = lds4(dz + r * LD + 4 * (tj + CT * jg));
+                            const float dd[4] = {dv.x, dv.y, dv.z, dv.w};
+#pragma unroll
+                            for (int kq = 0; kq < KQ2; ++kq) {
+                                if (4 * RT * KQ2 > HW && 4 * (tk + RT * kq) >= HW) continue;   // idle k lanes at HW = 32
+                                const float4 hv = lds4(h1 + r * LD + 4 * (tk + RT * kq));
+#pragma unroll
+                                for (int jj = 0; jj < 4; ++jj) {
+                                    float *gw = gW2[jg][kq][jj];
+                                    gw[0] = fmaf(dd[jj], hv.x, gw[0]); gw[1] = fmaf(dd[jj], hv.y, gw[1]);
+                                    gw[2] = fmaf(dd[jj], hv.z, gw[2]); gw[3] = fmaf(dd[jj], hv.w, gw[3]);
+                                }
+                            }
+                            if (tk == 0) { gb2[jg][0] += dv.x; gb2[jg][1] += dv.y; gb2[jg][2] += dv.z; gb2[jg][3] += dv.w; }
                         }
-                        if (tk == 0) { gb2[0] += dv.x; gb2[1] += dv.y; gb2[2] += dv.z; gb2[3] += dv.w; }
                     }
-                    float acc[TM][4];
+                    float acc[RPT][CG][4];
 #pragma unroll
-                    for (int i = 0; i < TM; ++i) acc[i][0] = acc[i][1] = acc[i][2] = acc[i][3] = 0.f;
+                    for (int i = 0; i < RPT; ++i)
+#pragma unroll
+                        for (int jg = 0; jg < CG; ++jg) acc[i][jg][0] = acc[i][jg][1] = acc[i][jg][2] = acc[i][jg][3] = 0.f;
 #pragma unroll 2
-                    for (int j = 0; j < H; j += 4) {
-                        float4 av[TM], bv[4];
+                    for (int j = 0; j < HW; j += 4) {
+                        float4 av[RPT], bv[CG][4];
 #pragma unroll
-                        for (int i = 0; i < TM; ++i) av[i] = lds4(dz + (tr + 16 * i) * LDH + j);
+                        for (int i = 0; i < RPT; ++i) av[i] = lds4(dz + (tr + RT * i) * LD + j);
 #pragma unroll
-                        for (int jj = 0; jj < 4; ++jj) bv[jj] = lds4(n.W2 + (j + jj) * LDH + 4 * tc);
+                        for (int jg = 0; jg < CG; ++jg)
 #pragma unroll
-                        for (int i = 0; i < TM; ++i) {
+                            for (int jj = 0; jj < 4; ++jj) bv[jg][jj] = lds4(n.W2 + (j + jj) * LD + 4 * (tc + CT * jg));
+#pragma unroll
+                        for (int i = 0; i < RPT; ++i) {
                             const float aa[4] = {av[i].x, av[i].y, av[i].z, av[i].w};
 #pragma unroll
+                            for (int jg = 0; jg < CG; ++jg)
+#pragma unroll
                             for (int jj = 0; jj < 4; ++jj) {
-                                acc[i][0] = fmaf(aa[jj], bv[jj].x, acc[i][0]); acc[i][1] = fmaf(aa[jj], bv[jj].y, acc[i][1]);
-                                acc[i][2] = fmaf(aa[jj], bv[jj].z, acc[i][2]); acc[i][3] = fmaf(aa[jj], bv[jj].w, acc[i][3]);
+                                float *ac = acc[i][jg];
+                                ac[0] = fmaf(aa[jj], bv[jg][jj].x, ac[0]); ac[1] = fmaf(aa[jj], bv[jg][jj].y, ac[1]);
+                                ac[2] = fmaf(aa[jj], bv[jg][jj].z, ac[2]); ac[3] = fmaf(aa[jj], bv[jg][jj].w, ac[3]);
                             }
                         }
                     }
 #pragma unroll
-                    for (int i = 0; i < TM; ++i) {
-                        const float4 hv = lds4(h1 + (tr + 16 * i) * LDH + 4 * tc);
-                        sts4(h2 + (tr + 16 * i) * LDH + 4 * tc,
-                             make_float4(acc[i][0] * (1.f - hv.x * hv.x), acc[i][1] * (1.f - hv.y * hv.y),
-                                         acc[i][2] * (1.f - hv.z * hv.z), acc[i][3] * (1.f - hv.w * hv.w)));
+                    for (int i = 0; i < RPT; ++i)
+#pragma unroll
+                    for (int jg = 0; jg < CG; ++jg) {
+                        const int o = (tr + RT * i) * LD + 4 * (tc + CT * jg);
+                        const float4 hv = lds4(h1 + o);
+                        const float *ac = acc[i][jg];
+                        sts4(h2 + o, make_float4(ac[0] * (1.f - hv.x * hv.x), ac[1] * (1.f - hv.y * hv.y),
+                                                 ac[2] * (1.f - hv.z * hv.z), ac[3] * (1.f - hv.w * hv.w)));
                     }
                 }
                 __syncthreads();
@@ -394,22 +441,26 @@ __global__ void __launch_bounds__(NTHREADS, 1) k3_ppo_kernel(const K3Args a) {
                 PGM_TR(5)
                 // ---------------- phase C: dW1, db1 ----------------
                 {
-                    const int tj = tid & 15, tk = tid >> 4;
+                    const int tj = tid & (CT - 1), tk = tid >> T::CT_LOG2;
 #pragma unroll
                     for (int q = 0; q < KG1; ++q) {
-                        const int k0 = 4 * (tk + 16 * q);
+                        const int k0 = 4 * (tk + RT * q);
                         if (k0 < OP) {
 #pragma unroll 4
                             for (int r = 0; r < RC; ++r) {
-                                const float4 dv = lds4(h2 + r * LDH + 4 * tj);
-                                const float4 xv = lds4(x + r * RSS + k0);
-                                const float dd[4] = {dv.x, dv.y, dv.z, dv.w};
 #pragma unroll
-                                for (int jj = 0; jj < 4; ++jj) {
-                                    gW1[q][jj][0] = fmaf(dd[jj], xv.x, gW1[q][jj][0]); gW1[q][jj][1] = fmaf(dd[jj], xv.y, gW1[q][jj][1]);
-                                    gW1[q][jj][2] = fmaf(dd[jj], xv.z, gW1[q][jj][2]); gW1[q][jj][3] = fmaf(dd[jj], xv.w, gW1[q][jj][3]);
+                                for (int jg = 0; jg < CG; ++jg) {
+                                    const float4 dv = lds4(h2 + r * LD + 4 * (tj + CT * jg));
+                                    const float4 xv = lds4(x + r * RSS + k0);
+                                    const float dd[4] = {dv.x, dv.y, dv.z, dv.w};
+#pragma unroll
+                                    for (int jj = 0; jj < 4; ++jj) {
+                                        float *gw = gW1[q][jg][jj];
+                                        gw[0] = fmaf(dd[jj], xv.x, gw[0]); gw[1] = fmaf(dd[jj], xv.y, gw[1]);
+                                        gw[2] = fmaf(dd[jj], xv.z, gw[2]); gw[3] = fmaf(dd[jj], xv.w, gw[3]);
+                                    }
+                                    if (q == 0 && tk == 0) { gb1[jg][0] += dv.x; gb1[jg][1] += dv.y; gb1[jg][2] += dv.z; gb1[jg][3] += dv.w; }
                                 }
-                                if (q == 0 && tk == 0) { gb1[0] += dv.x; gb1[1] += dv.y; gb1[2] += dv.z; gb1[3] += dv.w; }
                             }
                         }
                     }
@@ -422,30 +473,45 @@ __global__ void __launch_bounds__(NTHREADS, 1) k3_ppo_kernel(const K3Args a) {
             // ---- write this CTA's partial gradient of `half` to its scratch slot ----
             {
                 float *gp = a.gpart + ((size_t)(task * 2 + half) * G + g) * a.NHP;
-                const int tj = tid & 15, tk = tid >> 4;
-                const int lb1 = H * O, lW2 = lb1 + H, lb2 = lW2 + H * H, lWh = lb2 + H, lbh = lWh + KH * H, lls = lbh + KH;
+                const int tj = tid & (CT - 1), tk = tid >> T::CT_LOG2;
+                const int lb1 = HW * O, lW2 = lb1 + HW, lb2 = lW2 + HW * HW, lWh = lb2 + HW, lbh = lWh + KH * HW, lls = lbh + KH;
 #pragma unroll
                 for (int q = 0; q < KG1; ++q)
+#pragma unroll
+                    for (int jg = 0; jg < CG; ++jg)
 #pragma unroll
                     for (int jj = 0; jj < 4; ++jj)
 #pragma unroll
                         for (int kk = 0; kk < 4; ++kk) {
-                            const int k = 4 * (tk + 16 * q) + kk;
-                            if (k < O) gp[(4 * tj + jj) * O + k] = gW1[q][jj][kk];
+                            const int k = 4 * (tk + RT * q) + kk;
+                            if (k < O) gp[(4 * (tj + CT * jg) + jj) * O + k] = gW1[q][jg][jj][kk];
                         }
 #pragma unroll
-                for (int jj = 0; jj < 4; ++jj)
-                    sts4(gp + lW2 + (4 * tj + jj) * H + 4 * tk, make_float4(gW2[jj][0], gW2[jj][1], gW2[jj][2], gW2[jj][3]));
+                for (int jg = 0; jg < CG; ++jg)
+#pragma unroll
+                    for (int kq = 0; kq < KQ2; ++kq) {
+                        if (4 * RT * KQ2 > HW && 4 * (tk + RT * kq) >= HW) continue;
+#pragma unroll
+                        for (int jj = 0; jj < 4; ++jj) {
+                            const float *gw = gW2[jg][kq][jj];
+                            sts4(gp + lW2 + (4 * (tj + CT * jg) + jj) * HW + 4 * (tk + RT * kq), make_float4(gw[0], gw[1], gw[2], gw[3]));
+                        }
+                    }
                 if (tk == 0) {
-                    sts4(gp + lb1 + 4 * tj, make_float4(gb1[0], gb1[1], gb1[2], gb1[3]));
-                    sts4(gp + lb2 + 4 * tj, make_float4(gb2[0], gb2[1], gb2[2], gb2[3]));
+#pragma unroll
+                    for (int jg = 0; jg < CG; ++jg) {
+                        sts4(gp + lb1 + 4 * (tj + CT * jg), make_float4(gb1[jg][0], gb1[jg][1], gb1[jg][2], gb1[jg][3]));
+                        sts4(gp + lb2 + 4 * (tj + CT * jg), make_float4(gb2[jg][0], gb2[jg][1], gb2[jg][2], gb2[jg][3]));
+                    }
                 }
-                const int kg = tid & 15, a0 = tid >> 4;
+                const int kg = tid & (CT - 1), a0 = tid >> T::CT_LOG2;
 #pragma unroll
                 for (int ia = 0; ia < NA; ++ia) {
-                    const int aa = a0 + 16 * ia;
+                    const int aa = a0 + RT * ia;
                     if (aa < KH) {
-                        sts4(gp + lWh + aa * H + 4 * kg, make_float4(gWh[ia][0], gWh[ia][1], gWh[ia][2], gWh[ia][3]));
+#pragma unroll
+                        for (int jg = 0; jg < CG; ++jg)
+                            sts4(gp + lWh + aa * HW + 4 * (kg + CT * jg), make_float4(gWh[ia][jg][0], gWh[ia][jg][1], gWh[ia][jg][2], gWh[ia][jg][3]));
                         if (kg == 0) gp[lbh + aa] = gbh[ia];
                         if (half == 0 && kg == 1) gp[lls + aa] = gls[ia];
                     }
@@ -467,11 +533,11 @@ __global__ void __launch_bounds__(NTHREADS, 1) k3_ppo_kernel(const K3Args a) {
 #pragma unroll
         for (int hh = 0; hh < NHALF; ++hh) {
             const int half = half0 + hh;
-            const int nH = L.half_size(half);
+            const int nH = L.half_size(half, HW);
             const int per = round_up((nH + G - 1) / G, 4);
             const int s0 = g * per, s1 = min(nH, s0 + per);
             float *slot0 = a.gpart + (size_t)(task * 2 + half) * G * a.NHP;
-            const int lls = L.n_base + L.head_dim(half) * H + L.head_dim(half);
+            const int lls = L.n_base + L.head_dim(half) * HW + L.head_dim(half);
             for (int e = s0 + tid; e < s1; e += NTHREADS) {
                 float gs = 0.f;
 #pragma unroll
@@ -501,7 +567,7 @@ __global__ void __launch_bounds__(NTHREADS, 1) k3_ppo_kernel(const K3Args a) {
 #pragma unroll
         for (int hh = 0; hh < NHALF; ++hh) {
             const int half = half0 + hh;
-            const int nH = L.half_size(half);
+            const int nH = L.half_size(half, HW);
             const int per = round_up((nH + G - 1) / G, 4);
             const int s0 = g * per, s1 = min(nH, s0 + per);
             const float *mine = a.gpart + ((size_t)(task * 2 + half) * G + g) * a.NHP;
@@ -518,7 +584,7 @@ __global__ void __launch_bounds__(NTHREADS, 1) k3_ppo_kernel(const K3Args a) {
         }
         sync_group<C>();   // (3) new parameters of this task are in L2
 #pragma unroll
-        for (int hh = 0; hh < NHALF; ++hh) halfnet_load<true>(net[hh], gparams, L, half0 + hh);
+        for (int hh = 0; hh < NHALF; ++hh) halfnet_load<true, HW>(net[hh], gparams, L, half0 + hh);
         __syncthreads();
     }
 
@@ -547,6 +613,12 @@ __global__ void __launch_bounds__(NTHREADS, 1) k3_ppo_kernel(const K3Args a) {
     }
 }
 
+template <int C, int TM, int KG1, int NA, bool DB, bool VU = false>
+__global__ void __launch_bounds__(NTHREADS, 1) k3_ppo_kernel(const K3Args a) { k3_ppo_body<C, TM, KG1, NA, DB, VU, H>(a); }
+
+template <int HW, int C, int TM, int KG1, int NA, bool DB, bool VU>
+__global__ void __launch_bounds__(NTHREADS, 1) k3_ppo_h_kernel(const K3Args a) { k3_ppo_body<C, TM, KG1, NA, DB, VU, HW>(a); }
+
 }  // namespace pgm
 #include "k3_fast.cuh"
 #include "k3_tc.cuh"
@@ -560,6 +632,7 @@ struct K3Plan {
     int C, G, TM, KG1, NA, RC, Rg, RSG, RSS, NHP;
     bool DB, fast, tc, tcw;
     bool vu;      // unclipped value loss (PGM_PPO_VALUE_UNCLIPPED): the VU = true instantiation of the chosen kernel
+    int hidden;   // hidden width: 64, or 32 / 128 (generic kernel k3_ppo_h_kernel only)
     int tail;     // fast path step tail (k3_fast.cuh): 0 three cluster barriers, 1 redundant Adam, 2 TMA multicast broadcast
     int rs;
     int stage_floats;
@@ -568,13 +641,14 @@ struct K3Plan {
     size_t off_xp, off_scr, off_w1img, off_pmv;      // wide tensor-core path (k3_tcw.cuh)
 };
 
-static size_t k3_smem_bytes(const NetLayout &L, int C, int TM, bool DB, int RSS) {
+static size_t k3_smem_bytes(const NetLayout &L, int C, int TM, bool DB, int RSS, int hw = H) {
     const int RC = 16 * TM;
     const int ldo = ((L.A > L.M ? L.A : L.M) | 1);
+    const size_t i0 = halfnet_smem_floats(L, 0, hw), i1 = halfnet_smem_floats(L, 1, hw);
     size_t f = 0;
-    if (C == 1) f += halfnet_smem_floats(L, 0) + halfnet_smem_floats(L, 1);
-    else f += halfnet_smem_floats(L, 0) > halfnet_smem_floats(L, 1) ? halfnet_smem_floats(L, 0) : halfnet_smem_floats(L, 1);
-    f += 3 * (size_t)RC * LDH + 2 * (size_t)round_up(RC * ldo, 4);
+    if (C == 1) f += i0 + i1;
+    else f += i0 > i1 ? i0 : i1;
+    f += 3 * (size_t)RC * (hw + 4) + 2 * (size_t)round_up(RC * ldo, 4);
     f += (size_t)(DB ? 2 : 1) * RC * RSS;
     return f * sizeof(float);
 }
@@ -643,17 +717,25 @@ constexpr int K3_CLUSTER_TAILEP = 0x4000;  // tail 6
 constexpr int K3_CLUSTER_FLAGS = K3_CLUSTER_TAIL2 | K3_CLUSTER_TAILMC | K3_CLUSTER_TAILGL | K3_CLUSTER_TAIL0 | K3_CLUSTER_TAILBP |
                                  K3_CLUSTER_TAILNB | K3_CLUSTER_TAILEP | PGM_PPO_VALUE_UNCLIPPED;
 
-static int k3_plan(K3Plan &pl, int P, int S, int mb, int O, int A, int M, int cluster, int sms) {
-    NetLayout L(O, A, M);
+static int k3_plan(K3Plan &pl, int P, int S, int mb, int O, int A, int M, int cluster, int sms, int hidden) {
+    NetLayout L(O, A, M, hidden);
     const bool tail2 = (cluster & K3_CLUSTER_TAIL2) != 0, tailmc = (cluster & K3_CLUSTER_TAILMC) != 0;
     const bool tailgl = (cluster & K3_CLUSTER_TAILGL) != 0, tail0 = (cluster & K3_CLUSTER_TAIL0) != 0;
     const bool tailbp = (cluster & K3_CLUSTER_TAILBP) != 0, tailnb = (cluster & K3_CLUSTER_TAILNB) != 0;
     const bool tailep = (cluster & K3_CLUSTER_TAILEP) != 0;
     pl.vu = (cluster & PGM_PPO_VALUE_UNCLIPPED) != 0;
     cluster &= ~K3_CLUSTER_FLAGS;
-    pl.tc = false; pl.tcw = false; pl.tail = 0; pl.off_mv = 0;
+    pl.tc = false; pl.tcw = false; pl.tail = 0; pl.off_mv = 0; pl.hidden = hidden;
+    // the tensor-core kernels, the fast cluster kernel and cluster = 1 are built for hidden width 64; other widths run on
+    // the generic cluster kernel at 2..16 CTAs per task
+    if (hidden != H) {
+        PGM_REQUIRE(cluster != K3_CLUSTER_TC && cluster != K3_CLUSTER_TC2 && cluster != K3_CLUSTER_TC4,
+                    "ppo: the tensor-core paths (cluster 32, 64, 128) are built for hidden width 64, got hidden width %d", hidden);
+        PGM_REQUIRE(cluster != 1, "ppo: cluster 1 (both halves in one CTA) is built for hidden width 64, got hidden width %d "
+                    "(use cluster 0, 2, 4, 8 or 16)", hidden);
+    }
     // wide observations (Humanoid): the streamed tensor-core kernel; row split over as many CTAs per half as fill the SMs
-    if (k3_tcw_dims(O, A, M) && (cluster == 0 || cluster == K3_CLUSTER_TC || cluster == K3_CLUSTER_TC2 || cluster == K3_CLUSTER_TC4)) {
+    if (hidden == H && k3_tcw_dims(O, A, M) && (cluster == 0 || cluster == K3_CLUSTER_TC || cluster == K3_CLUSTER_TC2 || cluster == K3_CLUSTER_TC4)) {
         const int tiles = (mb + 127) / 128;
         if (cluster == 0) {
             // most CTAs per task whose clusters are all resident at once (a second wave of clusters doubles the step)
@@ -686,7 +768,7 @@ static int k3_plan(K3Plan &pl, int P, int S, int mb, int O, int A, int M, int cl
     }
     // auto: the tensor-core path wins as soon as the FFMA path can no longer give every task a 16-CTA cluster (measured on
     // a B200, profiles/k3_sweep.py: 1.2x at P = 8, 2.4x at 16, 3.3x from 37 tasks on; below 8 tasks FFMA is 6 % faster)
-    if (cluster == 0 && k3_tc_dims(O, A, M) && P >= 8) {
+    if (hidden == H && cluster == 0 && k3_tc_dims(O, A, M) && P >= 8) {
         // 4 CTAs per task (row tiles split over two CTAs per half) while they fit in one wave: 4-CTA clusters tile the 148
         // SMs less densely than pairs (measured: 32 clusters run in one wave, 37 need two)
         cluster = (mb > 128 && 4 * P <= sms - 20) ? K3_CLUSTER_TC2 : K3_CLUSTER_TC;
@@ -727,7 +809,12 @@ static int k3_plan(K3Plan &pl, int P, int S, int mb, int O, int A, int M, int cl
     }
     const bool big = (L.OP > 64) || (A > 16) || (M > 16);
     pl.C = C; pl.G = C == 1 ? 1 : C / 2;
-    pl.KG1 = big ? 6 : 1; pl.NA = big ? 2 : 1;
+    // dW1 k lanes: 16 (64 features per KG1 group) at hidden width 64 and 128, 32 (128 per group) at 32; head rows: 16 per
+    // NA at 64 and 128, 32 at 32. At 128 the wide variant stops at KG1 = 2 (OP <= 128): its dW1 tile then stays in
+    // registers next to the 64 dW2 accumulators (KG1 = 3 spills); at 32, KG1 = 3 covers Humanoid's 376 features
+    if (hidden == H) { pl.KG1 = big ? 6 : 1; pl.NA = big ? 2 : 1; }
+    else if (hidden == 128) { pl.KG1 = big ? 2 : 1; pl.NA = big ? 2 : 1; }
+    else { pl.KG1 = big ? 3 : 1; pl.NA = 1; }
     const int rows = (mb + pl.G - 1) / pl.G;          // rows per CTA per step
     pl.TM = big ? 2 : (rows <= 32 ? 2 : 4);
     pl.RC = 16 * pl.TM;
@@ -735,11 +822,11 @@ static int k3_plan(K3Plan &pl, int P, int S, int mb, int O, int A, int M, int cl
     pl.RSG = rec_stride(L);
     pl.RSS = stride4odd(pl.RSG);
     {
-        const int i0 = halfnet_smem_floats(L, 0), i1 = halfnet_smem_floats(L, 1);
+        const int i0 = halfnet_smem_floats(L, 0, hidden), i1 = halfnet_smem_floats(L, 1, hidden);
         pl.NHP = round_up(i0 > i1 ? i0 : i1, 64);   // covers both the reference-order half and its padded image
     }
     pl.DB = (C > 1) && !big;
-    pl.fast = (C > 1) && !big && L.OP <= 48 && pl.RC * (pl.RSG / 4) <= 4 * NTHREADS;
+    pl.fast = hidden == H && (C > 1) && !big && L.OP <= 48 && pl.RC * (pl.RSG / 4) <= 4 * NTHREADS;
     pl.stage_floats = 0;
     if (pl.fast) {
         const int s0 = k3_fast_stage_floats(L.OP, A), s1 = k3_fast_stage_floats(L.OP, M);
@@ -763,8 +850,10 @@ static int k3_plan(K3Plan &pl, int P, int S, int mb, int O, int A, int M, int cl
         }
         if (pl.smem > 227 * 1024) { pl.fast = false; pl.stage_floats = 0; pl.tail = 0; }
     }
-    if (!pl.fast) pl.smem = k3_smem_bytes(L, C, pl.TM, pl.DB, pl.RSS);
-    PGM_REQUIRE(pl.smem <= 227 * 1024, "ppo: configuration needs %zu B of shared memory (O=%d, cluster=%d)", pl.smem, O, C);
+    if (!pl.fast) pl.smem = k3_smem_bytes(L, C, pl.TM, pl.DB, pl.RSS, hidden);
+    PGM_REQUIRE(pl.smem <= 227 * 1024, "ppo: configuration needs %zu B of shared memory (O=%d, cluster=%d, hidden width %d)",
+                pl.smem, O, C, hidden);
+    PGM_REQUIRE(L.OP <= (hidden == 32 ? 128 : 64) * pl.KG1, "ppo: obs dim %d exceeds the dW1 tile at hidden width %d", O, hidden);
     size_t off = 0;
     auto seg = [&](size_t bytes) { size_t o = off; off += (bytes + 255) / 256 * 256; return o; };
     pl.off_rec = seg((size_t)P * S * pl.RSG * sizeof(float));
@@ -830,6 +919,27 @@ static int k3_launch_c(const K3Args &a, const K3Plan &pl, int P, cudaStream_t st
     }
 }
 
+// hidden width 32 / 128: the generic kernel at 2..16 CTAs per task
+template <int HW, int C, bool VU>
+static int k3_launch_hc(const K3Args &a, const K3Plan &pl, int P, cudaStream_t st) {
+    constexpr int KGB = HW == 128 ? 2 : 3, NAB = HW == 128 ? 2 : 1;   // the wide ("big") instantiation, k3_plan
+    if (pl.KG1 > 1) return k3_launch_k(k3_ppo_h_kernel<HW, C, 2, KGB, NAB, false, VU>, C, a, pl, P, st);
+    return pl.TM == 2 ? k3_launch_k(k3_ppo_h_kernel<HW, C, 2, 1, 1, true, VU>, C, a, pl, P, st)
+                      : k3_launch_k(k3_ppo_h_kernel<HW, C, 4, 1, 1, true, VU>, C, a, pl, P, st);
+}
+
+template <int HW, bool VU>
+static int k3_launch_h(const K3Args &a, const K3Plan &pl, int P, cudaStream_t st) {
+    switch (pl.C) {
+        case 2: return k3_launch_hc<HW, 2, VU>(a, pl, P, st);
+        case 4: return k3_launch_hc<HW, 4, VU>(a, pl, P, st);
+        case 8: return k3_launch_hc<HW, 8, VU>(a, pl, P, st);
+        case 16: return k3_launch_hc<HW, 16, VU>(a, pl, P, st);
+    }
+    set_error("ppo: bad cluster %d at hidden width %d", pl.C, HW);
+    return PGM_ERR_ARG;
+}
+
 template <typename Kern>
 static int k3_launch_w(Kern kern, const K3Args &a, const TwExtra &x, const K3Plan &pl, int P, cudaStream_t st) {
     PGM_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)pl.smem));
@@ -845,6 +955,8 @@ static int k3_launch_w(Kern kern, const K3Args &a, const TwExtra &x, const K3Pla
 
 template <bool VU>
 static int k3_launch(const K3Args &a, const K3Plan &pl, int P, cudaStream_t st) {
+    if (pl.hidden == 32) return k3_launch_h<32, VU>(a, pl, P, st);
+    if (pl.hidden == 128) return k3_launch_h<128, VU>(a, pl, P, st);
     if (pl.tc) {
         if (a.L.O == 17) return pl.rs == 2 ? k3_launch_k(k3_tc_kernel<17, 6, 2, 2, VU>, pl.C, a, pl, P, st)
                                            : k3_launch_k(k3_tc_kernel<17, 6, 2, 1, VU>, pl.C, a, pl, P, st);
@@ -886,12 +998,13 @@ static size_t g_last_trace_offset = 0;
 extern "C" size_t pgm_ppo_last_trace_offset() { return g_last_trace_offset; }
 #endif
 
-extern "C" size_t pgm_ppo_workspace_bytes(int P, int S, int O, int A, int M, int cluster) {
+extern "C" size_t pgm_ppo_workspace_bytes_h(int P, int S, int O, int A, int M, int cluster, int hidden) {
     // upper bound over every plan the launcher may choose for these dims (cluster 0 = auto)
-    NetLayout L(O, A, M);
+    if (!hidden_supported(hidden)) return 0;
+    NetLayout L(O, A, M, hidden);
     cluster &= ~K3_CLUSTER_FLAGS;
     const int G = cluster == 0 ? 8 : (cluster == 1 ? 1 : cluster / 2);
-    const int i0 = halfnet_smem_floats(L, 0), i1 = halfnet_smem_floats(L, 1);
+    const int i0 = halfnet_smem_floats(L, 0, hidden), i1 = halfnet_smem_floats(L, 1, hidden);
     const int NHP = round_up(i0 > i1 ? i0 : i1, 64);
     size_t t = 0;
     auto seg = [&](size_t b) { t += (b + 255) / 256 * 256; };
@@ -899,12 +1012,16 @@ extern "C" size_t pgm_ppo_workspace_bytes(int P, int S, int O, int A, int M, int
     seg((size_t)P * 2 * (G + 1) * NHP * sizeof(float));
     seg((size_t)P * 16 * sizeof(float));
     seg((size_t)P * 64 * sizeof(float));
-    if (k3_tc_dims(O, A, M)) seg(k3_tc_mv_bytes(P));
-    if (k3_tcw_dims(O, A, M)) seg(k3_tcw_bytes(P, S, O, A, nullptr, nullptr, nullptr, nullptr) + 1024);
+    if (hidden == H && k3_tc_dims(O, A, M)) seg(k3_tc_mv_bytes(P));
+    if (hidden == H && k3_tcw_dims(O, A, M)) seg(k3_tcw_bytes(P, S, O, A, nullptr, nullptr, nullptr, nullptr) + 1024);
 #ifdef PGM_K3_TRACE
     seg((size_t)P * 16 * 4 * 16 * 2 * sizeof(long long));
 #endif
     return t;
+}
+
+extern "C" size_t pgm_ppo_workspace_bytes(int P, int S, int O, int A, int M, int cluster) {
+    return pgm_ppo_workspace_bytes_h(P, S, O, A, M, cluster, H);
 }
 
 static int ppo_common(float *params, float *adam_m, float *adam_v, int32_t *adam_step, const double *lr,
@@ -912,15 +1029,16 @@ static int ppo_common(float *params, float *adam_m, float *adam_v, int32_t *adam
                       const float *value_old, size_t v_ts, const float *returns, const float *adv,
                       const int32_t *perm, int perm_shared, int E, int B, int mb, const pgm_ppo_hyper *hy,
                       float *losses, float *grad_out, void *workspace, size_t wbytes, int cluster, int P, int S,
-                      int O, int A, int M, cudaStream_t st) {
+                      int O, int A, int M, int hidden, cudaStream_t st) {
     PGM_REQUIRE(params && obs && action && logp_old && value_old && returns && adv && perm && hy && losses && workspace,
                 "ppo: null pointer argument");
+    PGM_REQUIRE(hidden_supported(hidden), "ppo: hidden width %d is not one of {32, 64, 128}", hidden);
     PGM_REQUIRE(P > 0 && S > 0 && mb > 0 && mb <= S, "ppo: bad sizes P=%d S=%d mb=%d", P, S, mb);
     PGM_REQUIRE(((uintptr_t)workspace & 255) == 0, "ppo: workspace must be 256-byte aligned");
     int sms = 148;
     if (int rc = sm_count(sms)) return rc;
     K3Plan pl;
-    if (int rc = k3_plan(pl, P, S, mb, O, A, M, cluster, sms)) return rc;
+    if (int rc = k3_plan(pl, P, S, mb, O, A, M, cluster, sms, hidden)) return rc;
     if (pl.total > wbytes) {
         set_error("ppo: workspace too small: need %zu bytes, got %zu", pl.total, wbytes);
         return PGM_ERR_WORKSPACE;
@@ -939,7 +1057,7 @@ static int ppo_common(float *params, float *adam_m, float *adam_v, int32_t *adam
     a.mv = (float *)(ws + pl.off_mv);
     a.grad_out = grad_out; a.perm_shared = perm_shared; a.E = E; a.B = B; a.mb = mb; a.S = S;
     a.grad_only = grad_out != nullptr; a.nsteps = a.grad_only ? 1 : E * B;
-    a.Rg = pl.Rg; a.RSG = pl.RSG; a.RSS = pl.RSS; a.NHP = pl.NHP; a.stage_floats = pl.stage_floats; a.rs = pl.rs; a.hy = *hy; a.L = NetLayout(O, A, M);
+    a.Rg = pl.Rg; a.RSG = pl.RSG; a.RSS = pl.RSS; a.NHP = pl.NHP; a.stage_floats = pl.stage_floats; a.rs = pl.rs; a.hy = *hy; a.L = NetLayout(O, A, M, hidden);
     if (pl.tcw) {
         TwExtra x;
         x.xp = (const __half *)(ws + pl.off_xp); x.scr = (const float *)(ws + pl.off_scr);
@@ -967,13 +1085,13 @@ static int ppo_common(float *params, float *adam_m, float *adam_v, int32_t *adam
     return pl.vu ? k3_launch<true>(a, pl, P, st) : k3_launch<false>(a, pl, P, st);
 }
 
-extern "C" int pgm_ppo_update_f32(float *params, float *adam_m, float *adam_v, int32_t *adam_step, const double *lr,
-                                  const float *obs, size_t obs_task_stride, const float *action,
-                                  const float *logp_old, const float *value_old, size_t value_task_stride,
-                                  const float *returns, const float *adv, const int32_t *perm, int perm_shared,
-                                  int E, int B, const pgm_ppo_hyper *hyper_host, float *losses, void *workspace,
-                                  size_t workspace_bytes, int cluster, int P, int S, int O, int A, int M,
-                                  void *stream) {
+extern "C" int pgm_ppo_update_h_f32(float *params, float *adam_m, float *adam_v, int32_t *adam_step, const double *lr,
+                                    const float *obs, size_t obs_task_stride, const float *action,
+                                    const float *logp_old, const float *value_old, size_t value_task_stride,
+                                    const float *returns, const float *adv, const int32_t *perm, int perm_shared,
+                                    int E, int B, const pgm_ppo_hyper *hyper_host, float *losses, void *workspace,
+                                    size_t workspace_bytes, int cluster, int P, int S, int O, int A, int M, int hidden,
+                                    void *stream) {
     PGM_REQUIRE(adam_m && adam_v && adam_step && lr, "pgm_ppo_update_f32: null optimizer state");
     PGM_REQUIRE(E > 0 && B > 0 && S / B > 0, "pgm_ppo_update_f32: bad E=%d B=%d for S=%d", E, B, S);
     // the reference's BatchSampler(drop_last=True) yields S // (S // B) minibatches per epoch (a2c/storage.py:133-137), which
@@ -982,7 +1100,31 @@ extern "C" int pgm_ppo_update_f32(float *params, float *adam_m, float *adam_v, i
                 "minibatch: the reference would run %d minibatches per epoch; choose S, B with S %% B < S / B", S, B, S / B, S % B, S / (S / B));
     return ppo_common(params, adam_m, adam_v, adam_step, lr, obs, obs_task_stride, action, logp_old, value_old,
                       value_task_stride, returns, adv, perm, perm_shared, E, B, S / B, hyper_host, losses, nullptr,
-                      workspace, workspace_bytes, cluster, P, S, O, A, M, (cudaStream_t)stream);
+                      workspace, workspace_bytes, cluster, P, S, O, A, M, hidden, (cudaStream_t)stream);
+}
+
+extern "C" int pgm_ppo_update_f32(float *params, float *adam_m, float *adam_v, int32_t *adam_step, const double *lr,
+                                  const float *obs, size_t obs_task_stride, const float *action,
+                                  const float *logp_old, const float *value_old, size_t value_task_stride,
+                                  const float *returns, const float *adv, const int32_t *perm, int perm_shared,
+                                  int E, int B, const pgm_ppo_hyper *hyper_host, float *losses, void *workspace,
+                                  size_t workspace_bytes, int cluster, int P, int S, int O, int A, int M,
+                                  void *stream) {
+    return pgm_ppo_update_h_f32(params, adam_m, adam_v, adam_step, lr, obs, obs_task_stride, action, logp_old, value_old,
+                                value_task_stride, returns, adv, perm, perm_shared, E, B, hyper_host, losses, workspace,
+                                workspace_bytes, cluster, P, S, O, A, M, H, stream);
+}
+
+extern "C" int pgm_ppo_grad_h_f32(const float *params, const float *obs, size_t obs_task_stride, const float *action,
+                                  const float *logp_old, const float *value_old, size_t value_task_stride,
+                                  const float *returns, const float *adv, const int32_t *idx, int mb,
+                                  const pgm_ppo_hyper *hyper_host, float *grad, float *losses, void *workspace,
+                                  size_t workspace_bytes, int cluster, int P, int S, int O, int A, int M, int hidden,
+                                  void *stream) {
+    PGM_REQUIRE(grad, "pgm_ppo_grad_f32: null grad");
+    return ppo_common(const_cast<float *>(params), nullptr, nullptr, nullptr, nullptr, obs, obs_task_stride, action,
+                      logp_old, value_old, value_task_stride, returns, adv, idx, 1, 1, 1, mb, hyper_host, losses, grad,
+                      workspace, workspace_bytes, cluster, P, S, O, A, M, hidden, (cudaStream_t)stream);
 }
 
 extern "C" int pgm_ppo_grad_f32(const float *params, const float *obs, size_t obs_task_stride, const float *action,
@@ -990,8 +1132,7 @@ extern "C" int pgm_ppo_grad_f32(const float *params, const float *obs, size_t ob
                                 const float *returns, const float *adv, const int32_t *idx, int mb,
                                 const pgm_ppo_hyper *hyper_host, float *grad, float *losses, void *workspace,
                                 size_t workspace_bytes, int cluster, int P, int S, int O, int A, int M, void *stream) {
-    PGM_REQUIRE(grad, "pgm_ppo_grad_f32: null grad");
-    return ppo_common(const_cast<float *>(params), nullptr, nullptr, nullptr, nullptr, obs, obs_task_stride, action,
-                      logp_old, value_old, value_task_stride, returns, adv, idx, 1, 1, 1, mb, hyper_host, losses, grad,
-                      workspace, workspace_bytes, cluster, P, S, O, A, M, (cudaStream_t)stream);
+    return pgm_ppo_grad_h_f32(params, obs, obs_task_stride, action, logp_old, value_old, value_task_stride, returns, adv,
+                              idx, mb, hyper_host, grad, losses, workspace, workspace_bytes, cluster, P, S, O, A, M, H,
+                              stream);
 }

@@ -49,9 +49,9 @@ def policy_forward(params, obs, dims: NetDims, eps=None, action=None, mode=ACT_S
     if mode == ACT_SAMPLE and rows_a > 0:
         assert eps is not None and eps.shape[1:] == (rows_a, dims.act) and eps.shape[0] in (1, P)
         eps_shared = int(eps.shape[0] == 1 and P > 1)
-    check(lib().pgm_policy_forward_f32(ptr(params), ptr(obs), ptr(eps), eps_shared, ptr(act_out), ptr(value),
-                                       ptr(logp), mode, P, rows_v, rows_a, dims.obs, dims.act, dims.obj,
-                                       _stream()))
+    check(lib().pgm_policy_forward_h_f32(ptr(params), ptr(obs), ptr(eps), eps_shared, ptr(act_out), ptr(value),
+                                         ptr(logp), mode, P, rows_v, rows_a, dims.obs, dims.act, dims.obj, dims.hidden,
+                                         _stream()))
     return value, act_out, logp
 
 
@@ -64,10 +64,10 @@ def policy_step(params, ctl, obs_stage, eps, obs_buf, value_buf, action_buf, log
                  ("action_buf", action_buf), ("logp_buf", logp_buf), ("act_out", act_out)):
         _f32c(t, n)
     assert eps.shape[-2:] == (N, dims.act) and eps.shape[0] in (1, P)
-    check(lib().pgm_policy_step_f32(ptr(params), ptr(ctl), ptr(obs_stage), ptr(eps), int(eps.shape[0] == 1 and P > 1),
-                                    ptr(obs_buf), obs_buf.stride(0), ptr(value_buf), value_buf.stride(0),
-                                    ptr(action_buf), action_buf.stride(0), ptr(logp_buf), logp_buf.stride(0), ptr(act_out),
-                                    P, N, dims.obs, dims.act, dims.obj, _stream()))
+    check(lib().pgm_policy_step_h_f32(ptr(params), ptr(ctl), ptr(obs_stage), ptr(eps), int(eps.shape[0] == 1 and P > 1),
+                                      ptr(obs_buf), obs_buf.stride(0), ptr(value_buf), value_buf.stride(0),
+                                      ptr(action_buf), action_buf.stride(0), ptr(logp_buf), logp_buf.stride(0), ptr(act_out),
+                                      P, N, dims.obs, dims.act, dims.obj, dims.hidden, _stream()))
 
 
 def gae_adv(rewards, value, masks, bad_masks, gamma, lam, weights=None, obj_var=None, out=None):
@@ -113,7 +113,7 @@ def returns_adv(rewards, value, masks, bad_masks, gamma, lam, use_gae=True, use_
 
 
 def ppo_workspace(P, S, dims: NetDims, device, cluster=0):
-    n = lib().pgm_ppo_workspace_bytes(P, S, dims.obs, dims.act, dims.obj, cluster)
+    n = lib().pgm_ppo_workspace_bytes_h(P, S, dims.obs, dims.act, dims.obj, cluster, dims.hidden)
     return torch.empty(n + 256, dtype=torch.uint8, device=device)
 
 
@@ -145,11 +145,12 @@ def ppo_update(params, adam_m, adam_v, adam_step, lr, obs, action, logp_old, val
     if losses is None:
         losses = torch.empty(P, 3, device=params.device, dtype=torch.float32)
     E = perm.shape[1]
-    check(lib().pgm_ppo_update_f32(
+    check(lib().pgm_ppo_update_h_f32(
         ptr(params), ptr(adam_m), ptr(adam_v), ptr(adam_step), ptr(lr), ptr(obs), obs.stride(0), ptr(action),
         ptr(logp_old), ptr(value_old), value_old.stride(0), ptr(returns), ptr(adv), ptr(perm),
         int(perm.shape[0] == 1 and P > 1), E, num_mini_batch, C.byref(hyper), ptr(losses), wp, wn,
-        cluster if clipped_value_loss else cluster | PPO_VALUE_UNCLIPPED, P, S, dims.obs, dims.act, dims.obj, _stream()))
+        cluster if clipped_value_loss else cluster | PPO_VALUE_UNCLIPPED, P, S, dims.obs, dims.act, dims.obj, dims.hidden,
+        _stream()))
     return losses
 
 
@@ -163,11 +164,11 @@ def ppo_grad(params, obs, action, logp_old, value_old, returns, adv, idx, dims: 
     wp, wn = _aligned(ws)
     grad = torch.zeros(P, dims.n_par, device=params.device, dtype=torch.float32)
     losses = torch.empty(P, 3, device=params.device, dtype=torch.float32)
-    check(lib().pgm_ppo_grad_f32(ptr(params), ptr(obs), obs.stride(0), ptr(action), ptr(logp_old), ptr(value_old),
-                                 value_old.stride(0), ptr(returns), ptr(adv), ptr(idx), idx.numel(),
-                                 C.byref(hyper), ptr(grad), ptr(losses), wp, wn,
-                                 cluster if clipped_value_loss else cluster | PPO_VALUE_UNCLIPPED, P, S, dims.obs, dims.act,
-                                 dims.obj, _stream()))
+    check(lib().pgm_ppo_grad_h_f32(ptr(params), ptr(obs), obs.stride(0), ptr(action), ptr(logp_old), ptr(value_old),
+                                   value_old.stride(0), ptr(returns), ptr(adv), ptr(idx), idx.numel(),
+                                   C.byref(hyper), ptr(grad), ptr(losses), wp, wn,
+                                   cluster if clipped_value_loss else cluster | PPO_VALUE_UNCLIPPED, P, S, dims.obs, dims.act,
+                                   dims.obj, dims.hidden, _stream()))
     return grad, losses
 
 

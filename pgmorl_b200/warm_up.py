@@ -27,7 +27,8 @@ def initialize_warm_up_batch(args, device):
         # same construction order as the reference: policy (consumes torch's global RNG for the orthogonal init),
         # agent, then a throw-away vectorised env whose initial running moments become the sample's env_params
         actor_critic = Policy(probe.observation_space.shape, probe.action_space,
-                              base_kwargs={'layernorm': args.layernorm}, obj_num=args.obj_num, device=device)
+                              base_kwargs={'layernorm': args.layernorm, 'hidden_size': getattr(args, 'hidden_size', 64)},
+                              obj_num=args.obj_num, device=device)
         actor_critic.to(device).double()
         agent = algo.PPO(actor_critic, args.clip_param, args.ppo_epoch, args.num_mini_batch, args.value_loss_coef,
                          args.entropy_coef, lr=args.lr, eps=1e-5, max_grad_norm=args.max_grad_norm)
