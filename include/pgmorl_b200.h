@@ -52,6 +52,14 @@ enum {
     PGM_ACT_EVALUATE = 2       /* action given, only log-prob        (a2c/model.py:75-82)  */
 };
 
+/* action distribution head (`dist` argument of the _x entry points) */
+enum {
+    PGM_DIST_GAUSSIAN = 0,   /* Box actions: DiagGaussian, mean head + state-independent logstd (a2c/distributions.py:71-90) */
+    PGM_DIST_CATEGORICAL = 1 /* Discrete(n) actions: Categorical, logits head, no logstd (a2c/distributions.py Categorical) */
+};
+/* categories of a Categorical head the kernels accept: 1 <= n <= PGM_CATEGORICAL_MAX (the head rows of K3's generic kernel) */
+#define PGM_CATEGORICAL_MAX 32
+
 int pgm_abi_version(void);
 const char *pgm_last_error(void);
 
@@ -64,6 +72,12 @@ int pgm_n_par_h(int obs_dim, int act_dim, int obj_num, int hidden);
  * base.critic_linear.{weight,bias}, dist.fc_mean.{weight,bias}, dist.logstd._bias (a2c/model.py:201-256) */
 int pgm_param_offsets(int obs_dim, int act_dim, int obj_num, int *out13);
 int pgm_param_offsets_h(int obs_dim, int act_dim, int obj_num, int hidden, int *out13);
+/* _x forms: hidden width `hidden` and action head `dist`. For PGM_DIST_CATEGORICAL, act_dim is the number of categories n
+ * and the layout has 12 tensors: the 10 base tensors, then dist.linear.{weight [n,H], bias [n]} (the Categorical
+ * module of a2c/distributions.py; Policy.__init__ in a2c/model.py builds base, then dist), no logstd. pgm_param_offsets_x writes one offset per
+ * tensor (13 or 12). Both return -1 / PGM_ERR_ARG and set pgm_last_error() for an unsupported width, head or n. */
+int pgm_n_par_x(int obs_dim, int act_dim, int obj_num, int hidden, int dist);
+int pgm_param_offsets_x(int obs_dim, int act_dim, int obj_num, int hidden, int dist, int *out);
 
 /* ---------------------------------------------------------------------------
  * K1  population-batched actor-critic forward.
@@ -89,6 +103,19 @@ int pgm_policy_forward_f32(const float *params, const float *obs, const float *e
 int pgm_policy_forward_h_f32(const float *params, const float *obs, const float *eps, int eps_shared,
                              float *action, float *value, float *logp, int mode, int P, int rows_v,
                              int rows_a, int O, int A, int M, int hidden, void *stream);
+/* pgm_policy_forward_x_f32: the _h form with the action head `dist`; _h is its PGM_DIST_GAUSSIAN case (entropy NULL).
+ * PGM_DIST_CATEGORICAL (Categorical / FixedCategorical of a2c/distributions.py), A = n categories
+ * (1 <= n <= PGM_CATEGORICAL_MAX), logits z = W h2 + b:
+ *   eps     [P or 1, rows_a, n]  Exponential(1) draws q (SAMPLE mode): action = first argmax_j softmax(z)_j / q_j, the
+ *                                single-sample path of torch.multinomial(probs, 1, True) in torch 2.11 (dist.sample())
+ *   action  [P, rows_a, 1]       the category index as a float (exact up to 2^24); DETERMINISTIC = first argmax_j z_j
+ *                                (dist.mode()), EVALUATE reads it
+ *   logp    [P, rows_a]          z_a - logsumexp(z)
+ *   entropy [P, rows_a] or NULL  per-row -sum_j p_j log p_j (Categorical only; must be NULL for a Gaussian head)
+ * Categorical heads always run on the FP32 FFMA kernel (no tensor-core forward). */
+int pgm_policy_forward_x_f32(const float *params, const float *obs, const float *eps, int eps_shared,
+                             float *action, float *value, float *logp, float *entropy, int mode, int P, int rows_v,
+                             int rows_a, int O, int A, int M, int hidden, int dist, void *stream);
 
 /* K1 in per-step mode for real environment loops (morl/mopg.py:103-135: one Policy.act per environment step): every
  * task's N current observations -> value / sampled action / log-prob written STRAIGHT INTO time slot t of the rollout
@@ -110,6 +137,13 @@ int pgm_policy_step_h_f32(const float *params, const int32_t *ctl, const float *
                           size_t value_task_stride, float *action_buf, size_t action_task_stride, float *logp_buf,
                           size_t logp_task_stride, float *act_out, int P, int N, int O, int A, int M, int hidden,
                           void *stream);
+/* the _h form with the action head `dist`; for PGM_DIST_CATEGORICAL eps is [P or 1, N, n] Exponential(1) draws and
+ * action_buf [P,TN,1] / act_out [P,N,1] receive the sampled category index (pgm_policy_forward_x_f32) */
+int pgm_policy_step_x_f32(const float *params, const int32_t *ctl, const float *obs_stage, const float *eps,
+                          int eps_shared, float *obs_buf, size_t obs_task_stride, float *value_buf,
+                          size_t value_task_stride, float *action_buf, size_t action_task_stride, float *logp_buf,
+                          size_t logp_task_stride, float *act_out, int P, int N, int O, int A, int M, int hidden,
+                          int dist, void *stream);
 
 /* ---------------------------------------------------------------------------
  * K2  vector-reward returns + scalarised, normalised advantage.
@@ -176,6 +210,13 @@ int pgm_gae_adv_f32(const float *rewards, const float *value, const float *masks
  *   error naming the width. A shape whose network half exceeds 227 KB of shared memory is refused (Humanoid at 128);
  *   at 128 the observation width is also limited to O <= 128 (the register tile of dW1), at 32 to O <= 384.
  *   At 64 they are the functions without `hidden`.
+ * The _x forms take the hidden width and the action head `dist`; the _h forms are their PGM_DIST_GAUSSIAN case.
+ *   PGM_DIST_CATEGORICAL: A = n categories (1 <= n <= PGM_CATEGORICAL_MAX), action [P,S,1] holds the category index as a
+ *   float; log-prob z_a - logsumexp(z) and entropy -sum_j p_j log p_j per row (FixedCategorical of a2c/distributions.py),
+ *   whose gradient d(-entropy_coef * mean_i H_i)/dz_ij = entropy_coef / mb * p_ij (log p_ij + H_i) joins the surrogate's;
+ *   losses[:,2] is the entropy averaged over rows and updates. Only the generic FFMA cluster kernel serves this head, at
+ *   every hidden width: cluster 0 (auto), 2, 4, 8 or 16. cluster 1 and the tensor-core values 32 / 64 / 128 are refused
+ *   with an error naming the categorical head.
  */
 #define PGM_PPO_VALUE_UNCLIPPED 0x10000
 
@@ -191,6 +232,8 @@ typedef struct {
 size_t pgm_ppo_workspace_bytes(int P, int S, int O, int A, int M, int cluster);
 /* 0 for an unsupported hidden width */
 size_t pgm_ppo_workspace_bytes_h(int P, int S, int O, int A, int M, int cluster, int hidden);
+/* 0 for an unsupported hidden width or head */
+size_t pgm_ppo_workspace_bytes_x(int P, int S, int O, int A, int M, int cluster, int hidden, int dist);
 
 int pgm_ppo_update_f32(float *params, float *adam_m, float *adam_v, int32_t *adam_step,
                        const double *lr, const float *obs, size_t obs_task_stride,
@@ -208,6 +251,14 @@ int pgm_ppo_update_h_f32(float *params, float *adam_m, float *adam_v, int32_t *a
                          const pgm_ppo_hyper *hyper_host, float *losses, void *workspace,
                          size_t workspace_bytes, int cluster, int P, int S, int O, int A, int M, int hidden,
                          void *stream);
+int pgm_ppo_update_x_f32(float *params, float *adam_m, float *adam_v, int32_t *adam_step,
+                         const double *lr, const float *obs, size_t obs_task_stride,
+                         const float *action, const float *logp_old, const float *value_old,
+                         size_t value_task_stride, const float *returns, const float *adv,
+                         const int32_t *perm, int perm_shared, int E, int B,
+                         const pgm_ppo_hyper *hyper_host, float *losses, void *workspace,
+                         size_t workspace_bytes, int cluster, int P, int S, int O, int A, int M, int hidden,
+                         int dist, void *stream);
 
 /* Debug/verification aid: gradient of one minibatch (rows idx[0..mb)) of every task,
  * before clipping; grad [P, n_par], losses [P,3]. Same device code as pgm_ppo_update_f32. */
@@ -223,6 +274,12 @@ int pgm_ppo_grad_h_f32(const float *params, const float *obs, size_t obs_task_st
                        const int32_t *idx, int mb, const pgm_ppo_hyper *hyper_host, float *grad,
                        float *losses, void *workspace, size_t workspace_bytes, int cluster, int P,
                        int S, int O, int A, int M, int hidden, void *stream);
+int pgm_ppo_grad_x_f32(const float *params, const float *obs, size_t obs_task_stride,
+                       const float *action, const float *logp_old, const float *value_old,
+                       size_t value_task_stride, const float *returns, const float *adv,
+                       const int32_t *idx, int mb, const pgm_ppo_hyper *hyper_host, float *grad,
+                       float *losses, void *workspace, size_t workspace_bytes, int cluster, int P,
+                       int S, int O, int A, int M, int hidden, int dist, void *stream);
 
 /* ---------------------------------------------------------------------------
  * K4  batched fit of the hyperbolic prediction model (FLOAT64, one warp per fit).

@@ -65,6 +65,16 @@ SIGNATURES = {
                                   C.POINTER(PpoHyper), _P, _P, _Z, _I, _I, _I, _I, _I, _I, _I, _P]),
     "pgm_ppo_grad_h_f32": (_I, [_P, _P, _Z, _P, _P, _P, _Z, _P, _P, _P, _I, C.POINTER(PpoHyper), _P, _P, _P,
                                 _Z, _I, _I, _I, _I, _I, _I, _I, _P]),
+    "pgm_n_par_x": (_I, [_I, _I, _I, _I, _I]),
+    "pgm_param_offsets_x": (_I, [_I, _I, _I, _I, _I, _P]),
+    "pgm_policy_forward_x_f32": (_I, [_P, _P, _P, _I, _P, _P, _P, _P, _I, _I, _I, _I, _I, _I, _I, _I, _I, _P]),
+    "pgm_policy_step_x_f32": (_I, [_P, _P, _P, _P, _I, _P, _Z, _P, _Z, _P, _Z, _P, _Z, _P, _I, _I, _I, _I, _I, _I, _I,
+                                   _P]),
+    "pgm_ppo_workspace_bytes_x": (_Z, [_I, _I, _I, _I, _I, _I, _I, _I]),
+    "pgm_ppo_update_x_f32": (_I, [_P, _P, _P, _P, _P, _P, _Z, _P, _P, _P, _Z, _P, _P, _P, _I, _I, _I,
+                                  C.POINTER(PpoHyper), _P, _P, _Z, _I, _I, _I, _I, _I, _I, _I, _I, _P]),
+    "pgm_ppo_grad_x_f32": (_I, [_P, _P, _Z, _P, _P, _P, _Z, _P, _P, _P, _I, C.POINTER(PpoHyper), _P, _P, _P,
+                                _Z, _I, _I, _I, _I, _I, _I, _I, _I, _P]),
 }
 
 

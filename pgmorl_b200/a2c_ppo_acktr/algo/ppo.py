@@ -13,7 +13,7 @@ from ...layout import param_layout
 
 class DeviceAdam:
     """Adam moments as flat float32 CUDA vectors + the scalar step; state_dict()/load_state_dict() speak
-    torch.optim.Adam's format (13 parameter tensors in named_parameters() order)."""
+    torch.optim.Adam's format (13 parameter tensors in named_parameters() order, 12 for a Categorical head)."""
 
     def __init__(self, actor_critic, lr, eps):
         self.dims, self.device = actor_critic.dims, actor_critic.flat.device
@@ -21,7 +21,7 @@ class DeviceAdam:
         self.exp_avg_sq = torch.zeros_like(actor_critic.flat)
         self.step_count = 0
         self.param_groups = [{"lr": lr, "betas": (0.9, 0.999), "eps": eps, "weight_decay": 0, "amsgrad": False,
-                              "params": list(range(13))}]
+                              "params": list(range(len(param_layout(self.dims)[0])))}]
 
     def state_dict(self):
         layout, _ = param_layout(self.dims)
@@ -100,7 +100,7 @@ class PPO():
                          opt.param_groups[0]["betas"][0], opt.param_groups[0]["betas"][1], opt.param_groups[0]["eps"])
         params, m, v = pol.flat[None], opt.exp_avg[None], opt.exp_avg_sq[None]
         losses = K.ppo_update(params, m, v, step, lr, rollouts.obs.view(1, (T + 1) * N, d.obs),
-                              rollouts.actions.view(1, S, d.act), rollouts.action_log_probs.view(1, S),
+                              rollouts.actions.view(1, S, d.act_cols).to(torch.float32), rollouts.action_log_probs.view(1, S),
                               rollouts.value_preds.view(1, (T + 1) * N, M), ret.view(1, S, M), adv.view(1, S), perm,
                               self.num_mini_batch, d, hyper=hyper, cluster=self.cluster,
                               clipped_value_loss=self.use_clipped_value_loss)

@@ -1,17 +1,17 @@
 """Policy with the reference's interface (a2c_ppo_acktr/model.py:15-82) whose parameters live in ONE flat
 float32 CUDA vector (order: pgmorl_b200/layout.py) and whose forward passes are K1 launches.
 
-Only the configuration PG-MORL instantiates is supported (warm_up.py:34-40): 1-D observations, Box actions,
-MOMLPBase H-H tanh without LayerNorm (H = base_kwargs['hidden_size'], default 64; 32, 64 and 128 run on the device),
-DiagGaussian with state-independent logstd. CNN / GRU / Categorical
-bases of the upstream class are never reached by morl/ and are not provided."""
+Supported: 1-D observations, MOMLPBase H-H tanh without LayerNorm (H = base_kwargs['hidden_size'], default 64; 32, 64
+and 128 run on the device), and the head the action space selects as in the reference: Box -> DiagGaussian with
+state-independent logstd (the configuration PG-MORL instantiates, warm_up.py:34-40), Discrete(n) -> Categorical
+(1 <= n <= 32). CNN / GRU bases and MultiBinary (Bernoulli) heads are not provided."""
 from collections import OrderedDict
 
 import numpy as np
 import torch
 
 from .. import kernels as K
-from ..layout import NetDims, param_layout
+from ..layout import CATEGORICAL_MAX, DIST_CATEGORICAL, DIST_GAUSSIAN, NetDims, param_layout
 from ..synthetic import init_policy_flat
 
 HIDDEN_SIZES = (32, 64, 128)     # hidden widths the K1 / K3 kernels are built for (include/pgmorl_b200.h)
@@ -19,15 +19,23 @@ HIDDEN_SIZES = (32, 64, 128)     # hidden widths the K1 / K3 kernels are built f
 
 class Policy:
     def __init__(self, obs_shape, action_space, base=None, base_kwargs=None, obj_num=1, device="cuda", flat=None):
-        if len(obs_shape) != 1 or action_space.__class__.__name__ != "Box":
-            raise NotImplementedError("Policy: only 1-D observations with Box actions (the MO-MuJoCo configuration)")
+        kind = action_space.__class__.__name__
+        if len(obs_shape) != 1 or kind not in ("Box", "Discrete"):
+            raise NotImplementedError("Policy: only 1-D observations with Box or Discrete actions")
         if base_kwargs and base_kwargs.get("layernorm", False):
             raise NotImplementedError("Policy: layernorm=True is not part of the PG-MORL configuration (warm_up.py:37)")
         hidden = int((base_kwargs or {}).get("hidden_size", 64))
         if hidden not in HIDDEN_SIZES:
             raise NotImplementedError(f"Policy: hidden_size={hidden} is not supported; the kernels are built for "
                                       f"hidden_size in {{32, 64, 128}}")
-        self.dims = NetDims(int(obs_shape[0]), int(action_space.shape[0]), int(obj_num), hidden)
+        if kind == "Discrete":
+            n = int(action_space.n)
+            if not 1 <= n <= CATEGORICAL_MAX:
+                raise NotImplementedError(f"Policy: Discrete({n}) is not supported; the kernels are built for categorical "
+                                          f"heads of 1 to {CATEGORICAL_MAX} actions")
+            self.dims = NetDims(int(obs_shape[0]), n, int(obj_num), hidden, DIST_CATEGORICAL)
+        else:
+            self.dims = NetDims(int(obs_shape[0]), int(action_space.shape[0]), int(obj_num), hidden, DIST_GAUSSIAN)
         self.device = torch.device(device)
         if flat is None:
             flat = init_policy_flat(self.dims)          # draws from torch's global CPU generator like the reference
@@ -73,16 +81,19 @@ class Policy:
     def act(self, inputs, rnn_hxs, masks, deterministic=False):
         """-> value [N,M], action [N,A], action_log_probs [N,1], rnn_hxs (model.py:57-69). Sampling noise comes from
         torch's global CPU generator, one normal_(0,1) draw of shape [N,A] in float64, exactly the stream
-        dist.sample() consumes in the reference."""
+        dist.sample() consumes in the reference. Categorical head: one exponential_(1) draw of shape [N,n] in float64
+        (torch.multinomial's single-sample path), and the action is int64 [N,1]."""
         obs = self._obs(inputs)
         n = obs.shape[1]
         if deterministic:
             value, action, logp = K.policy_forward(self.flat[None], obs, self.dims, mode=K.ACT_DETERMINISTIC)
         else:
-            eps = torch.empty(n, self.dims.act, dtype=torch.float64).normal_(0, 1)
+            eps = torch.empty(n, self.dims.act, dtype=torch.float64)
+            eps.exponential_(1) if self.dims.categorical else eps.normal_(0, 1)
             value, action, logp = K.policy_forward(self.flat[None], obs, self.dims,
                                                    eps=eps.to(self.device, torch.float32)[None].contiguous())
-        return value[0], action[0], logp[0].unsqueeze(-1), rnn_hxs
+        action = action[0].to(torch.int64) if self.dims.categorical else action[0]
+        return value[0], action, logp[0].unsqueeze(-1), rnn_hxs
 
     def get_value(self, inputs, rnn_hxs, masks):
         value, _, _ = K.policy_forward(self.flat[None], self._obs(inputs), self.dims, rows_a=0, mode=K.ACT_DETERMINISTIC)
@@ -91,7 +102,12 @@ class Policy:
     def evaluate_actions(self, inputs, rnn_hxs, masks, action):
         """-> value, action_log_probs [N,1], dist_entropy (scalar), rnn_hxs (model.py:75-82)."""
         obs = self._obs(inputs)
-        act = torch.as_tensor(action).to(self.device, torch.float32).reshape(1, -1, self.dims.act).contiguous()
+        act = torch.as_tensor(action).to(self.device, torch.float32).reshape(1, -1, self.dims.act_cols).contiguous()
+        if self.dims.categorical:        # per-row entropy from K1, mean over the rows (FixedCategorical.entropy().mean())
+            ent_rows = torch.empty(1, act.shape[1], device=self.device, dtype=torch.float32)
+            value, _, logp = K.policy_forward(self.flat[None], obs, self.dims, action=act, mode=K.ACT_EVALUATE,
+                                              entropy=ent_rows)
+            return value[0], logp[0].unsqueeze(-1), ent_rows.mean(), rnn_hxs
         value, _, logp = K.policy_forward(self.flat[None], obs, self.dims, action=act, mode=K.ACT_EVALUATE)
         logstd = self.flat[-self.dims.act:]
         entropy = (0.5 + 0.5 * float(np.log(2 * np.pi)) + logstd).sum()

@@ -8,8 +8,9 @@ from .. import kernels as K
 class RolloutStorage(object):
     def __init__(self, num_steps, num_processes, obs_shape, action_space, recurrent_hidden_state_size, obj_num=1,
                  device="cuda"):
-        if action_space.__class__.__name__ != "Box":
-            raise NotImplementedError("RolloutStorage: Box action spaces only (MO-MuJoCo)")
+        kind = action_space.__class__.__name__
+        if kind not in ("Box", "Discrete"):
+            raise NotImplementedError("RolloutStorage: Box or Discrete action spaces only")
         dv, T, N = torch.device(device), num_steps, num_processes
         z = lambda *s: torch.zeros(*s, device=dv, dtype=torch.float32)
         self.obs = z(T + 1, N, *obs_shape)
@@ -18,7 +19,9 @@ class RolloutStorage(object):
         self.value_preds = z(T + 1, N, obj_num)
         self.returns = z(T + 1, N, obj_num)
         self.action_log_probs = z(T, N, 1)
-        self.actions = z(T, N, action_space.shape[0])
+        # Discrete: one int64 column per step, as the reference stores the sampled category (RolloutStorage.__init__)
+        self.actions = (torch.zeros(T, N, 1, device=dv, dtype=torch.int64) if kind == "Discrete"
+                        else z(T, N, action_space.shape[0]))
         self.masks = torch.ones(T + 1, N, 1, device=dv)
         self.bad_masks = torch.ones(T + 1, N, 1, device=dv)
         self.num_steps = num_steps
@@ -33,7 +36,7 @@ class RolloutStorage(object):
         dv = self.obs.device
         f = lambda t: torch.as_tensor(t).to(dv, torch.float32)
         self.obs[self.step + 1].copy_(f(obs))
-        self.actions[self.step].copy_(f(actions))
+        self.actions[self.step].copy_(torch.as_tensor(actions).to(dv, self.actions.dtype))
         self.action_log_probs[self.step].copy_(f(action_log_probs))
         self.value_preds[self.step].copy_(f(value_preds))
         self.rewards[self.step].copy_(f(rewards))

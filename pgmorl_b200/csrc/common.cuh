@@ -12,6 +12,8 @@ constexpr int H = PGM_HIDDEN;   // default hidden width (a2c/model.py:202); the 
 constexpr int LDH = H + 4;      // smem row stride of 64-wide tiles: 68 = 4*17 -> 8 consecutive rows
                                 // at the same column land in 8 distinct 16-byte bank groups
 __host__ __device__ inline bool hidden_supported(int hw) { return hw == 32 || hw == 64 || hw == 128; }
+__host__ __device__ inline bool dist_supported(int d) { return d == PGM_DIST_GAUSSIAN || d == PGM_DIST_CATEGORICAL; }
+constexpr int CAT_MAX = 32;     // categories of a Categorical head: K3's generic kernel holds at most 32 head rows
 constexpr int NTHREADS = 256;   // every MLP kernel uses 256-thread CTAs (16x16 tiles at hidden width 64, net.cuh)
 
 void set_error(const char *fmt, ...);
@@ -38,27 +40,36 @@ __host__ __device__ inline int stride4odd(int x) {
     return ((s / 4) & 1) ? s : s + 4;
 }
 
-// Offsets of the 13 tensors inside one flat parameter vector (reference order,
-// pgmorl_b200/layout.py) and the two "halves" (actor / critic) the kernels work on.
+// Offsets of the 13 tensors (12 for a Categorical head: no logstd) inside one flat parameter vector (reference order,
+// pgmorl_b200/layout.py) and the two "halves" (actor / critic) the kernels work on. A is the head width: the action
+// dimension of a DiagGaussian head, the number of categories of a Categorical head.
 struct NetLayout {
     int O, A, M;
     int OP;        // O rounded up to a multiple of 4 (zero padded contraction length of layer 1)
     int ldw1;      // smem row stride of W1 rows / observation rows
     int oW1a, ob1a, oW2a, ob2a, oW1c, ob1c, oW2c, ob2c, oWv, obv, oWmu, obmu, ols, n_par;
     int n_base;    // W1+b1+W2+b2 of one half
+    int dist;      // PGM_DIST_GAUSSIAN or PGM_DIST_CATEGORICAL
+    int AC;        // action columns of the rollout buffers and K3 records: A (Gaussian) or 1 (the category index)
+    int nls;       // logstd entries: A (Gaussian) or 0
     __host__ __device__ NetLayout() {}
     // hw = hidden width (32, 64 or 128)
-    __host__ __device__ NetLayout(int O_, int A_, int M_, int hw = H) : O(O_), A(A_), M(M_) {
+    __host__ __device__ NetLayout(int O_, int A_, int M_, int hw = H, int dist_ = PGM_DIST_GAUSSIAN)
+        : O(O_), A(A_), M(M_), dist(dist_) {
+        AC = dist == PGM_DIST_CATEGORICAL ? 1 : A;
+        nls = dist == PGM_DIST_CATEGORICAL ? 0 : A;
         OP = round_up(O, 4);
         ldw1 = stride4odd(OP);
         oW1a = 0; ob1a = oW1a + hw * O; oW2a = ob1a + hw; ob2a = oW2a + hw * hw;
         oW1c = ob2a + hw; ob1c = oW1c + hw * O; oW2c = ob1c + hw; ob2c = oW2c + hw * hw;
         oWv = ob2c + hw; obv = oWv + M * hw; oWmu = obv + M; obmu = oWmu + A * hw;
-        ols = obmu + A; n_par = ols + A;
+        ols = obmu + A; n_par = ols + nls;
         n_base = hw * O + hw + hw * hw + hw;
     }
-    // half 0 = actor (base at 0, head [Wmu bmu logstd] at oWmu), half 1 = critic (contiguous)
-    __host__ __device__ int half_size(int half, int hw = H) const { return n_base + (half == 0 ? A * hw + 2 * A : M * hw + M); }
+    // half 0 = actor (base at 0, head [Wmu bmu logstd] at oWmu), half 1 = critic (contiguous). CAT: a Categorical actor head
+    // [W b] has no logstd; the kernels pass the head as a compile-time flag, so the Gaussian code reads no extra field.
+    template <bool CAT = false>
+    __host__ __device__ int half_size(int half, int hw = H) const { return n_base + (half == 0 ? A * hw + (CAT ? A : 2 * A) : M * hw + M); }
     __host__ __device__ int head_dim(int half) const { return half == 0 ? A : M; }
     __host__ __device__ int half_base(int half) const { return half == 0 ? oW1a : oW1c; }
     __host__ __device__ int half_head(int half) const { return half == 0 ? oWmu : oWv; }

@@ -26,35 +26,9 @@
 #include <cooperative_groups.h>
 #include <stdlib.h>
 
-#include "net.cuh"
+#include "k3_body.cuh"
 
 namespace pgm {
-
-struct K3Args {
-    float *params, *adam_m, *adam_v;
-    int32_t *adam_step;
-    const double *lr;
-    const float *rec;       // packed records [P][S][RSG]
-    const int32_t *perm;    // [P or 1][E][S]  (update)  or  [mb] (grad mode)
-    float *losses;          // [P][3]
-    float *gpart;           // scratch: partial / reduced gradients [P][2][G][NHP]
-    float *pstage;          // scratch: updated parameters on their way to the TMA multicast [P][2][NHP] (fast path, TAIL >= 2)
-    float *ssq;             // scratch: squared-norm partials       [P][16]
-    float *lpart;           // scratch: loss partial sums           [P][16][4]
-    float *grad_out;        // grad mode only: [P][n_par]
-    float *mv;              // tensor-core path: Adam moments per half in reference order [P][2 halves][m|v][TC_NHP]
-    long long *trace;       // PGM_K3_TRACE builds only: [CTA][4 steps][16 marks] clock64 / globaltimer
-    int perm_shared, E, B, mb, S, nsteps, grad_only;
-    int Rg;                 // rows per CTA per step (multiple of the chunk size)
-    int RSG, RSS, NHP;      // record stride in global / shared memory; padded half size
-    int stage_floats;       // fast path: staging floats for row-split partials
-    int rs;                 // tensor-core path: CTAs per network half (row split), 1 or 2
-    pgm_ppo_hyper hy;
-    NetLayout L;
-};
-
-// record field offsets (floats): x[0,OP) act[OP,OP+A) logp_old v_old[M] ret[M] adv
-__host__ __device__ inline int rec_stride(const NetLayout &L) { return round_up(L.OP + L.A + 2 * L.M + 2, 4); }
 
 __global__ void k3_pack_kernel(const float *__restrict__ obs, size_t obs_ts, const float *__restrict__ action,
                                const float *__restrict__ logp, const float *__restrict__ vold, size_t v_ts,
@@ -66,7 +40,7 @@ __global__ void k3_pack_kernel(const float *__restrict__ obs, size_t obs_ts, con
         const size_t ts = i / RSG;
         const int s = (int)(ts % S);
         const int task = (int)(ts / S);
-        const int O = L.O, OP = L.OP, A = L.A, M = L.M;
+        const int O = L.O, OP = L.OP, A = L.AC, M = L.M;   // A: action columns
         float v = 0.f;
         if (f < O) v = obs[task * obs_ts + (size_t)s * O + f];
         else if (f < OP) v = 0.f;
@@ -76,540 +50,6 @@ __global__ void k3_pack_kernel(const float *__restrict__ obs, size_t obs_ts, con
         else if (f < OP + A + 1 + 2 * M) v = ret[((size_t)task * S + s) * M + (f - OP - A - 1 - M)];
         else if (f == OP + A + 1 + 2 * M) v = adv[(size_t)task * S + s];
         rec[i] = v;
-    }
-}
-
-#ifdef PGM_K3_TRACE
-#define PGM_TR(ph)                                                                                   \
-    if (a.trace && tid == 0 && s >= 8 && s < 12) {                                                   \
-        long long gt_; asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(gt_));                       \
-        a.trace[(((size_t)blockIdx.x * 4 + (s - 8)) * 16 + (ph)) * 2] = clock64();                   \
-        a.trace[(((size_t)blockIdx.x * 4 + (s - 8)) * 16 + (ph)) * 2 + 1] = gt_;                     \
-    }
-#else
-#define PGM_TR(ph)
-#endif
-
-template <int C>
-__device__ __forceinline__ void sync_group() {
-    if (C == 1) {
-        __syncthreads();
-    } else {
-        asm volatile("barrier.cluster.arrive.release.aligned;\n" ::: "memory");
-        asm volatile("barrier.cluster.wait.acquire.aligned;\n" ::: "memory");
-    }
-}
-
-template <int C>
-__device__ __forceinline__ unsigned group_rank() {
-    if (C == 1) return 0;
-    unsigned r;
-    asm volatile("mov.u32 %0, %%cluster_ctarank;\n" : "=r"(r));
-    return r;
-}
-
-// half-local flat parameter index -> offset inside the padded shared-memory image of the half
-template <int HW = H>
-__device__ __forceinline__ int half_img_off(const HalfNet &n, const NetLayout &L, int e) {
-    constexpr int LD = RowTile<HW>::LD, LOG2 = RowTile<HW>::LOG2;
-    const int O = L.O;
-    if (e < HW * O) { const int j = e / O; return j * L.ldw1 + (e - j * O); }
-    e -= HW * O;
-    if (e < HW) return (int)(n.b1 - n.W1) + e;
-    e -= HW;
-    if (e < HW * HW) return (int)(n.W2 - n.W1) + (e >> LOG2) * LD + (e & (HW - 1));
-    e -= HW * HW;
-    if (e < HW) return (int)(n.b2 - n.W1) + e;
-    e -= HW;
-    if (e < n.KH * HW) return (int)(n.Wh - n.W1) + (e >> LOG2) * LD + (e & (HW - 1));
-    e -= n.KH * HW;
-    if (e < n.KH) return (int)(n.bh - n.W1) + e;
-    return (int)(n.ls - n.W1) + (e - n.KH);
-}
-
-__device__ __forceinline__ float fast_sqrt(float x) { float r; asm("sqrt.approx.f32 %0, %1;" : "=f"(r) : "f"(x)); return r; }
-
-// C: CTAs per task; TM: rows per thread per chunk (chunk = 16*TM rows);
-// KG1: 4-column groups of dW1 per thread (OP <= 64*KG1); NA: head rows per thread (A,M <= 16*NA);
-// DB: double-buffered record gather; VU: unclipped value loss (every kernel family takes it as a template parameter, so the
-// clipped instantiations are the code they were before the option existed).
-// HW: hidden width (net.cuh RowTile). A thread's dW2 tile is CG x KQ2 quads by 4x4, its dW1 tile KG1 x CG; at HW = 32
-// the 32 k lanes cover OP <= 128 * KG1, at 64 and 128 the 16 k lanes cover OP <= 64 * KG1.
-// Generic path (any supported dims, incl. wide observations and C == 1): each CTA updates a 1/G
-// slice of its half in global memory and all CTAs reload the parameters (three barriers per step).
-// Small networks on C >= 2 take the fast path in k3_fast.cuh instead (hidden width 64).
-// The body is shared by k3_ppo_kernel (HW = 64) and k3_ppo_h_kernel (HW = 32, 128).
-template <int C, int TM, int KG1, int NA, bool DB, bool VU, int HW>
-__device__ __forceinline__ void k3_ppo_body(const K3Args &a) {
-    using T = RowTile<HW>;
-    constexpr int RC = 16 * TM;
-    constexpr int RT = T::RT, CT = T::CT, CG = T::CG, LD = T::LD, RPT = RC / RT;
-    constexpr int KQ2 = (HW / 4 + RT - 1) / RT;          // k quads of dW2 per thread
-    constexpr int NHALF = (C == 1) ? 2 : 1;
-    constexpr int G = (C == 1) ? 1 : C / 2;
-    static_assert(!(DB && NHALF == 2), "double-buffered gather needs one half per CTA");
-    static_assert(RC % RT == 0, "chunk rows must be a multiple of the row lanes");
-    extern __shared__ __align__(16) float smem[];
-    __shared__ float red[34];
-    __shared__ double sh_d[4];
-
-    const NetLayout &L = a.L;
-    const int tid = threadIdx.x, tr = tid & (RT - 1), tc = tid >> T::RT_LOG2;
-    const int task = blockIdx.x / C;
-    const unsigned rank = group_rank<C>();
-    const int half0 = (C == 1) ? 0 : (int)(rank / G);
-    const int g = (C == 1) ? 0 : (int)(rank % G);
-    const int O = L.O, OP = L.OP, A = L.A, M = L.M;
-    const int ldo = ((A > M ? A : M) | 1);
-    const int RSS = a.RSS, RSG = a.RSG;
-    const int nchunk = a.Rg / RC;
-
-    // ---- shared memory carve ----
-    HalfNet net[NHALF];
-    float *p = smem;
-#pragma unroll
-    for (int hh = 0; hh < NHALF; ++hh) p = halfnet_carve<HW>(net[hh], p, L, half0 + hh);
-    float *h1 = p; p += RC * LD;
-    float *h2 = p; p += RC * LD;
-    float *dz = p; p += RC * LD;
-    float *ho = p; p += round_up(RC * ldo, 4);
-    float *els = p; p += round_up(RC * ldo, 4);
-    float *recb = p;   // [DB ? 2 : 1][RC][RSS]
-
-    float *gparams = a.params + (size_t)task * L.n_par;
-#pragma unroll
-    for (int hh = 0; hh < NHALF; ++hh) halfnet_load<false, HW>(net[hh], gparams, L, half0 + hh);
-
-    const float clip = (float)a.hy.clip_param;
-    const float inv_mb = 1.f / (float)a.mb;
-    const float vscale = (float)(a.hy.value_loss_coef * 0.5 / ((double)a.mb * M));
-    const float omb1 = (float)(1.0 - a.hy.beta1);
-    const float b2f = (float)a.hy.beta2, omb2 = (float)(1.0 - a.hy.beta2);
-    const float aeps = (float)a.hy.adam_eps;
-    const float ecoef = (float)a.hy.entropy_coef;
-    const int step0 = a.grad_only ? 0 : a.adam_step[task];
-    double b1pow = pow(a.hy.beta1, (double)step0), b2pow = pow(a.hy.beta2, (double)step0);   // thread 0 uses them
-    const double lr = a.grad_only ? 0.0 : a.lr[task];
-
-    float loss_act = 0.f, loss_val = 0.f, loss_ent = 0.f;   // running sums (per thread)
-
-    const int32_t *perm = a.perm + ((a.perm_shared || a.grad_only) ? 0 : (size_t)task * a.E * a.S);
-    const float *recg = a.rec + (size_t)task * a.S * RSG;
-    const int q4 = RSG / 4;
-
-    // gather chunk `ci` (flat index over steps x chunks) into buffer `buf`
-    auto gather = [&](int ci, int buf) {
-        const int s = ci / nchunk, c = ci - s * nchunk;
-        const int e = s / a.B, b = s - e * a.B;
-        const int row0 = g * a.Rg + c * RC;                       // first row of this chunk inside the minibatch
-        const int32_t *pb = perm + (size_t)e * a.S + (size_t)b * a.mb;
-        float *dst = recb + buf * RC * RSS;
-        for (int i = tid; i < RC * q4; i += NTHREADS) {
-            const int r = i / q4, q = i - r * q4;
-            float *d = dst + r * RSS + 4 * q;
-            if (row0 + r < a.mb) {
-                const int idx = __ldg(pb + row0 + r);
-                cp_async16(d, recg + (size_t)idx * RSG + 4 * q);
-            } else {
-                sts4(d, make_float4(0.f, 0.f, 0.f, 0.f));
-            }
-        }
-        cp_async_commit();
-    };
-
-    const int total_chunks = a.nsteps * nchunk;
-    if (DB) gather(0, 0);
-    __syncthreads();
-
-    for (int s = 0; s < a.nsteps; ++s) {
-        PGM_TR(0)
-#pragma unroll
-        for (int hh = 0; hh < NHALF; ++hh) {
-            const int half = half0 + hh;
-            const HalfNet &n = net[hh];
-            const int KH = n.KH;
-            // gradient accumulators (registers, persist over the chunks of this step)
-            float gW2[CG][KQ2][4][4], gb2[CG][4], gW1[KG1][CG][4][4], gb1[CG][4], gWh[NA][CG][4], gbh[NA], gls[NA];
-#pragma unroll
-            for (int jg = 0; jg < CG; ++jg)
-#pragma unroll
-            for (int i = 0; i < 4; ++i) {
-                gb2[jg][i] = 0.f; gb1[jg][i] = 0.f;
-#pragma unroll
-                for (int j = 0; j < 4; ++j) {
-#pragma unroll
-                    for (int kq = 0; kq < KQ2; ++kq) gW2[jg][kq][i][j] = 0.f;
-#pragma unroll
-                    for (int q = 0; q < KG1; ++q) gW1[q][jg][i][j] = 0.f;
-                }
-            }
-#pragma unroll
-            for (int ia = 0; ia < NA; ++ia) {
-                gbh[ia] = 0.f; gls[ia] = 0.f;
-#pragma unroll
-                for (int jg = 0; jg < CG; ++jg) gWh[ia][jg][0] = gWh[ia][jg][1] = gWh[ia][jg][2] = gWh[ia][jg][3] = 0.f;
-            }
-
-            for (int c = 0; c < nchunk; ++c) {
-                const int ci = s * nchunk + c;
-                const float *x;
-                if (DB) {
-                    cp_async_wait<0>();
-                    __syncthreads();            // chunk ci landed; every thread is done with chunk ci-1
-                    if (ci + 1 < total_chunks) gather(ci + 1, (ci + 1) & 1);
-                    x = recb + (ci & 1) * RC * RSS;
-                } else {
-                    __syncthreads();            // previous users of recb are done
-                    gather(ci, 0);
-                    cp_async_wait<0>();
-                    __syncthreads();
-                    x = recb;
-                }
-                const int row0 = g * a.Rg + c * RC;
-
-                PGM_TR(1)
-                // ---------------- forward ----------------
-                half_forward<TM, HW>(x, RSS, n, L, h1, h2, ho, ldo, tr, tc);
-
-                PGM_TR(2)
-                // ---------------- loss + d(loss)/d(head output), thread per row ----------------
-                if (tid < RC) {
-                    const int r = tid;
-                    const bool valid = row0 + r < a.mb;
-                    const float *rp = x + r * RSS;
-                    if (half == 0) {
-                        float lp = 0.f;
-                        for (int d = 0; d < A; ++d) {
-                            const float ls = n.ls[d], sd = expf(ls);
-                            const float diff = rp[OP + d] - ho[r * ldo + d];
-                            lp += -(diff * diff) / (2.f * sd * sd) - ls - 0.91893853320467274178f;
-                        }
-                        const float ratio = expf(lp - rp[OP + A]);
-                        const float adv = rp[OP + A + 1 + 2 * M];
-                        const float surr1 = ratio * adv;
-                        const float rcl = fminf(fmaxf(ratio, 1.f - clip), 1.f + clip);
-                        const float surr2 = rcl * adv;
-                        const float w1 = surr1 < surr2 ? 1.f : (surr1 == surr2 ? 0.5f : 0.f);
-                        const float inr = (ratio >= 1.f - clip && ratio <= 1.f + clip) ? 1.f : 0.f;
-                        const float dmin = w1 * adv + (1.f - w1) * adv * inr;
-                        const float dlp = valid ? -inv_mb * dmin * ratio : 0.f;
-                        if (valid) loss_act -= fminf(surr1, surr2);
-                        for (int d = 0; d < A; ++d) {
-                            const float sd = expf(n.ls[d]);
-                            const float iv = 1.f / (sd * sd);
-                            const float diff = rp[OP + d] - ho[r * ldo + d];
-                            ho[r * ldo + d] = dlp * diff * iv;
-                            els[r * ldo + d] = dlp * (diff * diff * iv - 1.f);
-                        }
-                    } else {
-                        for (int m = 0; m < M; ++m) {
-                            const float V = ho[r * ldo + m];
-                            const float vo = rp[OP + A + 1 + m];
-                            const float R = rp[OP + A + 1 + M + m];
-                            const float d = V - vo;
-                            const float vcl = vo + fminf(fmaxf(d, -clip), clip);
-                            const float ea = V - R, eb = vcl - R;
-                            // unclipped value loss (VU): lb = -1 < 0 <= la, so max(la, lb) = la and wa = 1, gradient 2 * ea exactly
-                            const float la = ea * ea, lb = VU ? -1.f : eb * eb;
-                            const float wa = la > lb ? 1.f : (la == lb ? 0.5f : 0.f);
-                            const float pas = (d >= -clip && d <= clip) ? 1.f : 0.f;
-                            if (valid) loss_val += fmaxf(la, lb);
-                            ho[r * ldo + m] = valid ? vscale * (wa * 2.f * ea + (1.f - wa) * 2.f * eb * pas) : 0.f;
-                        }
-                    }
-                }
-                __syncthreads();
-
-                PGM_TR(3)
-                // ---------------- phase A: head weight grads, dz2 ----------------
-                {
-                    const int kg = tid & (CT - 1), a0 = tid >> T::CT_LOG2;
-#pragma unroll
-                    for (int ia = 0; ia < NA; ++ia) {
-                        const int aa = a0 + RT * ia;
-                        if (aa < KH) {
-#pragma unroll 4
-                            for (int r = 0; r < RC; ++r) {
-                                const float sv = ho[r * ldo + aa];
-#pragma unroll
-                                for (int jg = 0; jg < CG; ++jg) {
-                                    const float4 hv = lds4(h2 + r * LD + 4 * (kg + CT * jg));
-                                    float *gw = gWh[ia][jg];
-                                    gw[0] = fmaf(sv, hv.x, gw[0]); gw[1] = fmaf(sv, hv.y, gw[1]);
-                                    gw[2] = fmaf(sv, hv.z, gw[2]); gw[3] = fmaf(sv, hv.w, gw[3]);
-                                }
-                                if (kg == 0) gbh[ia] += sv;
-                                if (half == 0 && kg == 1) gls[ia] += els[r * ldo + aa];
-                            }
-                        }
-                    }
-                    float acc[RPT][CG][4];
-#pragma unroll
-                    for (int i = 0; i < RPT; ++i)
-#pragma unroll
-                        for (int jg = 0; jg < CG; ++jg) acc[i][jg][0] = acc[i][jg][1] = acc[i][jg][2] = acc[i][jg][3] = 0.f;
-                    for (int aa = 0; aa < KH; ++aa) {
-#pragma unroll
-                        for (int jg = 0; jg < CG; ++jg) {
-                            const float4 w = lds4(n.Wh + aa * LD + 4 * (tc + CT * jg));
-#pragma unroll
-                            for (int i = 0; i < RPT; ++i) {
-                                const float sv = ho[(tr + RT * i) * ldo + aa];
-                                float *ac = acc[i][jg];
-                                ac[0] = fmaf(sv, w.x, ac[0]); ac[1] = fmaf(sv, w.y, ac[1]);
-                                ac[2] = fmaf(sv, w.z, ac[2]); ac[3] = fmaf(sv, w.w, ac[3]);
-                            }
-                        }
-                    }
-#pragma unroll
-                    for (int i = 0; i < RPT; ++i)
-#pragma unroll
-                    for (int jg = 0; jg < CG; ++jg) {
-                        const int o = (tr + RT * i) * LD + 4 * (tc + CT * jg);
-                        const float4 hv = lds4(h2 + o);
-                        const float *ac = acc[i][jg];
-                        sts4(dz + o, make_float4(ac[0] * (1.f - hv.x * hv.x), ac[1] * (1.f - hv.y * hv.y),
-                                                 ac[2] * (1.f - hv.z * hv.z), ac[3] * (1.f - hv.w * hv.w)));
-                    }
-                }
-                __syncthreads();
-
-                PGM_TR(4)
-                // ---------------- phase B: dW2, db2, dz1 (into the h2 buffer) ----------------
-                {
-                    const int tj = tid & (CT - 1), tk = tid >> T::CT_LOG2;
-#pragma unroll 4
-                    for (int r = 0; r < RC; ++r) {
-#pragma unroll
-                        for (int jg = 0; jg < CG; ++jg) {
-                            const float4 dv = lds4(dz + r * LD + 4 * (tj + CT * jg));
-                            const float dd[4] = {dv.x, dv.y, dv.z, dv.w};
-#pragma unroll
-                            for (int kq = 0; kq < KQ2; ++kq) {
-                                if (4 * RT * KQ2 > HW && 4 * (tk + RT * kq) >= HW) continue;   // idle k lanes at HW = 32
-                                const float4 hv = lds4(h1 + r * LD + 4 * (tk + RT * kq));
-#pragma unroll
-                                for (int jj = 0; jj < 4; ++jj) {
-                                    float *gw = gW2[jg][kq][jj];
-                                    gw[0] = fmaf(dd[jj], hv.x, gw[0]); gw[1] = fmaf(dd[jj], hv.y, gw[1]);
-                                    gw[2] = fmaf(dd[jj], hv.z, gw[2]); gw[3] = fmaf(dd[jj], hv.w, gw[3]);
-                                }
-                            }
-                            if (tk == 0) { gb2[jg][0] += dv.x; gb2[jg][1] += dv.y; gb2[jg][2] += dv.z; gb2[jg][3] += dv.w; }
-                        }
-                    }
-                    float acc[RPT][CG][4];
-#pragma unroll
-                    for (int i = 0; i < RPT; ++i)
-#pragma unroll
-                        for (int jg = 0; jg < CG; ++jg) acc[i][jg][0] = acc[i][jg][1] = acc[i][jg][2] = acc[i][jg][3] = 0.f;
-#pragma unroll 2
-                    for (int j = 0; j < HW; j += 4) {
-                        float4 av[RPT], bv[CG][4];
-#pragma unroll
-                        for (int i = 0; i < RPT; ++i) av[i] = lds4(dz + (tr + RT * i) * LD + j);
-#pragma unroll
-                        for (int jg = 0; jg < CG; ++jg)
-#pragma unroll
-                            for (int jj = 0; jj < 4; ++jj) bv[jg][jj] = lds4(n.W2 + (j + jj) * LD + 4 * (tc + CT * jg));
-#pragma unroll
-                        for (int i = 0; i < RPT; ++i) {
-                            const float aa[4] = {av[i].x, av[i].y, av[i].z, av[i].w};
-#pragma unroll
-                            for (int jg = 0; jg < CG; ++jg)
-#pragma unroll
-                            for (int jj = 0; jj < 4; ++jj) {
-                                float *ac = acc[i][jg];
-                                ac[0] = fmaf(aa[jj], bv[jg][jj].x, ac[0]); ac[1] = fmaf(aa[jj], bv[jg][jj].y, ac[1]);
-                                ac[2] = fmaf(aa[jj], bv[jg][jj].z, ac[2]); ac[3] = fmaf(aa[jj], bv[jg][jj].w, ac[3]);
-                            }
-                        }
-                    }
-#pragma unroll
-                    for (int i = 0; i < RPT; ++i)
-#pragma unroll
-                    for (int jg = 0; jg < CG; ++jg) {
-                        const int o = (tr + RT * i) * LD + 4 * (tc + CT * jg);
-                        const float4 hv = lds4(h1 + o);
-                        const float *ac = acc[i][jg];
-                        sts4(h2 + o, make_float4(ac[0] * (1.f - hv.x * hv.x), ac[1] * (1.f - hv.y * hv.y),
-                                                 ac[2] * (1.f - hv.z * hv.z), ac[3] * (1.f - hv.w * hv.w)));
-                    }
-                }
-                __syncthreads();
-
-                PGM_TR(5)
-                // ---------------- phase C: dW1, db1 ----------------
-                {
-                    const int tj = tid & (CT - 1), tk = tid >> T::CT_LOG2;
-#pragma unroll
-                    for (int q = 0; q < KG1; ++q) {
-                        const int k0 = 4 * (tk + RT * q);
-                        if (k0 < OP) {
-#pragma unroll 4
-                            for (int r = 0; r < RC; ++r) {
-#pragma unroll
-                                for (int jg = 0; jg < CG; ++jg) {
-                                    const float4 dv = lds4(h2 + r * LD + 4 * (tj + CT * jg));
-                                    const float4 xv = lds4(x + r * RSS + k0);
-                                    const float dd[4] = {dv.x, dv.y, dv.z, dv.w};
-#pragma unroll
-                                    for (int jj = 0; jj < 4; ++jj) {
-                                        float *gw = gW1[q][jg][jj];
-                                        gw[0] = fmaf(dd[jj], xv.x, gw[0]); gw[1] = fmaf(dd[jj], xv.y, gw[1]);
-                                        gw[2] = fmaf(dd[jj], xv.z, gw[2]); gw[3] = fmaf(dd[jj], xv.w, gw[3]);
-                                    }
-                                    if (q == 0 && tk == 0) { gb1[jg][0] += dv.x; gb1[jg][1] += dv.y; gb1[jg][2] += dv.z; gb1[jg][3] += dv.w; }
-                                }
-                            }
-                        }
-                    }
-                }
-                // no barrier needed here: the next chunk's forward (or the barrier below) orders
-                // the reuse of h2 / x behind every thread's phase C
-            }
-
-            PGM_TR(6)
-            // ---- write this CTA's partial gradient of `half` to its scratch slot ----
-            {
-                float *gp = a.gpart + ((size_t)(task * 2 + half) * G + g) * a.NHP;
-                const int tj = tid & (CT - 1), tk = tid >> T::CT_LOG2;
-                const int lb1 = HW * O, lW2 = lb1 + HW, lb2 = lW2 + HW * HW, lWh = lb2 + HW, lbh = lWh + KH * HW, lls = lbh + KH;
-#pragma unroll
-                for (int q = 0; q < KG1; ++q)
-#pragma unroll
-                    for (int jg = 0; jg < CG; ++jg)
-#pragma unroll
-                    for (int jj = 0; jj < 4; ++jj)
-#pragma unroll
-                        for (int kk = 0; kk < 4; ++kk) {
-                            const int k = 4 * (tk + RT * q) + kk;
-                            if (k < O) gp[(4 * (tj + CT * jg) + jj) * O + k] = gW1[q][jg][jj][kk];
-                        }
-#pragma unroll
-                for (int jg = 0; jg < CG; ++jg)
-#pragma unroll
-                    for (int kq = 0; kq < KQ2; ++kq) {
-                        if (4 * RT * KQ2 > HW && 4 * (tk + RT * kq) >= HW) continue;
-#pragma unroll
-                        for (int jj = 0; jj < 4; ++jj) {
-                            const float *gw = gW2[jg][kq][jj];
-                            sts4(gp + lW2 + (4 * (tj + CT * jg) + jj) * HW + 4 * (tk + RT * kq), make_float4(gw[0], gw[1], gw[2], gw[3]));
-                        }
-                    }
-                if (tk == 0) {
-#pragma unroll
-                    for (int jg = 0; jg < CG; ++jg) {
-                        sts4(gp + lb1 + 4 * (tj + CT * jg), make_float4(gb1[jg][0], gb1[jg][1], gb1[jg][2], gb1[jg][3]));
-                        sts4(gp + lb2 + 4 * (tj + CT * jg), make_float4(gb2[jg][0], gb2[jg][1], gb2[jg][2], gb2[jg][3]));
-                    }
-                }
-                const int kg = tid & (CT - 1), a0 = tid >> T::CT_LOG2;
-#pragma unroll
-                for (int ia = 0; ia < NA; ++ia) {
-                    const int aa = a0 + RT * ia;
-                    if (aa < KH) {
-#pragma unroll
-                        for (int jg = 0; jg < CG; ++jg)
-                            sts4(gp + lWh + aa * HW + 4 * (kg + CT * jg), make_float4(gWh[ia][jg][0], gWh[ia][jg][1], gWh[ia][jg][2], gWh[ia][jg][3]));
-                        if (kg == 0) gp[lbh + aa] = gbh[ia];
-                        if (half == 0 && kg == 1) gp[lls + aa] = gls[ia];
-                    }
-                }
-            }
-            if (half == 0 && g == 0 && tid == 0) {   // entropy with the parameters this step started from
-                float ent = 0.f;
-                for (int d = 0; d < A; ++d) ent += 0.5f + 0.91893853320467274178f + n.ls[d];
-                loss_ent += ent;
-            }
-        }   // halves
-
-        PGM_TR(7)
-        sync_group<C>();   // (1) all partial gradients of this task are in L2
-        PGM_TR(8)
-
-        // ---- reduce my slice over the G partials, squared-norm partial ----
-        float sq = 0.f;
-#pragma unroll
-        for (int hh = 0; hh < NHALF; ++hh) {
-            const int half = half0 + hh;
-            const int nH = L.half_size(half, HW);
-            const int per = round_up((nH + G - 1) / G, 4);
-            const int s0 = g * per, s1 = min(nH, s0 + per);
-            float *slot0 = a.gpart + (size_t)(task * 2 + half) * G * a.NHP;
-            const int lls = L.n_base + L.head_dim(half) * HW + L.head_dim(half);
-            for (int e = s0 + tid; e < s1; e += NTHREADS) {
-                float gs = 0.f;
-#pragma unroll
-                for (int gg = 0; gg < G; ++gg) gs += __ldcg(slot0 + (size_t)gg * a.NHP + e);
-                if (half == 0 && e >= lls) gs -= ecoef;      // d(-ecoef * entropy)/d logstd
-                sq = fmaf(gs, gs, sq);
-                if (a.grad_only) a.grad_out[(size_t)task * L.n_par + L.to_global(half, e)] = gs;
-                else slot0[(size_t)g * a.NHP + e] = gs;   // keep the reduced value in my own slot (only I read it)
-            }
-        }
-        sq = block_sum(sq, red);
-        if (tid == 0) a.ssq[task * 16 + rank] = sq;
-        if (a.grad_only) break;
-
-        if (tid == 0) {   // Adam scalars of step k = step0 + s + 1, in double
-            b1pow *= a.hy.beta1; b2pow *= a.hy.beta2;
-            sh_d[0] = lr / (1.0 - b1pow);            // step_size
-            sh_d[1] = 1.0 / sqrt(1.0 - b2pow);       // 1 / bias_correction2_sqrt
-        }
-        sync_group<C>();   // (2) squared-norm partials visible
-
-        float tot = 0.f;
-#pragma unroll
-        for (int rr = 0; rr < C; ++rr) tot += __ldcg(a.ssq + task * 16 + rr);
-        const float coef = fminf(1.f, (float)a.hy.max_grad_norm / (sqrtf(tot) + 1e-6f));
-        const float step_size = (float)sh_d[0], ibc2 = (float)sh_d[1];
-#pragma unroll
-        for (int hh = 0; hh < NHALF; ++hh) {
-            const int half = half0 + hh;
-            const int nH = L.half_size(half, HW);
-            const int per = round_up((nH + G - 1) / G, 4);
-            const int s0 = g * per, s1 = min(nH, s0 + per);
-            const float *mine = a.gpart + ((size_t)(task * 2 + half) * G + g) * a.NHP;
-            for (int e = s0 + tid; e < s1; e += NTHREADS) {
-                const size_t gi = (size_t)task * L.n_par + L.to_global(half, e);
-                const float gr = __ldcg(mine + e) * coef;
-                float m = a.adam_m[gi], v = a.adam_v[gi], pw = a.params[gi];
-                m = fmaf(gr - m, omb1, m);                 // exp_avg.lerp_(grad, 1 - beta1)
-                v = fmaf(omb2 * gr, gr, v * b2f);          // exp_avg_sq.mul_(beta2).addcmul_(grad, grad, 1 - beta2)
-                const float denom = sqrtf(v) * ibc2 + aeps;
-                pw -= step_size * (m / denom);
-                a.adam_m[gi] = m; a.adam_v[gi] = v; a.params[gi] = pw;
-            }
-        }
-        sync_group<C>();   // (3) new parameters of this task are in L2
-#pragma unroll
-        for (int hh = 0; hh < NHALF; ++hh) halfnet_load<true, HW>(net[hh], gparams, L, half0 + hh);
-        __syncthreads();
-    }
-
-    // ---- losses: per-CTA partial sums -> rank 0 combines in fixed order ----
-    {
-        const float la = block_sum(loss_act, red), lv = block_sum(loss_val, red), le = block_sum(loss_ent, red);
-        if (tid == 0) {
-            a.lpart[(task * 16 + rank) * 4 + 0] = lv;
-            a.lpart[(task * 16 + rank) * 4 + 1] = la;
-            a.lpart[(task * 16 + rank) * 4 + 2] = le;
-        }
-        sync_group<C>();
-        if (rank == 0 && tid == 0) {
-            float sv = 0.f, sa = 0.f, se = 0.f;
-            for (int rr = 0; rr < C; ++rr) {
-                sv += __ldcg(a.lpart + (task * 16 + rr) * 4 + 0);
-                sa += __ldcg(a.lpart + (task * 16 + rr) * 4 + 1);
-                se += __ldcg(a.lpart + (task * 16 + rr) * 4 + 2);
-            }
-            const float ns = (float)a.nsteps;
-            a.losses[task * 3 + 0] = sv * 0.5f / ((float)a.mb * M) / ns;
-            a.losses[task * 3 + 1] = sa * inv_mb / ns;
-            a.losses[task * 3 + 2] = se / ns;
-            if (!a.grad_only) a.adam_step[task] = step0 + a.nsteps;
-        }
     }
 }
 
@@ -633,6 +73,7 @@ struct K3Plan {
     bool DB, fast, tc, tcw;
     bool vu;      // unclipped value loss (PGM_PPO_VALUE_UNCLIPPED): the VU = true instantiation of the chosen kernel
     int hidden;   // hidden width: 64, or 32 / 128 (generic kernel k3_ppo_h_kernel only)
+    bool cat;     // Categorical head: the generic kernel k3_ppo_cat_kernel (k3_cat.cu) at every width
     int tail;     // fast path step tail (k3_fast.cuh): 0 three cluster barriers, 1 redundant Adam, 2 TMA multicast broadcast
     int rs;
     int stage_floats;
@@ -717,15 +158,24 @@ constexpr int K3_CLUSTER_TAILEP = 0x4000;  // tail 6
 constexpr int K3_CLUSTER_FLAGS = K3_CLUSTER_TAIL2 | K3_CLUSTER_TAILMC | K3_CLUSTER_TAILGL | K3_CLUSTER_TAIL0 | K3_CLUSTER_TAILBP |
                                  K3_CLUSTER_TAILNB | K3_CLUSTER_TAILEP | PGM_PPO_VALUE_UNCLIPPED;
 
-static int k3_plan(K3Plan &pl, int P, int S, int mb, int O, int A, int M, int cluster, int sms, int hidden) {
-    NetLayout L(O, A, M, hidden);
+static int k3_plan(K3Plan &pl, int P, int S, int mb, int O, int A, int M, int cluster, int sms, int hidden, int dist) {
+    NetLayout L(O, A, M, hidden, dist);
+    const bool cat = dist == PGM_DIST_CATEGORICAL;
     const bool tail2 = (cluster & K3_CLUSTER_TAIL2) != 0, tailmc = (cluster & K3_CLUSTER_TAILMC) != 0;
     const bool tailgl = (cluster & K3_CLUSTER_TAILGL) != 0, tail0 = (cluster & K3_CLUSTER_TAIL0) != 0;
     const bool tailbp = (cluster & K3_CLUSTER_TAILBP) != 0, tailnb = (cluster & K3_CLUSTER_TAILNB) != 0;
     const bool tailep = (cluster & K3_CLUSTER_TAILEP) != 0;
     pl.vu = (cluster & PGM_PPO_VALUE_UNCLIPPED) != 0;
     cluster &= ~K3_CLUSTER_FLAGS;
-    pl.tc = false; pl.tcw = false; pl.tail = 0; pl.off_mv = 0; pl.hidden = hidden;
+    pl.tc = false; pl.tcw = false; pl.tail = 0; pl.off_mv = 0; pl.hidden = hidden; pl.cat = cat;
+    // Categorical heads run on the generic cluster kernel only, at every hidden width
+    if (cat) {
+        PGM_REQUIRE(A >= 1 && A <= CAT_MAX, "ppo: a categorical head has 1..%d categories, got %d", CAT_MAX, A);
+        PGM_REQUIRE(cluster != K3_CLUSTER_TC && cluster != K3_CLUSTER_TC2 && cluster != K3_CLUSTER_TC4,
+                    "ppo: the tensor-core paths (cluster 32, 64, 128) are built for Gaussian heads, got a categorical head");
+        PGM_REQUIRE(cluster != 1, "ppo: cluster 1 (both halves in one CTA) is built for Gaussian heads, got a categorical "
+                    "head (use cluster 0, 2, 4, 8 or 16)");
+    }
     // the tensor-core kernels, the fast cluster kernel and cluster = 1 are built for hidden width 64; other widths run on
     // the generic cluster kernel at 2..16 CTAs per task
     if (hidden != H) {
@@ -735,7 +185,7 @@ static int k3_plan(K3Plan &pl, int P, int S, int mb, int O, int A, int M, int cl
                     "(use cluster 0, 2, 4, 8 or 16)", hidden);
     }
     // wide observations (Humanoid): the streamed tensor-core kernel; row split over as many CTAs per half as fill the SMs
-    if (hidden == H && k3_tcw_dims(O, A, M) && (cluster == 0 || cluster == K3_CLUSTER_TC || cluster == K3_CLUSTER_TC2 || cluster == K3_CLUSTER_TC4)) {
+    if (hidden == H && !cat && k3_tcw_dims(O, A, M) && (cluster == 0 || cluster == K3_CLUSTER_TC || cluster == K3_CLUSTER_TC2 || cluster == K3_CLUSTER_TC4)) {
         const int tiles = (mb + 127) / 128;
         if (cluster == 0) {
             // most CTAs per task whose clusters are all resident at once (a second wave of clusters doubles the step)
@@ -768,7 +218,7 @@ static int k3_plan(K3Plan &pl, int P, int S, int mb, int O, int A, int M, int cl
     }
     // auto: the tensor-core path wins as soon as the FFMA path can no longer give every task a 16-CTA cluster (measured on
     // a B200, profiles/k3_sweep.py: 1.2x at P = 8, 2.4x at 16, 3.3x from 37 tasks on; below 8 tasks FFMA is 6 % faster)
-    if (hidden == H && cluster == 0 && k3_tc_dims(O, A, M) && P >= 8) {
+    if (hidden == H && !cat && cluster == 0 && k3_tc_dims(O, A, M) && P >= 8) {
         // 4 CTAs per task (row tiles split over two CTAs per half) while they fit in one wave: 4-CTA clusters tile the 148
         // SMs less densely than pairs (measured: 32 clusters run in one wave, 37 need two)
         cluster = (mb > 128 && 4 * P <= sms - 20) ? K3_CLUSTER_TC2 : K3_CLUSTER_TC;
@@ -826,7 +276,7 @@ static int k3_plan(K3Plan &pl, int P, int S, int mb, int O, int A, int M, int cl
         pl.NHP = round_up(i0 > i1 ? i0 : i1, 64);   // covers both the reference-order half and its padded image
     }
     pl.DB = (C > 1) && !big;
-    pl.fast = hidden == H && (C > 1) && !big && L.OP <= 48 && pl.RC * (pl.RSG / 4) <= 4 * NTHREADS;
+    pl.fast = hidden == H && !cat && (C > 1) && !big && L.OP <= 48 && pl.RC * (pl.RSG / 4) <= 4 * NTHREADS;
     pl.stage_floats = 0;
     if (pl.fast) {
         const int s0 = k3_fast_stage_floats(L.OP, A), s1 = k3_fast_stage_floats(L.OP, M);
@@ -955,6 +405,7 @@ static int k3_launch_w(Kern kern, const K3Args &a, const TwExtra &x, const K3Pla
 
 template <bool VU>
 static int k3_launch(const K3Args &a, const K3Plan &pl, int P, cudaStream_t st) {
+    if (pl.cat) return k3_launch_cat(a, pl.hidden, pl.C, pl.TM, pl.KG1 > 1, VU, pl.smem, P, st);
     if (pl.hidden == 32) return k3_launch_h<32, VU>(a, pl, P, st);
     if (pl.hidden == 128) return k3_launch_h<128, VU>(a, pl, P, st);
     if (pl.tc) {
@@ -998,10 +449,11 @@ static size_t g_last_trace_offset = 0;
 extern "C" size_t pgm_ppo_last_trace_offset() { return g_last_trace_offset; }
 #endif
 
-extern "C" size_t pgm_ppo_workspace_bytes_h(int P, int S, int O, int A, int M, int cluster, int hidden) {
+extern "C" size_t pgm_ppo_workspace_bytes_x(int P, int S, int O, int A, int M, int cluster, int hidden, int dist) {
     // upper bound over every plan the launcher may choose for these dims (cluster 0 = auto)
-    if (!hidden_supported(hidden)) return 0;
-    NetLayout L(O, A, M, hidden);
+    if (!hidden_supported(hidden) || !dist_supported(dist)) return 0;
+    const bool cat = dist == PGM_DIST_CATEGORICAL;
+    NetLayout L(O, A, M, hidden, dist);
     cluster &= ~K3_CLUSTER_FLAGS;
     const int G = cluster == 0 ? 8 : (cluster == 1 ? 1 : cluster / 2);
     const int i0 = halfnet_smem_floats(L, 0, hidden), i1 = halfnet_smem_floats(L, 1, hidden);
@@ -1012,12 +464,16 @@ extern "C" size_t pgm_ppo_workspace_bytes_h(int P, int S, int O, int A, int M, i
     seg((size_t)P * 2 * (G + 1) * NHP * sizeof(float));
     seg((size_t)P * 16 * sizeof(float));
     seg((size_t)P * 64 * sizeof(float));
-    if (hidden == H && k3_tc_dims(O, A, M)) seg(k3_tc_mv_bytes(P));
-    if (hidden == H && k3_tcw_dims(O, A, M)) seg(k3_tcw_bytes(P, S, O, A, nullptr, nullptr, nullptr, nullptr) + 1024);
+    if (hidden == H && !cat && k3_tc_dims(O, A, M)) seg(k3_tc_mv_bytes(P));
+    if (hidden == H && !cat && k3_tcw_dims(O, A, M)) seg(k3_tcw_bytes(P, S, O, A, nullptr, nullptr, nullptr, nullptr) + 1024);
 #ifdef PGM_K3_TRACE
     seg((size_t)P * 16 * 4 * 16 * 2 * sizeof(long long));
 #endif
     return t;
+}
+
+extern "C" size_t pgm_ppo_workspace_bytes_h(int P, int S, int O, int A, int M, int cluster, int hidden) {
+    return pgm_ppo_workspace_bytes_x(P, S, O, A, M, cluster, hidden, PGM_DIST_GAUSSIAN);
 }
 
 extern "C" size_t pgm_ppo_workspace_bytes(int P, int S, int O, int A, int M, int cluster) {
@@ -1029,16 +485,17 @@ static int ppo_common(float *params, float *adam_m, float *adam_v, int32_t *adam
                       const float *value_old, size_t v_ts, const float *returns, const float *adv,
                       const int32_t *perm, int perm_shared, int E, int B, int mb, const pgm_ppo_hyper *hy,
                       float *losses, float *grad_out, void *workspace, size_t wbytes, int cluster, int P, int S,
-                      int O, int A, int M, int hidden, cudaStream_t st) {
+                      int O, int A, int M, int hidden, int dist, cudaStream_t st) {
     PGM_REQUIRE(params && obs && action && logp_old && value_old && returns && adv && perm && hy && losses && workspace,
                 "ppo: null pointer argument");
     PGM_REQUIRE(hidden_supported(hidden), "ppo: hidden width %d is not one of {32, 64, 128}", hidden);
+    PGM_REQUIRE(dist_supported(dist), "ppo: unknown action head %d", dist);
     PGM_REQUIRE(P > 0 && S > 0 && mb > 0 && mb <= S, "ppo: bad sizes P=%d S=%d mb=%d", P, S, mb);
     PGM_REQUIRE(((uintptr_t)workspace & 255) == 0, "ppo: workspace must be 256-byte aligned");
     int sms = 148;
     if (int rc = sm_count(sms)) return rc;
     K3Plan pl;
-    if (int rc = k3_plan(pl, P, S, mb, O, A, M, cluster, sms, hidden)) return rc;
+    if (int rc = k3_plan(pl, P, S, mb, O, A, M, cluster, sms, hidden, dist)) return rc;
     if (pl.total > wbytes) {
         set_error("ppo: workspace too small: need %zu bytes, got %zu", pl.total, wbytes);
         return PGM_ERR_WORKSPACE;
@@ -1057,7 +514,7 @@ static int ppo_common(float *params, float *adam_m, float *adam_v, int32_t *adam
     a.mv = (float *)(ws + pl.off_mv);
     a.grad_out = grad_out; a.perm_shared = perm_shared; a.E = E; a.B = B; a.mb = mb; a.S = S;
     a.grad_only = grad_out != nullptr; a.nsteps = a.grad_only ? 1 : E * B;
-    a.Rg = pl.Rg; a.RSG = pl.RSG; a.RSS = pl.RSS; a.NHP = pl.NHP; a.stage_floats = pl.stage_floats; a.rs = pl.rs; a.hy = *hy; a.L = NetLayout(O, A, M, hidden);
+    a.Rg = pl.Rg; a.RSG = pl.RSG; a.RSS = pl.RSS; a.NHP = pl.NHP; a.stage_floats = pl.stage_floats; a.rs = pl.rs; a.hy = *hy; a.L = NetLayout(O, A, M, hidden, dist);
     if (pl.tcw) {
         TwExtra x;
         x.xp = (const __half *)(ws + pl.off_xp); x.scr = (const float *)(ws + pl.off_scr);
@@ -1085,13 +542,13 @@ static int ppo_common(float *params, float *adam_m, float *adam_v, int32_t *adam
     return pl.vu ? k3_launch<true>(a, pl, P, st) : k3_launch<false>(a, pl, P, st);
 }
 
-extern "C" int pgm_ppo_update_h_f32(float *params, float *adam_m, float *adam_v, int32_t *adam_step, const double *lr,
+extern "C" int pgm_ppo_update_x_f32(float *params, float *adam_m, float *adam_v, int32_t *adam_step, const double *lr,
                                     const float *obs, size_t obs_task_stride, const float *action,
                                     const float *logp_old, const float *value_old, size_t value_task_stride,
                                     const float *returns, const float *adv, const int32_t *perm, int perm_shared,
                                     int E, int B, const pgm_ppo_hyper *hyper_host, float *losses, void *workspace,
                                     size_t workspace_bytes, int cluster, int P, int S, int O, int A, int M, int hidden,
-                                    void *stream) {
+                                    int dist, void *stream) {
     PGM_REQUIRE(adam_m && adam_v && adam_step && lr, "pgm_ppo_update_f32: null optimizer state");
     PGM_REQUIRE(E > 0 && B > 0 && S / B > 0, "pgm_ppo_update_f32: bad E=%d B=%d for S=%d", E, B, S);
     // the reference's BatchSampler(drop_last=True) yields S // (S // B) minibatches per epoch (a2c/storage.py:133-137), which
@@ -1100,7 +557,19 @@ extern "C" int pgm_ppo_update_h_f32(float *params, float *adam_m, float *adam_v,
                 "minibatch: the reference would run %d minibatches per epoch; choose S, B with S %% B < S / B", S, B, S / B, S % B, S / (S / B));
     return ppo_common(params, adam_m, adam_v, adam_step, lr, obs, obs_task_stride, action, logp_old, value_old,
                       value_task_stride, returns, adv, perm, perm_shared, E, B, S / B, hyper_host, losses, nullptr,
-                      workspace, workspace_bytes, cluster, P, S, O, A, M, hidden, (cudaStream_t)stream);
+                      workspace, workspace_bytes, cluster, P, S, O, A, M, hidden, dist, (cudaStream_t)stream);
+}
+
+extern "C" int pgm_ppo_update_h_f32(float *params, float *adam_m, float *adam_v, int32_t *adam_step, const double *lr,
+                                    const float *obs, size_t obs_task_stride, const float *action,
+                                    const float *logp_old, const float *value_old, size_t value_task_stride,
+                                    const float *returns, const float *adv, const int32_t *perm, int perm_shared,
+                                    int E, int B, const pgm_ppo_hyper *hyper_host, float *losses, void *workspace,
+                                    size_t workspace_bytes, int cluster, int P, int S, int O, int A, int M, int hidden,
+                                    void *stream) {
+    return pgm_ppo_update_x_f32(params, adam_m, adam_v, adam_step, lr, obs, obs_task_stride, action, logp_old, value_old,
+                                value_task_stride, returns, adv, perm, perm_shared, E, B, hyper_host, losses, workspace,
+                                workspace_bytes, cluster, P, S, O, A, M, hidden, PGM_DIST_GAUSSIAN, stream);
 }
 
 extern "C" int pgm_ppo_update_f32(float *params, float *adam_m, float *adam_v, int32_t *adam_step, const double *lr,
@@ -1115,16 +584,27 @@ extern "C" int pgm_ppo_update_f32(float *params, float *adam_m, float *adam_v, i
                                 workspace_bytes, cluster, P, S, O, A, M, H, stream);
 }
 
+extern "C" int pgm_ppo_grad_x_f32(const float *params, const float *obs, size_t obs_task_stride, const float *action,
+                                  const float *logp_old, const float *value_old, size_t value_task_stride,
+                                  const float *returns, const float *adv, const int32_t *idx, int mb,
+                                  const pgm_ppo_hyper *hyper_host, float *grad, float *losses, void *workspace,
+                                  size_t workspace_bytes, int cluster, int P, int S, int O, int A, int M, int hidden,
+                                  int dist, void *stream) {
+    PGM_REQUIRE(grad, "pgm_ppo_grad_f32: null grad");
+    return ppo_common(const_cast<float *>(params), nullptr, nullptr, nullptr, nullptr, obs, obs_task_stride, action,
+                      logp_old, value_old, value_task_stride, returns, adv, idx, 1, 1, 1, mb, hyper_host, losses, grad,
+                      workspace, workspace_bytes, cluster, P, S, O, A, M, hidden, dist, (cudaStream_t)stream);
+}
+
 extern "C" int pgm_ppo_grad_h_f32(const float *params, const float *obs, size_t obs_task_stride, const float *action,
                                   const float *logp_old, const float *value_old, size_t value_task_stride,
                                   const float *returns, const float *adv, const int32_t *idx, int mb,
                                   const pgm_ppo_hyper *hyper_host, float *grad, float *losses, void *workspace,
                                   size_t workspace_bytes, int cluster, int P, int S, int O, int A, int M, int hidden,
                                   void *stream) {
-    PGM_REQUIRE(grad, "pgm_ppo_grad_f32: null grad");
-    return ppo_common(const_cast<float *>(params), nullptr, nullptr, nullptr, nullptr, obs, obs_task_stride, action,
-                      logp_old, value_old, value_task_stride, returns, adv, idx, 1, 1, 1, mb, hyper_host, losses, grad,
-                      workspace, workspace_bytes, cluster, P, S, O, A, M, hidden, (cudaStream_t)stream);
+    return pgm_ppo_grad_x_f32(params, obs, obs_task_stride, action, logp_old, value_old, value_task_stride, returns, adv,
+                              idx, mb, hyper_host, grad, losses, workspace, workspace_bytes, cluster, P, S, O, A, M, hidden,
+                              PGM_DIST_GAUSSIAN, stream);
 }
 
 extern "C" int pgm_ppo_grad_f32(const float *params, const float *obs, size_t obs_task_stride, const float *action,

@@ -32,7 +32,7 @@ struct HalfNet {           // pointers into shared memory
     float *b2;             // [HW]
     float *Wh;             // [KH][HW+4]   head: fc_mean (actor) or critic_linear (critic)
     float *bh;             // [KH]
-    float *ls;             // [A] logstd (actor only)
+    float *ls;             // [A] logstd (actor only; not loaded for a Categorical head)
     int KH;
 };
 
@@ -61,7 +61,8 @@ __device__ __forceinline__ float ldp(const float *p) { return CG ? __ldcg(p) : _
 
 // Copy one half's parameters from the flat global vector `g` (reference order) into the padded
 // shared-memory image. CG=true reads through L2 only (other CTAs of the cluster just wrote them).
-template <bool CG, int HW = H>
+// LS=false: a Categorical head, whose flat vector ends at the head bias (no logstd to load).
+template <bool CG, int HW = H, bool LS = true>
 __device__ inline void halfnet_load(const HalfNet &n, const float *__restrict__ g, const NetLayout &L, int half) {
     constexpr int LD = RowTile<HW>::LD, LOG2 = RowTile<HW>::LOG2;
     const int tid = threadIdx.x, nt = blockDim.x;
@@ -78,7 +79,7 @@ __device__ inline void halfnet_load(const HalfNet &n, const float *__restrict__ 
     for (int i = tid; i < n.KH * HW; i += nt) n.Wh[(i >> LOG2) * LD + (i & (HW - 1))] = ldp<CG>(head + i);
     const float *bh = head + n.KH * HW;
     for (int i = tid; i < n.KH; i += nt) n.bh[i] = ldp<CG>(bh + i);
-    if (half == 0)
+    if (LS && half == 0)
         for (int i = tid; i < L.A; i += nt) n.ls[i] = ldp<CG>(bh + n.KH + i);
 }
 

@@ -27,10 +27,12 @@ def _f32c(t, name):
 
 
 def policy_forward(params, obs, dims: NetDims, eps=None, action=None, mode=ACT_SAMPLE, rows_a=None,
-                   out=None):
+                   out=None, entropy=None):
     """K1. params [P,n_par]; obs [P,rows_v,O]; eps [P or 1,rows_a,A] (SAMPLE);
-    action [P,rows_a,A] given for EVALUATE. Returns (value [P,rows_v,M], action, logp [P,rows_a])."""
-    _f32c(params, "params"); _f32c(obs, "obs"); _f32c(eps, "eps")
+    action [P,rows_a,A] given for EVALUATE. Returns (value [P,rows_v,M], action, logp [P,rows_a]).
+    Categorical head (dims.categorical, A = n): eps holds Exponential(1) draws, actions are [P,rows_a,1] category indices
+    as float32, and `entropy` (float32 [P,rows_a], optional) receives each row's entropy."""
+    _f32c(params, "params"); _f32c(obs, "obs"); _f32c(eps, "eps"); _f32c(entropy, "entropy")
     P, rows_v, O = obs.shape
     assert O == dims.obs and params.shape == (P, dims.n_par)
     if rows_a is None:
@@ -40,34 +42,37 @@ def policy_forward(params, obs, dims: NetDims, eps=None, action=None, mode=ACT_S
         value, act_out, logp = out
     else:
         value = torch.empty(P, rows_v, dims.obj, device=dev, dtype=torch.float32)
-        act_out = torch.empty(P, rows_a, dims.act, device=dev, dtype=torch.float32) if mode != ACT_EVALUATE else None
+        act_out = torch.empty(P, rows_a, dims.act_cols, device=dev, dtype=torch.float32) if mode != ACT_EVALUATE else None
         logp = torch.empty(P, rows_a, device=dev, dtype=torch.float32)
     if mode == ACT_EVALUATE:
         act_out = _f32c(action, "action")
-        assert act_out.shape == (P, rows_a, dims.act)
+        assert act_out.shape == (P, rows_a, dims.act_cols)
+    if entropy is not None:
+        assert entropy.shape == (P, rows_a)
     eps_shared = 0
     if mode == ACT_SAMPLE and rows_a > 0:
         assert eps is not None and eps.shape[1:] == (rows_a, dims.act) and eps.shape[0] in (1, P)
         eps_shared = int(eps.shape[0] == 1 and P > 1)
-    check(lib().pgm_policy_forward_h_f32(ptr(params), ptr(obs), ptr(eps), eps_shared, ptr(act_out), ptr(value),
-                                         ptr(logp), mode, P, rows_v, rows_a, dims.obs, dims.act, dims.obj, dims.hidden,
-                                         _stream()))
+    check(lib().pgm_policy_forward_x_f32(ptr(params), ptr(obs), ptr(eps), eps_shared, ptr(act_out), ptr(value),
+                                         ptr(logp), ptr(entropy), mode, P, rows_v, rows_a, dims.obs, dims.act, dims.obj,
+                                         dims.hidden, dims.dist, _stream()))
     return value, act_out, logp
 
 
 def policy_step(params, ctl, obs_stage, eps, obs_buf, value_buf, action_buf, logp_buf, act_out, N, dims: NetDims):
     """K1 per-step mode (pgm_policy_step_f32): value / action / log-prob of every task's N current observations written
-    into time slot ctl[0] of the rollout buffers; ctl = int32 [2] on the device {t, sample flag}."""
+    into time slot ctl[0] of the rollout buffers; ctl = int32 [2] on the device {t, sample flag}. eps [P or 1,N,A] (A = n
+    Exponential(1) draws for a Categorical head, whose action_buf / act_out have one column)."""
     P = params.shape[0]
     assert ctl.is_cuda and ctl.dtype == torch.int32 and ctl.numel() >= 2
     for n, t in (("params", params), ("obs_stage", obs_stage), ("eps", eps), ("obs_buf", obs_buf), ("value_buf", value_buf),
                  ("action_buf", action_buf), ("logp_buf", logp_buf), ("act_out", act_out)):
         _f32c(t, n)
     assert eps.shape[-2:] == (N, dims.act) and eps.shape[0] in (1, P)
-    check(lib().pgm_policy_step_h_f32(ptr(params), ptr(ctl), ptr(obs_stage), ptr(eps), int(eps.shape[0] == 1 and P > 1),
+    check(lib().pgm_policy_step_x_f32(ptr(params), ptr(ctl), ptr(obs_stage), ptr(eps), int(eps.shape[0] == 1 and P > 1),
                                       ptr(obs_buf), obs_buf.stride(0), ptr(value_buf), value_buf.stride(0),
                                       ptr(action_buf), action_buf.stride(0), ptr(logp_buf), logp_buf.stride(0), ptr(act_out),
-                                      P, N, dims.obs, dims.act, dims.obj, dims.hidden, _stream()))
+                                      P, N, dims.obs, dims.act, dims.obj, dims.hidden, dims.dist, _stream()))
 
 
 def gae_adv(rewards, value, masks, bad_masks, gamma, lam, weights=None, obj_var=None, out=None):
@@ -113,7 +118,7 @@ def returns_adv(rewards, value, masks, bad_masks, gamma, lam, use_gae=True, use_
 
 
 def ppo_workspace(P, S, dims: NetDims, device, cluster=0):
-    n = lib().pgm_ppo_workspace_bytes_h(P, S, dims.obs, dims.act, dims.obj, cluster, dims.hidden)
+    n = lib().pgm_ppo_workspace_bytes_x(P, S, dims.obs, dims.act, dims.obj, cluster, dims.hidden, dims.dist)
     return torch.empty(n + 256, dtype=torch.uint8, device=device)
 
 
@@ -127,10 +132,12 @@ def ppo_update(params, adam_m, adam_v, adam_step, lr, obs, action, logp_old, val
                clipped_value_loss=True):
     """K3. In place on params/adam_m/adam_v [P,n_par] and adam_step [P] int32.
     obs [P,>=S,O] / value_old [P,>=S,M] may carry the extra T+1 slot (only the first S rows are read);
-    action [P,S,A]; logp_old, adv [P,S]; returns [P,S,M]; perm int32 [P or 1,E,S]; lr float64 [P].
+    action [P,S,A] ([P,S,1] category indices as float32 for a Categorical head); logp_old, adv [P,S]; returns [P,S,M];
+    perm int32 [P or 1,E,S]; lr float64 [P].
     clipped_value_loss=False: value loss 0.5 * mean((V - R)^2) (PPO(use_clipped_value_loss=False), ppo.py:86-94).
     Returns losses [P,3] = (value_loss, action_loss, entropy) averaged over the E*B updates."""
     P, S, A = action.shape
+    assert A == dims.act_cols
     for n, t in (("params", params), ("adam_m", adam_m), ("adam_v", adam_v), ("obs", obs), ("action", action),
                  ("logp_old", logp_old), ("value_old", value_old), ("returns", returns), ("adv", adv)):
         _f32c(t, n)
@@ -145,12 +152,12 @@ def ppo_update(params, adam_m, adam_v, adam_step, lr, obs, action, logp_old, val
     if losses is None:
         losses = torch.empty(P, 3, device=params.device, dtype=torch.float32)
     E = perm.shape[1]
-    check(lib().pgm_ppo_update_h_f32(
+    check(lib().pgm_ppo_update_x_f32(
         ptr(params), ptr(adam_m), ptr(adam_v), ptr(adam_step), ptr(lr), ptr(obs), obs.stride(0), ptr(action),
         ptr(logp_old), ptr(value_old), value_old.stride(0), ptr(returns), ptr(adv), ptr(perm),
         int(perm.shape[0] == 1 and P > 1), E, num_mini_batch, C.byref(hyper), ptr(losses), wp, wn,
         cluster if clipped_value_loss else cluster | PPO_VALUE_UNCLIPPED, P, S, dims.obs, dims.act, dims.obj, dims.hidden,
-        _stream()))
+        dims.dist, _stream()))
     return losses
 
 
@@ -159,16 +166,17 @@ def ppo_grad(params, obs, action, logp_old, value_old, returns, adv, idx, dims: 
     """Verification aid: gradient [P,n_par] (before the grad-norm clip) and losses [P,3] of one minibatch `idx`
     (int32 [mb]); clipped_value_loss as in ppo_update."""
     P, S, A = action.shape
+    assert A == dims.act_cols
     hyper = hyper or PpoHyper()
     ws = ppo_workspace(P, S, dims, params.device, cluster)
     wp, wn = _aligned(ws)
     grad = torch.zeros(P, dims.n_par, device=params.device, dtype=torch.float32)
     losses = torch.empty(P, 3, device=params.device, dtype=torch.float32)
-    check(lib().pgm_ppo_grad_h_f32(ptr(params), ptr(obs), obs.stride(0), ptr(action), ptr(logp_old), ptr(value_old),
+    check(lib().pgm_ppo_grad_x_f32(ptr(params), ptr(obs), obs.stride(0), ptr(action), ptr(logp_old), ptr(value_old),
                                    value_old.stride(0), ptr(returns), ptr(adv), ptr(idx), idx.numel(),
                                    C.byref(hyper), ptr(grad), ptr(losses), wp, wn,
                                    cluster if clipped_value_loss else cluster | PPO_VALUE_UNCLIPPED, P, S, dims.obs, dims.act,
-                                   dims.obj, dims.hidden, _stream()))
+                                   dims.obj, dims.hidden, dims.dist, _stream()))
     return grad, losses
 
 

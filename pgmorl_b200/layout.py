@@ -10,6 +10,9 @@ vector converts to / from a reference ``state_dict`` by plain slicing:
     base.critic_linear.{weight[M,H],bias[M]},
     dist.fc_mean.{weight[A,H],bias[A]}, dist.logstd._bias[A,1]
 
+A Categorical head (Discrete(n) actions, distributions.py Categorical) ends in
+``dist.linear.{weight[n,H],bias[n]}`` instead: 12 tensors, no logstd.
+
 The same offsets are compiled into the CUDA side (csrc/common.cuh,
 ``struct NetLayout``, exported as ``pgm_param_offsets``); tests/test_cabi.py checks
 that both agree for every named environment shape.
@@ -18,30 +21,44 @@ from collections import OrderedDict
 from dataclasses import dataclass
 
 
+DIST_GAUSSIAN, DIST_CATEGORICAL = 0, 1   # action heads (PGM_DIST_* of include/pgmorl_b200.h)
+CATEGORICAL_MAX = 32                     # categories the kernels accept (K3's head tile)
+
+
 @dataclass(frozen=True)
 class NetDims:
     obs: int      # O
-    act: int      # A
+    act: int      # A: action dimension (Gaussian) or number of categories n (Categorical)
     obj: int      # M
     hidden: int = 64
+    dist: int = DIST_GAUSSIAN
 
     @property
     def n_par(self):
         return param_layout(self)[1]
 
+    @property
+    def categorical(self):
+        return self.dist == DIST_CATEGORICAL
+
+    @property
+    def act_cols(self):
+        """Columns of an action in the rollout buffers: A, or 1 (the category index) for a Categorical head."""
+        return 1 if self.categorical else self.act
+
 
 def param_layout(d):
     """-> (OrderedDict name -> (offset, shape), n_par)."""
     O, A, M, H = d.obs, d.act, d.obj, d.hidden
+    head = ([("dist.linear.weight", (A, H)), ("dist.linear.bias", (A,))] if d.dist == DIST_CATEGORICAL else
+            [("dist.fc_mean.weight", (A, H)), ("dist.fc_mean.bias", (A,)), ("dist.logstd._bias", (A, 1))])
     spec = [
         ("base.actor.0.weight", (H, O)), ("base.actor.0.bias", (H,)),
         ("base.actor.2.weight", (H, H)), ("base.actor.2.bias", (H,)),
         ("base.critic.0.weight", (H, O)), ("base.critic.0.bias", (H,)),
         ("base.critic.2.weight", (H, H)), ("base.critic.2.bias", (H,)),
         ("base.critic_linear.weight", (M, H)), ("base.critic_linear.bias", (M,)),
-        ("dist.fc_mean.weight", (A, H)), ("dist.fc_mean.bias", (A,)),
-        ("dist.logstd._bias", (A, 1)),
-    ]
+    ] + head
     out, off = OrderedDict(), 0
     for name, shape in spec:
         n = 1

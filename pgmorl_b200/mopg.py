@@ -55,6 +55,20 @@ def _gym_make(name):
     return _HOOKS["gym_make"](name)
 
 
+def _step_noise(N, dims):
+    """The action noise of one environment step, drawn from torch's global CPU generator as the reference's
+    dist.sample() draws it: normal_(0,1) [N,A] for a Gaussian head, exponential_(1) [N,n] for a Categorical head
+    (torch.multinomial's single-sample path), float64."""
+    eps = torch.empty(N, dims.act, dtype=torch.float64)
+    return eps.exponential_(1) if dims.categorical else eps.normal_(0, 1)
+
+
+def _env_actions(act, dims):
+    """Actions as the environments receive them: int64 category indices [.., 1] for a Categorical head (the reference's
+    VecPyTorch.step_async squeezes a LongTensor), the float32 block otherwise."""
+    return act.to(torch.int64) if dims.categorical else act
+
+
 def evaluation(args, sample):
     """Average (optionally discounted) objective vector of `eval_num` deterministic episodes (mopg.py:25-46)."""
     eval_env = _gym_make(args.env_name)
@@ -114,7 +128,7 @@ def evaluation_batch(args, samples):
                     host_obs[p, 0] = torch.Tensor(ob)
                 dev_obs.copy_(host_obs, non_blocking=True)
                 out = K.policy_forward(flat, dev_obs, dims, mode=K.ACT_DETERMINISTIC, out=out)
-                action = out[1].cpu()
+                action = _env_actions(out[1].cpu(), dims)
                 still = []
                 for p in running:
                     obs[p], _, done, info = envs[p].step(action[p])
@@ -272,13 +286,14 @@ def _population_update_raw(args, task_batch, cache, device, start_iter, final_it
             pop.obs[:, 0:N].copy_(pop.obs[:, T * N:])                                               # after_update (storage.py:71-75)
         for step in range(T + 1):
             # slot `step`: normalise the simulators' answer to the previous actions (none at step 0), then act on it
-            eps_t = torch.empty(N, dims.act, dtype=torch.float64).normal_(0, 1) if step < T else None
+            eps_t = _step_noise(N, dims) if step < T else None
             act_host = pipe.step(step, eps_t, sample=step < T, normalise=step > 0)
             if step == T:
                 break
             t0 = time.perf_counter()
+            act_env = _env_actions(act_host, dims)
             for p, envs in enumerate(envs_all):
-                ob, rew, done, infos = envs.step(act_host[p])
+                ob, rew, done, infos = envs.step(act_env[p])
                 raw_obs[p] = ob
                 raw_rew[p] = np.asarray(rew, dtype=np.float64).reshape(N)
                 done_h[p] = done
@@ -352,11 +367,11 @@ def mopg_population_update(args, task_batch, device, iteration, num_updates, sta
         else:                                                             # after_update (storage.py:71-75)
             mask_h[:, 0] = mask_h[:, T]; bad_h[:, 0] = bad_h[:, T]
         for step in range(T):
-            eps_t = torch.empty(N, dims.act, dtype=torch.float64).normal_(0, 1)
-            act_host = pipe.step(step, eps_t)                             # one graph replay: H2D, K1 into slot `step`, D2H
+            act_host = pipe.step(step, _step_noise(N, dims))              # one graph replay: H2D, K1 into slot `step`, D2H
+            act_env = _env_actions(act_host, dims)
             t0 = time.perf_counter()
             for p, envs in enumerate(envs_all):
-                obs, _, done, infos = envs.step(act_host[p])
+                obs, _, done, infos = envs.step(act_env[p])
                 obs_h[p] = np.asarray(obs, dtype=np.float32)
                 for n, info in enumerate(infos):
                     rew_h[p, step, n] = info['obj']

@@ -52,7 +52,7 @@ class PopulationMOPG:
         self.eps = z(Pr, S, A)
         self.perm = z(Pr, self.E, S, dtype=torch.int32)
         self.value = z(P, (T + 1) * N, M)
-        self.action, self.logp = z(P, S, A), z(P, S)
+        self.action, self.logp = z(P, S, dims.act_cols), z(P, S)      # Categorical: one column, the category index
         self.returns, self.adv = z(P, T, N, M), z(P, T, N)
         self.losses = z(P, 3)
         self.workspace = K.ppo_workspace(P, S, dims, dv, cluster)
@@ -116,11 +116,12 @@ class PopulationMOPG:
     # ------------------------------------------------------------------ per-step mode (real environment loops)
     def act_step(self, t, obs_host, eps_t):
         """K1 in per-step mode: obs_host [P,N,O] (host) at time t, eps_t [N,A] float64 shared by all tasks.
-        Stores obs/value/action/logp of step t in the rollout buffers; returns actions [P,N,A] (device)."""
+        Stores obs/value/action/logp of step t in the rollout buffers; returns actions [P,N,A] (device; [P,N,1] category
+        indices as float32 for a Categorical head)."""
         P, N, d = self.P, self.N, self.dims
         if not hasattr(self, "_step_obs"):
             self._step_obs = torch.empty(P, N, d.obs, device=self.device)
-            self._step_out = (torch.empty(P, N, d.obj, device=self.device), torch.empty(P, N, d.act, device=self.device),
+            self._step_out = (torch.empty(P, N, d.obj, device=self.device), torch.empty(P, N, d.act_cols, device=self.device),
                               torch.empty(P, N, device=self.device))
         self._step_obs.copy_(obs_host)
         eps = eps_t.to(self.device, torch.float32)[None].contiguous()
@@ -136,7 +137,7 @@ class PopulationMOPG:
         P, N, d = self.P, self.N, self.dims
         if not hasattr(self, "_step_obs"):
             self._step_obs = torch.empty(P, N, d.obs, device=self.device)
-            self._step_out = (torch.empty(P, N, d.obj, device=self.device), torch.empty(P, N, d.act, device=self.device),
+            self._step_out = (torch.empty(P, N, d.obj, device=self.device), torch.empty(P, N, d.act_cols, device=self.device),
                               torch.empty(P, N, device=self.device))
         rows = slice(t * N, (t + 1) * N)
         self._step_obs.copy_(self.obs[:, rows])

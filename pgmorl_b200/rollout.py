@@ -40,6 +40,7 @@ class StepPipe:
         P, N, d = pop.P, pop.N, pop.dims
         O, A, M = d.obs, d.act, d.obj
         self.P, self.N, self.O, self.A, self.M = P, N, O, A, M
+        AC = d.act_cols        # noise block [1,N,A] (A = n Exponential(1) draws for a Categorical head), actions [P,N,AC]
         blocks = [("ctl", 16)]
         if vn is not None:
             blocks += [("raw_obs", 8 * P * N * O), ("raw_rew", 8 * P * N), ("raw_obj", 8 * P * N * M),
@@ -50,8 +51,8 @@ class StepPipe:
         self.layout, total = _carve(blocks)
         self.h = torch.zeros(total, dtype=torch.uint8, pin_memory=True)
         self.dv = torch.zeros(total, dtype=torch.uint8, device=pop.device)
-        self.h_act = torch.zeros(P, N, A, dtype=torch.float32, pin_memory=True)
-        self.d_act = torch.zeros(P, N, A, dtype=torch.float32, device=pop.device)
+        self.h_act = torch.zeros(P, N, AC, dtype=torch.float32, pin_memory=True)
+        self.d_act = torch.zeros(P, N, AC, dtype=torch.float32, device=pop.device)
 
         def view(buf, name, dtype, shape):
             o, n = self.layout[name]
@@ -120,7 +121,7 @@ class StepPipe:
     def step(self, t, eps_t, sample=True, normalise=False):
         """Run slot t for all tasks on whatever the staging block holds (fill `h_obs` or the raw blocks first).
         eps_t: float64 [N,A] draw of this step (None for the bootstrap). Returns the pinned action block [P,N,A]
-        (valid until the next call)."""
+        ([P,N,1] float32 category indices for a Categorical head; valid until the next call)."""
         self.np_ctl[0] = t
         self.np_ctl[1] = (1 if sample else 0) | (2 if normalise else 0)
         if eps_t is not None:

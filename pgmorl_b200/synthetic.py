@@ -18,6 +18,8 @@ def init_policy_flat(dims: NetDims, seed=None):
     False}, obj_num=M).double()`` (warm_up.py:34-40): each ``nn.Linear`` first runs its
     default init, then ``orthogonal_`` with the reference's gain
     (model.py:208-216,252-254; distributions.py:75-78). Returns float64 [n_par].
+    A Categorical head (``Policy(obs_shape, Discrete(n))``) is built after the base in the same way: ``dist.linear =
+    nn.Linear(H, n)``, orthogonal with gain 0.01, bias 0 (the Categorical module of distributions.py), and has no logstd.
     """
     if seed is not None:
         torch.manual_seed(seed)
@@ -35,9 +37,9 @@ def init_policy_flat(dims: NetDims, seed=None):
     c0 = lin(O, H, g2); c2 = lin(H, H, g2)
     lin(H, 1, g2)                      # MLPBase.critic_linear, replaced by MOMLPBase
     cl = lin(H, M, g2)
-    fm = lin(H, A, 1.0)
+    fm = lin(H, A, 0.01 if dims.categorical else 1.0)
     tensors = [a0.weight, a0.bias, a2.weight, a2.bias, c0.weight, c0.bias, c2.weight, c2.bias,
-               cl.weight, cl.bias, fm.weight, fm.bias, torch.zeros(A, 1, dtype=f64)]
+               cl.weight, cl.bias, fm.weight, fm.bias] + ([] if dims.categorical else [torch.zeros(A, 1, dtype=f64)])
     flat = torch.cat([t.detach().reshape(-1) for t in tensors])
     assert flat.numel() == param_layout(dims)[1]
     return flat
@@ -81,17 +83,23 @@ def make_trajectories(P, T, N, dims: NetDims, seed=1, p_done=0.002):
     return {"obs": obs, "rewards": rewards, "masks": masks, "bad_masks": bad_masks}
 
 
-def host_rng_streams(j, T, N, A, epochs, eps_dtype=torch.float64):
+def host_rng_streams(j, T, N, A, epochs, eps_dtype=torch.float64, categorical=False):
     """The reference's per-iteration random streams (mopg.py:96 ``torch.manual_seed(j)``):
     T draws of action noise ``[N,A]`` in rollout order (distributions.py:30-40 via
     ``dist.sample()`` == ``mean + std*normal_(0,1)``), then one ``randperm(T*N)`` per PPO
     epoch (storage.py:133-137 ``BatchSampler(SubsetRandomSampler(range(T*N)))``).
+    categorical=True (A = n categories): the noise of each step is ``exponential_(1)`` of shape ``[N,n]``, what
+    ``Categorical.sample()`` draws in torch 2.11 (``torch.multinomial(probs, 1, True)`` takes ``argmax(probs / q)``
+    with ``q = empty_like(probs).exponential_(1)`` for a single sample).
     Returns eps f64 [T,N,A], perm int64 [epochs, T*N].
     """
     torch.manual_seed(j)
     eps = torch.empty(T, N, A, dtype=eps_dtype)
     for t in range(T):
-        eps[t].normal_(0, 1)
+        if categorical:
+            eps[t].exponential_(1)
+        else:
+            eps[t].normal_(0, 1)
     perm = torch.stack([torch.randperm(T * N) for _ in range(epochs)])
     return eps, perm
 
