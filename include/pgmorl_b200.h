@@ -342,7 +342,9 @@ int pgm_ep_filter_f64(const double *objs, int n, int M, int32_t *keep_idx, int32
  *   M == 2: Population.compute_hypervolume / compute_sparsity (morl/population_2d.py:185-202):
  *           Pareto-filter, then closed forms on the front sorted by objective 0.
  *   M == 3: utils.compute_hypervolume (InnerHyperVolume, morl/hypervolume.py:41-153, round(hv,4))
- *           and utils.compute_sparsity (morl/utils.py:87-100) of the given front (all coords >= 0).
+ *           and utils.compute_sparsity (morl/utils.py:87-100) of the given front (all coords >= 0). Any size:
+ *           fronts of up to 3 936 points are scored in one CTA's shared memory (52 bytes per point), larger ones
+ *           on the global-memory path (see pgm_select_greedy_x_f64), with bit-identical results.
  *   M == 4: the same two functions (hypervolume.py:41-153 with its stored volumes / areas and area-reuse
  *           flags, utils.py:87-100); points with a negative coordinate are left out of the hypervolume as
  *           hypervolume.py:55-61 does. At most 2 202 points (the scorer's 93 bytes of shared memory per
@@ -351,6 +353,10 @@ int pgm_ep_filter_f64(const double *objs, int n, int M, int32_t *keep_idx, int32
  * workspace >= pgm_select_workspace_bytes(n, 1, M, 1). */
 int pgm_front_metrics_f64(const double *pts, int n, int M, double *out, void *workspace,
                           size_t workspace_bytes, void *stream);
+/* pgm_front_metrics_x_f64: the same with `flags` (PGM_SEL_GLOBAL forces the global-memory path at M = 3);
+ * pgm_front_metrics_f64 is its flags = 0 case. workspace >= pgm_select_workspace_bytes_x(n, 1, M, 1, flags). */
+int pgm_front_metrics_x_f64(const double *pts, int n, int M, int flags, double *out, void *workspace,
+                            size_t workspace_bytes, void *stream);
 
 /* Replaces evaluate_hv / evaluate_sparsity and the greedy loop of prediction_guided_selection
  * (morl/population_2d.py:207-224,264-302; morl/population_3d.py:206-214,294-331, update_ep
@@ -361,8 +367,12 @@ int pgm_front_metrics_f64(const double *pts, int n, int M, double *out, void *wo
  * EP_{r+1} = EP_r with the winner's prediction folded in. n_front [1] out: size of the final
  * virtual front, written to front_out [E+num_tasks, M] (both optional / may be NULL).
  * 3 objectives: every candidate of a round is scored on top of the round's shared base front (sorted lists, slice areas
- * and the head of the hypervolume sum are built once per round in the workspace); the per-candidate scratch of
- * 97 * (E + num_tasks + 1) bytes must fit 200 KB of shared memory (archive fronts up to ~2 100 points), else an error.
+ * and the head of the hypervolume sum are built once per round in the workspace). No size limit besides the workspace:
+ * while the per-candidate scratch of 97 * (E + num_tasks + 1) bytes fits 200 KB of shared memory
+ * (E + num_tasks + 1 <= 2 111) one CTA per candidate scores in shared memory; past that (or with PGM_SEL_GLOBAL) a grid
+ * of at most 296 CTAs loops over the candidates with one scratch each in the workspace, about
+ * 97 * min(C, 296) * (E + num_tasks + 1) bytes, and the base front is built by multi-CTA kernels. Both paths perform
+ * the same float64 operations in the same order: their results are bit-identical.
  * 4 objectives (update_ep utils.py:42-65, hypervolume.py:41-153, compute_sparsity utils.py:87-100): one CTA per
  * candidate replays the reference's 4-D dimension sweep, stored level-2 volumes / areas and area-reuse flags included;
  * the per-candidate scratch of 93 * (E + num_tasks + 1) bytes must fit 200 KB of shared memory
@@ -373,6 +383,16 @@ int pgm_select_greedy_f64(const double *ep, int E, const double *cand, int C, in
                           int num_tasks, int32_t *best_ids, double *hv, double *sparsity,
                           double *front_out, int32_t *n_front, void *workspace, size_t workspace_bytes,
                           void *stream);
+
+/* Selection flags of the _x entry points. PGM_SEL_GLOBAL: take the 3-objective global-memory path even where the
+ * front fits shared memory (M = 3 only; other M: error), so both paths can be compared on one input. The entry points
+ * without _x are the flags = 0 case: the path follows the front's size. */
+#define PGM_SEL_GLOBAL 0x1
+size_t pgm_select_workspace_bytes_x(int E, int C, int M, int num_tasks, int flags);
+int pgm_select_greedy_x_f64(const double *ep, int E, const double *cand, int C, int M, double alpha,
+                            int num_tasks, int flags, int32_t *best_ids, double *hv, double *sparsity,
+                            double *front_out, int32_t *n_front, void *workspace, size_t workspace_bytes,
+                            void *stream);
 
 /* ---------------------------------------------------------------------------
  * K6  running normalisation of raw simulator output, all P x N environments of the shard in one launch per

@@ -75,6 +75,9 @@ SIGNATURES = {
                                   C.POINTER(PpoHyper), _P, _P, _Z, _I, _I, _I, _I, _I, _I, _I, _I, _P]),
     "pgm_ppo_grad_x_f32": (_I, [_P, _P, _Z, _P, _P, _P, _Z, _P, _P, _P, _I, C.POINTER(PpoHyper), _P, _P, _P,
                                 _Z, _I, _I, _I, _I, _I, _I, _I, _I, _P]),
+    "pgm_front_metrics_x_f64": (_I, [_P, _I, _I, _I, _P, _P, _Z, _P]),
+    "pgm_select_workspace_bytes_x": (_Z, [_I, _I, _I, _I, _I]),
+    "pgm_select_greedy_x_f64": (_I, [_P, _I, _P, _I, _I, C.c_double, _I, _I, _P, _P, _P, _P, _P, _P, _Z, _P]),
 }
 
 

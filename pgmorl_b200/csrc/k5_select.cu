@@ -413,11 +413,13 @@ __global__ void __launch_bounds__(1024) k5_base3d_kernel(SelState st, int buf, i
 //    order, so their areas and the head of the hypervolume chain are the base's; only the slices from n_same on are walked;
 //  * warps 0-7 walk slices while warp 8 forms the sparsity terms and runs that serial sum.
 // Points are named by id: position in the base front, or n0 for p.
+// The body scores candidate c with its arrays carved from `smraw` (score3d_inc_smem(nmax) bytes): shared memory in
+// k5_score3d_inc_kernel, a per-CTA slice of global memory in k5g_score3d_inc_kernel.
 constexpr int S3_WORKERS = 256, S3_THREADS = 288;
-__global__ void __launch_bounds__(S3_THREADS) k5_score3d_inc_kernel(SelState st, int buf, const double *__restrict__ cand, int C,
-                                                                    double *__restrict__ hv, double *__restrict__ sp, int nmax) {
-    extern __shared__ __align__(16) unsigned char smraw[];
-    const int c = blockIdx.x, tid = threadIdx.x, nt = blockDim.x, lane = tid & 31, warp = tid >> 5;
+__device__ __forceinline__ void score3d_inc_body(const SelState &st, int buf, const double *__restrict__ cand, int c,
+                                                 double *__restrict__ hv, double *__restrict__ sp, int nmax,
+                                                 unsigned char *smraw) {
+    const int tid = threadIdx.x, nt = blockDim.x, lane = tid & 31, warp = tid >> 5;
     if (*st.done || !st.mask[c]) {
         if (tid == 0) { hv[c] = 0.0; sp[c] = 0.0; }
         return;
@@ -539,6 +541,12 @@ __global__ void __launch_bounds__(S3_THREADS) k5_score3d_inc_kernel(SelState st,
         v = dsub(v, dmul(area[n - 1], cz[zl[n - 1]]));
         hv[c] = round4(v);
     }
+}
+
+__global__ void __launch_bounds__(S3_THREADS) k5_score3d_inc_kernel(SelState st, int buf, const double *__restrict__ cand, int C,
+                                                                    double *__restrict__ hv, double *__restrict__ sp, int nmax) {
+    extern __shared__ __align__(16) unsigned char smraw[];
+    score3d_inc_body(st, buf, cand, blockIdx.x, hv, sp, nmax, smraw);
 }
 
 // update_ep (utils.py:42-65) by all threads of one CTA: same result as update_front_3d. flags: [n] ints of shared memory.
@@ -856,11 +864,12 @@ __global__ void __launch_bounds__(256) k5_score4d_kernel(SelState st, int buf, c
 // ---- arg-max + virtual EP update: single CTA ---------------------------------------------------------
 // 3 objectives: dynamic shared memory of base3d_smem(nmax) bytes (first used as nmax ints by the front update); the new
 // front's base data for the next round's scorer is built here. 4 objectives: nmax ints for the front update.
-template <int M>
-__global__ void __launch_bounds__(1024) k5_pick_kernel(SelState st, int buf, const double *__restrict__ cand, int C,
-                                                       const double *__restrict__ hv, const double *__restrict__ sp,
-                                                       double alpha, int32_t *__restrict__ best_out, int nmax) {
-    extern __shared__ __align__(16) unsigned char pick_smem[];
+// GLOBAL (3 objectives only, k5g_pick3d_kernel): the front update's flags are pick_smem in global memory, and the base
+// data is left to the k5g_base3d_* kernels.
+template <int M, bool GLOBAL>
+__device__ __forceinline__ void pick_body(const SelState &st, int buf, const double *__restrict__ cand, int C,
+                                          const double *__restrict__ hv, const double *__restrict__ sp, double alpha,
+                                          int32_t *__restrict__ best_out, int nmax, unsigned char *pick_smem) {
     __shared__ double sv[32];
     __shared__ int si[32];
     __shared__ int wtot[32];
@@ -901,7 +910,7 @@ __global__ void __launch_bounds__(1024) k5_pick_kernel(SelState st, int buf, con
         if (M == 3 && s_bi >= 0) {
             update_front_3d_block(st.front[buf], st.count[buf], cand + 3 * s_bi, st.front[buf ^ 1], &st.count[buf ^ 1],
                                   reinterpret_cast<int *>(pick_smem), wtot);
-            base3d_build(st.front[buf ^ 1], st.count[buf ^ 1], nmax, st.b3, pick_smem);
+            if (!GLOBAL) base3d_build(st.front[buf ^ 1], st.count[buf ^ 1], nmax, st.b3, pick_smem);
         }
         if (M == 4 && s_bi >= 0)
             update_front_4d_block(st.front[buf], st.count[buf], cand + 4 * s_bi, st.front[buf ^ 1], &st.count[buf ^ 1],
@@ -911,6 +920,129 @@ __global__ void __launch_bounds__(1024) k5_pick_kernel(SelState st, int buf, con
         const int n = st.count[buf];
         for (int i = tid; i < n * M; i += blockDim.x) st.front[buf ^ 1][i] = st.front[buf][i];
         if (tid == 0) st.count[buf ^ 1] = n;
+    }
+}
+
+template <int M>
+__global__ void __launch_bounds__(1024) k5_pick_kernel(SelState st, int buf, const double *__restrict__ cand, int C,
+                                                       const double *__restrict__ hv, const double *__restrict__ sp,
+                                                       double alpha, int32_t *__restrict__ best_out, int nmax) {
+    extern __shared__ __align__(16) unsigned char pick_smem[];
+    pick_body<M, false>(st, buf, cand, C, hv, sp, alpha, best_out, nmax, pick_smem);
+}
+
+// ---- 3 objectives on fronts past the shared-memory layouts: global-memory scratch ------------------------------------
+// The same float64 operations in the same order as k5_base3d_kernel / k5_score3d_inc_kernel / k5_pick_kernel<3> /
+// k5_score3d_kernel, so every result is bit-identical to theirs wherever both run; the per-point arrays live in the
+// workspace instead of shared memory, so a front has no size limit besides the workspace.
+struct Glob3d {
+    double *hx, *hy;            // [nmax] x, y of the base front's points in y-list order
+    int *hz;                    // [nmax] their z ranks
+    int *flags;                 // [nmax] scratch of the front update
+    unsigned char *scratch;     // [S3G_CTAS][stride] one score3d_inc_smem(nmax) layout per CTA of the scorer
+    size_t stride;
+};
+// CTAs of the global scorer, each looping over candidates with one scratch: the workspace does not grow with C.
+// 296 = two per SM of a B200.
+constexpr int S3G_CTAS = 296;
+
+// The base data of base3d_build, in three launches over the whole grid. Ranks: one thread per point, the front streamed
+// through shared-memory tiles, the comparisons of base3d_build (integers, so any schedule gives the same lists).
+__global__ void __launch_bounds__(256) k5g_base3d_rank_kernel(SelState st, int buf, Glob3d g) {
+    __shared__ double tx[256], ty[256], tz[256];
+    const Base3d b = st.b3;
+    const double *f = st.front[buf];
+    const int n0 = st.count[buf], i = blockIdx.x * blockDim.x + threadIdx.x;
+    const bool valid = i < n0;
+    double xi = 0.0, yi = 0.0, zi = 0.0;
+    if (valid) {
+        xi = -f[3 * i]; yi = -f[3 * i + 1]; zi = -f[3 * i + 2];
+        b.nx[i] = xi; b.ny[i] = yi; b.nz[i] = zi;
+    }
+    if (i == 0) b.vpre[0] = 0.0;
+    int rx = 0, ry = 0, rz = 0;
+    for (int j0 = 0; j0 < n0; j0 += 256) {
+        const int nj = min(256, n0 - j0);
+        __syncthreads();
+        for (int t = threadIdx.x; t < nj; t += blockDim.x) {
+            tx[t] = -f[3 * (j0 + t)]; ty[t] = -f[3 * (j0 + t) + 1]; tz[t] = -f[3 * (j0 + t) + 2];
+        }
+        __syncthreads();
+        if (valid)
+#pragma unroll 4
+            for (int t = 0; t < nj; ++t) {
+                const int j = j0 + t;
+                const double xj = tx[t], yj = ty[t], zj = tz[t];
+                const bool xlt = xj < xi || (xj == xi && j < i);
+                const bool ylt = yj < yi || (yj == yi && xlt);
+                const bool zlt = zj < zi || (zj == zi && ylt);
+                rx += xlt; ry += ylt; rz += zlt;
+            }
+    }
+    if (valid) {
+        b.xl[rx] = i; b.yl[ry] = i; b.zl[rz] = i; b.zr[i] = rz;
+        g.hx[ry] = xi; g.hy[ry] = yi; g.hz[ry] = rz;
+    }
+}
+
+// slice areas: one thread per slice
+__global__ void __launch_bounds__(256) k5g_base3d_area_kernel(SelState st, int buf, Glob3d g) {
+    const int n0 = st.count[buf], k = blockIdx.x * blockDim.x + threadIdx.x;
+    if (k < n0) st.b3.area[k] = slice_area(g.hx, g.hy, g.hz, n0, k);
+}
+
+// the hypervolume chain: terms in parallel, the running sum on thread 0 (one CTA)
+__global__ void __launch_bounds__(1024) k5g_base3d_chain_kernel(SelState st, int buf) {
+    const Base3d b = st.b3;
+    const int n0 = st.count[buf], tid = threadIdx.x;
+    for (int k = 1 + tid; k < n0; k += blockDim.x) b.vpre[k] = dmul(b.area[k - 1], dsub(b.nz[b.zl[k]], b.nz[b.zl[k - 1]]));
+    __syncthreads();
+    if (tid == 0) {
+        double v = 0.0;
+#pragma unroll 8
+        for (int k = 1; k < n0; ++k) { v = dadd(v, b.vpre[k]); b.vpre[k] = v; }
+    }
+}
+
+// The incremental scorer on per-CTA global scratch: a grid of resident CTAs loops over the candidates.
+__global__ void __launch_bounds__(S3_THREADS) k5g_score3d_inc_kernel(SelState st, int buf, const double *__restrict__ cand, int C,
+                                                                     double *__restrict__ hv, double *__restrict__ sp, int nmax,
+                                                                     Glob3d g) {
+    unsigned char *scratch = g.scratch + (size_t)blockIdx.x * g.stride;
+    for (int c = blockIdx.x; c < C; c += gridDim.x) {
+        score3d_inc_body(st, buf, cand, c, hv, sp, nmax, scratch);
+        __syncthreads();                                   // the next candidate reuses the scratch and the shared words
+    }
+}
+
+__global__ void __launch_bounds__(1024) k5g_pick3d_kernel(SelState st, int buf, const double *__restrict__ cand, int C,
+                                                          const double *__restrict__ hv, const double *__restrict__ sp,
+                                                          double alpha, int32_t *__restrict__ best_out, Glob3d g) {
+    pick_body<3, true>(st, buf, cand, C, hv, sp, alpha, best_out, 0, reinterpret_cast<unsigned char *>(g.flags));
+}
+
+// Metrics of front[0] from its base data (pgm_front_metrics_f64): k5_score3d_kernel's hypervolume and sparsity, whose
+// sums are the base chain and the base lists read backwards. front[0] holds n >= 1 points.
+__global__ void k5g_metrics3d_kernel(SelState st, double *__restrict__ out) {
+    const Base3d b = st.b3;
+    const int n = st.count[0];
+    if (threadIdx.x == 0) {
+        const double v = dsub(b.vpre[n - 1], dmul(b.area[n - 1], b.nz[b.zl[n - 1]]));
+        out[0] = round4(v);
+    } else if (threadIdx.x == 32) {
+        double s = 0.0;
+        if (n >= 2) {
+            for (int d = 0; d < 3; ++d) {
+                const int *lst = d == 0 ? b.xl : (d == 1 ? b.yl : b.zl);
+                const double *v = d == 0 ? b.nx : (d == 1 ? b.ny : b.nz);
+                for (int i = 1; i < n; ++i) {
+                    const double gap = dsub(-v[lst[n - 1 - i]], -v[lst[n - i]]);
+                    s = dadd(s, dmul(gap, gap));
+                }
+            }
+            s = s / (double)(n - 1);
+        }
+        out[1] = s;
     }
 }
 
@@ -947,7 +1079,14 @@ __global__ void k5_metrics2d_kernel(const double *__restrict__ pts, const int32_
     out[1] = n < 2 ? 0.0 : sp / (double)(n - 1);
 }
 
-static size_t sel_carve(SelState &st, char *ws, int E, int C, int M, int num_tasks) {
+static size_t score3d_smem(int nmax) { return (size_t)nmax * (4 * sizeof(double) + 5 * sizeof(int)); }
+static size_t score3d_inc_smem(int nmax) { return (size_t)nmax * (9 * sizeof(double) + 6 * sizeof(int) + 1) + 16; }
+// Largest shared-memory layout of the 3-D kernels: fronts up to 2 111 points for the incremental scorer
+// (archive + num_tasks + 1) and 3 936 for the one-front scorer.
+constexpr size_t SCORE3D_SMEM_MAX = 200 * 1024;
+
+// global3: carve the global-memory 3-D path's arrays (Glob3d) as well, for up to C candidates.
+static size_t sel_carve(SelState &st, Glob3d &g, char *ws, int E, int C, int M, int num_tasks, bool global3) {
     size_t off = 0;
     auto seg = [&](size_t bytes) { size_t o = off; off += (bytes + 255) / 256 * 256; return o; };
     const size_t fb = (size_t)(E + num_tasks + 1) * M * sizeof(double);
@@ -965,12 +1104,34 @@ static size_t sel_carve(SelState &st, char *ws, int E, int C, int M, int num_tas
             st.b3.nx = d; st.b3.ny = d + nmax; st.b3.nz = d + 2 * nmax; st.b3.area = d + 3 * nmax; st.b3.vpre = d + 4 * nmax;
             st.b3.xl = i; st.b3.yl = i + nmax; st.b3.zl = i + 2 * nmax; st.b3.zr = i + 3 * nmax;
         }
+        if (global3) {
+            const size_t stride = (score3d_inc_smem((int)nmax) + 255) / 256 * 256;
+            const int ctas = C < 1 ? 1 : (C < S3G_CTAS ? C : S3G_CTAS);
+            const size_t ohx = seg(nmax * sizeof(double)), ohy = seg(nmax * sizeof(double)), ohz = seg(nmax * sizeof(int)),
+                         ofl = seg(nmax * sizeof(int)), osc = seg(ctas * stride);
+            if (ws) {
+                g.hx = (double *)(ws + ohx); g.hy = (double *)(ws + ohy); g.hz = (int *)(ws + ohz); g.flags = (int *)(ws + ofl);
+                g.scratch = (unsigned char *)(ws + osc); g.stride = stride;
+            }
+        }
     }
     return off;
 }
 
-static size_t score3d_smem(int nmax) { return (size_t)nmax * (4 * sizeof(double) + 5 * sizeof(int)); }
-static size_t score3d_inc_smem(int nmax) { return (size_t)nmax * (9 * sizeof(double) + 6 * sizeof(int) + 1) + 16; }
+// Which 3-D path pgm_select_greedy_x_f64 takes (the workspace query sizes for it; pgm_front_metrics_x_f64's own choice,
+// at 3 936 points, is never global where this one is not).
+static bool select_global3(int M, int nmax, int flags) {
+    return M == 3 && ((flags & PGM_SEL_GLOBAL) || score3d_inc_smem(nmax) > SCORE3D_SMEM_MAX);
+}
+
+// base data of front[buf] for the global path
+static void base3d_global(const SelState &st, int buf, const Glob3d &g, int nmax, cudaStream_t s) {
+    const int blocks = (nmax + 255) / 256;
+    k5g_base3d_rank_kernel<<<blocks, 256, 0, s>>>(st, buf, g);
+    k5g_base3d_area_kernel<<<blocks, 256, 0, s>>>(st, buf, g);
+    k5g_base3d_chain_kernel<<<1, 1024, 0, s>>>(st, buf);
+}
+
 static size_t score4d_smem(int nmax) { return (size_t)nmax * (8 * sizeof(double) + 7 * sizeof(int) + 1); }
 // Largest front (points of L = update_ep(front, p)) the 4-D scorer's shared-memory layout holds: 2 202 points.
 constexpr size_t SCORE4D_SMEM_MAX = 200 * 1024;
@@ -997,27 +1158,37 @@ extern "C" int pgm_ep_filter_f64(const double *objs, int n, int M, int32_t *keep
     return PGM_OK;
 }
 
-extern "C" size_t pgm_select_workspace_bytes(int E, int C, int M, int num_tasks) {
+extern "C" size_t pgm_select_workspace_bytes_x(int E, int C, int M, int num_tasks, int flags) {
     SelState st;
+    Glob3d g;
     // + room for the ep_filter scratch used by pgm_front_metrics_f64 (2 * n int32 + count)
-    return sel_carve(st, nullptr, E, C, M, num_tasks) + ((size_t)(2 * E + 2) * sizeof(int32_t) + 255) / 256 * 256;
+    return sel_carve(st, g, nullptr, E, C, M, num_tasks, select_global3(M, E + num_tasks + 1, flags)) +
+           ((size_t)(2 * E + 2) * sizeof(int32_t) + 255) / 256 * 256;
 }
 
-extern "C" int pgm_select_greedy_f64(const double *ep, int E, const double *cand, int C, int M, double alpha,
-                                     int num_tasks, int32_t *best_ids, double *hv, double *sparsity, double *front_out,
-                                     int32_t *n_front, void *workspace, size_t workspace_bytes, void *stream) {
+extern "C" size_t pgm_select_workspace_bytes(int E, int C, int M, int num_tasks) {
+    return pgm_select_workspace_bytes_x(E, C, M, num_tasks, 0);
+}
+
+extern "C" int pgm_select_greedy_x_f64(const double *ep, int E, const double *cand, int C, int M, double alpha,
+                                       int num_tasks, int flags, int32_t *best_ids, double *hv, double *sparsity,
+                                       double *front_out, int32_t *n_front, void *workspace, size_t workspace_bytes,
+                                       void *stream) {
     PGM_REQUIRE((ep || E == 0) && (cand || C == 0) && best_ids && hv && sparsity && workspace, "pgm_select_greedy_f64: null pointer");
     PGM_REQUIRE(M >= 2 && M <= 4, "pgm_select_greedy_f64: exact hypervolume is implemented for 2 to 4 objectives (got %d)", M);
     PGM_REQUIRE(E >= 0 && C >= 0 && num_tasks >= 1, "pgm_select_greedy_f64: bad sizes E=%d C=%d num_tasks=%d", E, C, num_tasks);
+    PGM_REQUIRE((flags & ~PGM_SEL_GLOBAL) == 0, "pgm_select_greedy_f64: unknown flags 0x%x", flags);
+    PGM_REQUIRE(!(flags & PGM_SEL_GLOBAL) || M == 3, "pgm_select_greedy_f64: PGM_SEL_GLOBAL is a 3-objective path (got M=%d)", M);
     PGM_REQUIRE(((uintptr_t)workspace & 255) == 0, "pgm_select_greedy_f64: workspace must be 256-byte aligned");
+    const int nmax = E + num_tasks + 1;
+    const bool global3 = select_global3(M, nmax, flags);
     SelState st;
-    const size_t need = sel_carve(st, (char *)workspace, E, C, M, num_tasks);
+    Glob3d g;
+    const size_t need = sel_carve(st, g, (char *)workspace, E, C, M, num_tasks, global3);
     if (need > workspace_bytes) { set_error("pgm_select_greedy_f64: workspace too small: need %zu, got %zu", need, workspace_bytes); return PGM_ERR_WORKSPACE; }
     cudaStream_t s = (cudaStream_t)stream;
-    const int nmax = E + num_tasks + 1;
     const size_t smem3 = score3d_inc_smem(nmax), smemb = base3d_smem(nmax);
-    if (M == 3) {
-        PGM_REQUIRE(smem3 <= 200 * 1024, "pgm_select_greedy_f64: front of %d points exceeds the 3-D scorer's shared memory", nmax);
+    if (M == 3 && !global3) {
         PGM_CUDA(cudaFuncSetAttribute(k5_score3d_inc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem3));
         PGM_CUDA(cudaFuncSetAttribute(k5_base3d_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smemb));
         PGM_CUDA(cudaFuncSetAttribute(k5_pick_kernel<3>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smemb));
@@ -1031,11 +1202,20 @@ extern "C" int pgm_select_greedy_f64(const double *ep, int E, const double *cand
     {
         const int nthr = (E * M > C ? E * M : C) + 1;
         k5_init_kernel<<<(nthr + 255) / 256, 256, 0, s>>>(st, ep, E, M, C);
-        if (M == 3 && C > 0) k5_base3d_kernel<<<1, 1024, smemb, s>>>(st, 0, nmax);
+        if (M == 3 && C > 0) {
+            if (global3) base3d_global(st, 0, g, nmax, s);
+            else k5_base3d_kernel<<<1, 1024, smemb, s>>>(st, 0, nmax);
+        }
     }
     for (int r = 0; r < num_tasks; ++r) {
         const int buf = r & 1;
         double *hv_r = hv + (size_t)r * C, *sp_r = sparsity + (size_t)r * C;
+        if (global3) {
+            if (C > 0) k5g_score3d_inc_kernel<<<C < S3G_CTAS ? C : S3G_CTAS, S3_THREADS, 0, s>>>(st, buf, cand, C, hv_r, sp_r, nmax, g);
+            k5g_pick3d_kernel<<<1, 1024, 0, s>>>(st, buf, cand, C, hv_r, sp_r, alpha, best_ids + r, g);
+            if (C > 0 && r + 1 < num_tasks) base3d_global(st, buf ^ 1, g, nmax, s);
+            continue;
+        }
         if (C > 0) {
             if (M == 2) k5_score2d_kernel<<<(C + 127) / 128, 128, 0, s>>>(st, buf, cand, C, hv_r, sp_r);
             else if (M == 3) k5_score3d_inc_kernel<<<C, S3_THREADS, smem3, s>>>(st, buf, cand, C, hv_r, sp_r, nmax);
@@ -1050,14 +1230,27 @@ extern "C" int pgm_select_greedy_f64(const double *ep, int E, const double *cand
     return PGM_OK;
 }
 
-extern "C" int pgm_front_metrics_f64(const double *pts, int n, int M, double *out, void *workspace,
-                                     size_t workspace_bytes, void *stream) {
+extern "C" int pgm_select_greedy_f64(const double *ep, int E, const double *cand, int C, int M, double alpha,
+                                     int num_tasks, int32_t *best_ids, double *hv, double *sparsity, double *front_out,
+                                     int32_t *n_front, void *workspace, size_t workspace_bytes, void *stream) {
+    return pgm_select_greedy_x_f64(ep, E, cand, C, M, alpha, num_tasks, 0, best_ids, hv, sparsity, front_out, n_front,
+                                   workspace, workspace_bytes, stream);
+}
+
+extern "C" int pgm_front_metrics_x_f64(const double *pts, int n, int M, int flags, double *out, void *workspace,
+                                       size_t workspace_bytes, void *stream) {
     PGM_REQUIRE(out && workspace && (pts || n == 0), "pgm_front_metrics_f64: null pointer");
     PGM_REQUIRE(M >= 2 && M <= 4, "pgm_front_metrics_f64: implemented for 2 to 4 objectives (got %d)", M);
+    PGM_REQUIRE(n >= 0, "pgm_front_metrics_f64: bad size n=%d", n);
+    PGM_REQUIRE((flags & ~PGM_SEL_GLOBAL) == 0, "pgm_front_metrics_f64: unknown flags 0x%x", flags);
+    PGM_REQUIRE(!(flags & PGM_SEL_GLOBAL) || M == 3, "pgm_front_metrics_f64: PGM_SEL_GLOBAL is a 3-objective path (got M=%d)", M);
     PGM_REQUIRE(((uintptr_t)workspace & 255) == 0, "pgm_front_metrics_f64: workspace must be 256-byte aligned");
     cudaStream_t s = (cudaStream_t)stream;
+    const int nmax3 = n + 2;
+    const bool global3 = M == 3 && ((flags & PGM_SEL_GLOBAL) || score3d_smem(nmax3) > SCORE3D_SMEM_MAX);
     SelState st;
-    const size_t base = sel_carve(st, (char *)workspace, n, 1, M, 1);
+    Glob3d g;
+    const size_t base = sel_carve(st, g, (char *)workspace, n, 1, M, 1, global3);
     const size_t need = base + ((size_t)(2 * n + 2) * sizeof(int32_t) + 255) / 256 * 256;
     if (need > workspace_bytes) { set_error("pgm_front_metrics_f64: workspace too small: need %zu, got %zu", need, workspace_bytes); return PGM_ERR_WORKSPACE; }
     if (n == 0) { PGM_CUDA(cudaMemsetAsync(out, 0, 2 * sizeof(double), s)); return PGM_OK; }
@@ -1076,14 +1269,21 @@ extern "C" int pgm_front_metrics_f64(const double *pts, int n, int M, double *ou
         PGM_CUDA(cudaFuncSetAttribute(k5_score4d_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem4));
         k5_init_kernel<<<(n * M + 256) / 256, 256, 0, s>>>(st, pts, n, M, 0);
         k5_score4d_kernel<<<1, 256, smem4, s>>>(st, 0, nullptr, 1, out, out + 1, n, 0);
+    } else if (global3) {
+        k5_init_kernel<<<(n * M + 256) / 256, 256, 0, s>>>(st, pts, n, M, 0);
+        base3d_global(st, 0, g, nmax3, s);
+        k5g_metrics3d_kernel<<<1, 64, 0, s>>>(st, out);
     } else {
-        const int nmax = n + 2;
-        const size_t smem3 = score3d_smem(nmax);
-        PGM_REQUIRE(smem3 <= 200 * 1024, "pgm_front_metrics_f64: %d points exceed the 3-D scorer's shared memory", n);
+        const size_t smem3 = score3d_smem(nmax3);
         PGM_CUDA(cudaFuncSetAttribute(k5_score3d_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem3));
         k5_init_kernel<<<(n * M + 256) / 256, 256, 0, s>>>(st, pts, n, M, 0);
-        k5_score3d_kernel<<<1, 256, smem3, s>>>(st, 0, nullptr, 1, out, out + 1, nmax, 0);
+        k5_score3d_kernel<<<1, 256, smem3, s>>>(st, 0, nullptr, 1, out, out + 1, nmax3, 0);
     }
     PGM_CUDA(cudaGetLastError());
     return PGM_OK;
+}
+
+extern "C" int pgm_front_metrics_f64(const double *pts, int n, int M, double *out, void *workspace,
+                                     size_t workspace_bytes, void *stream) {
+    return pgm_front_metrics_x_f64(pts, n, M, 0, out, workspace, workspace_bytes, stream);
 }

@@ -212,27 +212,34 @@ def ep_filter(objs):
     return idx[:k].cpu().numpy().astype(np.int64)
 
 
-def front_metrics(pts):
+SEL_GLOBAL = 0x1      # PGM_SEL_GLOBAL: the 3-objective global-memory path of K5 at any front size
+
+
+def front_metrics(pts, force_global=False):
     """(hypervolume, sparsity) of a point set: Population2d semantics for M=2 (get_ep_indices first, hypervolume not
     rounded); for M=3 and M=4 utils.compute_hypervolume (InnerHyperVolume, round(hv, 4)) and utils.compute_sparsity of
     the points as given. M=4 leaves points with a negative coordinate out of the hypervolume, as InnerHyperVolume does;
-    M=3 expects none. At most 2 202 points at M=4 (the 4-D scorer's shared memory); more raise."""
+    M=3 expects none. M=3 takes any size (past 3 936 points K5's global-memory path, with the same bits); at most
+    2 202 points at M=4 (the 4-D scorer's shared memory); more raise. force_global=True takes the global-memory path
+    at any size (M=3 only), so that tests can compare the two paths."""
     if len(pts) == 0:
         return 0.0, 0.0
     d = _dev_f64(pts)
     n, M = d.shape
+    flags = SEL_GLOBAL if force_global else 0
     out = torch.empty(2, dtype=torch.float64, device=d.device)
-    nb = lib().pgm_select_workspace_bytes(n, 1, M, 1)
+    nb = lib().pgm_select_workspace_bytes_x(n, 1, M, 1, flags)
     ws, (wp, wn) = _ws(nb, d.device)
-    check(lib().pgm_front_metrics_f64(ptr(d), n, M, ptr(out), wp, wn, _stream()))
+    check(lib().pgm_front_metrics_x_f64(ptr(d), n, M, flags, ptr(out), wp, wn, _stream()))
     h, s = out.cpu().tolist()
     return h, s
 
 
-def select_greedy(ep, cand, alpha, num_tasks):
+def select_greedy(ep, cand, alpha, num_tasks, force_global=False):
     """Greedy prediction-guided pick. ep [E,M] archive front, cand [C,M] predicted objectives.
     Returns (best_ids [num_tasks] (-1 = no candidate left), hv [num_tasks,C], sparsity [num_tasks,C],
-    final virtual front [n,M]) as numpy arrays."""
+    final virtual front [n,M]) as numpy arrays. M=3 takes any archive size (past E + num_tasks + 1 = 2 111 points
+    K5's global-memory path, with the same bits); force_global=True takes that path at any size (M=3 only)."""
     import numpy as np
     cand_d = _dev_f64(cand)
     C, M = cand_d.shape
@@ -245,11 +252,12 @@ def select_greedy(ep, cand, alpha, num_tasks):
     sp = torch.empty(num_tasks, max(C, 1), dtype=torch.float64, device=dev)
     front = torch.empty(E + num_tasks + 1, M, dtype=torch.float64, device=dev)
     nfront = torch.zeros(1, dtype=torch.int32, device=dev)
-    nb = lib().pgm_select_workspace_bytes(E, C, M, num_tasks)
+    flags = SEL_GLOBAL if force_global else 0
+    nb = lib().pgm_select_workspace_bytes_x(E, C, M, num_tasks, flags)
     ws, (wp, wn) = _ws(nb, dev)
     with _nvtx("selection.k5_greedy"):
-        check(lib().pgm_select_greedy_f64(ptr(ep_d), E, ptr(cand_d), C, M, float(alpha), num_tasks, ptr(best), ptr(hv),
-                                          ptr(sp), ptr(front), ptr(nfront), wp, wn, _stream()))
+        check(lib().pgm_select_greedy_x_f64(ptr(ep_d), E, ptr(cand_d), C, M, float(alpha), num_tasks, flags, ptr(best),
+                                            ptr(hv), ptr(sp), ptr(front), ptr(nfront), wp, wn, _stream()))
         nf = int(nfront.item())
     return (best.cpu().numpy().astype(np.int64), hv[:, :C].cpu().numpy(), sp[:, :C].cpu().numpy(),
             front[:nf].cpu().numpy())
