@@ -410,7 +410,12 @@ int pgm_select_greedy_x_f64(const double *ep, int E, const double *cand, int C, 
  *     ([N,O] rows, i.e. the slot of the rollout buffer K1 reads next); obj_out = clip(obj / sqrt(obj_var + epsilon), +-cliprew)
  *     at obj_out + p * obj_task_stride ([N,M]); mask_out [N] at mask_out + p * mask_task_stride = 1 - done.
  *   update = 0 freezes the observation moments (VecNormalize.eval()); reset = 1 is VecNormalize.reset(): only the
- *   observations are processed and ret_acc restarts at 0. N <= 128. */
+ *   observations are processed and ret_acc restarts at 0.
+ *   Preconditions: 1 <= N <= 128, O >= 1, M >= 0 (rc 1 otherwise, before any launch). Reductions follow numpy on
+ *   C-contiguous float64 blocks: rows one after the other, pairwise when the width is 1 (O == 1 or M == 1) and for the
+ *   return vector. Raw observations are float64, as MuJoCo delivers them; a simulator that returns float32 would have
+ *   the reference reduce in float32, which K6 does not reproduce. The clip is np.clip's: NaN stays NaN, so a NaN or
+ *   inf input makes that task's affected moments and outputs NaN instead of -clip. */
 int pgm_vecnorm_step_f64(const double *raw_obs, const double *raw_rew, const double *raw_obj, const uint8_t *done,
                          double *ob_mean, double *ob_var, double *ob_count, double *ret_acc, double *ret_stat,
                          double *obj_acc, int32_t *obj_started, double *obj_mean, double *obj_var, double *obj_count,

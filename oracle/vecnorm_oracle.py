@@ -46,6 +46,10 @@ def _sum_1d(a):
 def batch_moments(x):
     """(np.mean(x, axis=0), np.var(x, axis=0)) as RunningMeanStd.update computes them (running_mean_std.py:16-18)."""
     n = np.float64(x.shape[0])
+    if x.ndim == 2 and x.shape[1] == 1:
+        # numpy collapses a C-contiguous [N, 1] block into one contiguous 1-D reduction: pairwise, not row by row
+        mean, var = batch_moments(x[:, 0])
+        return np.array([mean]), np.array([var])
     if x.ndim == 1:
         mean = _sum_1d(x) / n
         d = x - mean

@@ -8,9 +8,11 @@
 //
 // FP64 in numpy's evaluation order with explicit round-to-nearest mul/add (no FMA contraction), so the running
 // moments and the float32 observations are bit-identical to the reference's:
-//   batch moments over the N envs (np.mean / np.var, axis 0): rows added one after the other; for the 1-D
-//   return vector numpy's reduction is the pairwise sum (a plain loop below 8 elements, 8 interleaved partial
-//   sums combined as ((r0+r1)+(r2+r3))+((r4+r5)+(r6+r7)) from 8 to 128).
+//   batch moments over the N envs (np.mean / np.var, axis 0) of an [N, W] block: rows added one after the other
+//   when W >= 2; when W == 1 (O == 1 observations, M == 1 objectives) numpy collapses the C-contiguous [N, 1]
+//   block into one contiguous 1-D reduction, which is the pairwise sum, as for the 1-D return vector (a plain loop
+//   below 8 elements, 8 interleaved partial sums combined as ((r0+r1)+(r2+r3))+((r4+r5)+(r6+r7)) from 8 to 128).
+//   Clipping is np.clip's: a NaN stays NaN (a NaN or inf from a simulator shows up in the outputs, never as -clip).
 // One CTA per task; threads stride over observation features, then over objectives; thread 0 owns the scalar
 // return statistics and the sample counts.
 #include "common.cuh"
@@ -48,12 +50,15 @@ __device__ __forceinline__ void rms_update(double &mean, double &var, double cou
     var = __ddiv_rn(m2, tot);
 }
 
-__device__ __forceinline__ double clipd(double x, double c) { return fmin(fmax(x, -c), c); }
+// np.clip(x, -c, c): comparisons, so a NaN passes through (fmin / fmax would return the bound) and -0.0 stays -0.0
+__device__ __forceinline__ double clipd(double x, double c) { return x < -c ? -c : (x > c ? c : x); }
 
-// numpy's pairwise sum of n <= 128 contiguous doubles (numpy/_core/src/umath/loops_utils.h.src)
+// np.add.reduce of n <= 128 doubles at(0..n-1), starting from its identity 0.0: one after the other when `rows` is set
+// (the rows of a C-contiguous [n, w >= 2] block), numpy's pairwise sum of a contiguous 1-D block otherwise
+// (numpy/_core/src/umath/loops_utils.h.src)
 template <typename F>
-__device__ __forceinline__ double np_pairwise(F at, int n) {
-    if (n < 8) {
+__device__ __forceinline__ double np_add_reduce(F at, int n, bool rows) {
+    if (rows || n < 8) {
         double res = 0.0;
         for (int i = 0; i < n; ++i) res = __dadd_rn(res, at(i));
         return res;
@@ -66,11 +71,18 @@ __device__ __forceinline__ double np_pairwise(F at, int n) {
     double res = __dadd_rn(__dadd_rn(__dadd_rn(r[0], r[1]), __dadd_rn(r[2], r[3])),
                            __dadd_rn(__dadd_rn(r[4], r[5]), __dadd_rn(r[6], r[7])));
     for (; i < n; ++i) res = __dadd_rn(res, at(i));
-    return res;
+    return __dadd_rn(0.0, res);
 }
-// np.add.reduce over a contiguous 1-D array is the pairwise sum of all of it
-template <typename F>
-__device__ __forceinline__ double np_sum1d(F at, int n) { return np_pairwise(at, n); }
+
+// (np.mean(x, axis=0)[j], np.var(x, axis=0)[j]) of a C-contiguous [n, w] block. numpy collapses a width-1 block into
+// one contiguous 1-D reduction (pairwise); wider blocks add their rows one after the other.
+__device__ __forceinline__ void np_col_moments(const double *x, int n, int w, int j, double &bmean, double &bvar) {
+    const double dn = (double)n;
+    const auto col = [&](int i) { return x[(size_t)i * w + j]; };
+    const double m = __ddiv_rn(np_add_reduce(col, n, w > 1), dn);
+    bmean = m;
+    bvar = __ddiv_rn(np_add_reduce([&](int i) { const double d = __dsub_rn(col(i), m); return __dmul_rn(d, d); }, n, w > 1), dn);
+}
 
 __global__ void __launch_bounds__(128) k6_vecnorm_kernel(K6Args a) {
     const int p = blockIdx.x, tid = threadIdx.x, N = a.N, O = a.O, M = a.M;
@@ -96,16 +108,9 @@ __global__ void __launch_bounds__(128) k6_vecnorm_kernel(K6Args a) {
             if (stats) {
                 mean = a.ob_mean[(size_t)p * O + j]; var = a.ob_var[(size_t)p * O + j];
                 if (a.update) {
-                    double s = x[j];
-                    for (int n = 1; n < N; ++n) s = __dadd_rn(s, x[(size_t)n * O + j]);
-                    const double bmean = __ddiv_rn(s, dN);
-                    double d0 = __dsub_rn(x[j], bmean);
-                    double v = __dmul_rn(d0, d0);
-                    for (int n = 1; n < N; ++n) {
-                        const double d = __dsub_rn(x[(size_t)n * O + j], bmean);
-                        v = __dadd_rn(v, __dmul_rn(d, d));
-                    }
-                    rms_update(mean, var, count, bmean, __ddiv_rn(v, dN), dN);
+                    double bmean, bvar;
+                    np_col_moments(x, N, O, j, bmean, bvar);
+                    rms_update(mean, var, count, bmean, bvar, dN);
                     a.ob_mean[(size_t)p * O + j] = mean; a.ob_var[(size_t)p * O + j] = var;
                 }
             }
@@ -138,16 +143,9 @@ __global__ void __launch_bounds__(128) k6_vecnorm_kernel(K6Args a) {
             double sd = 1.0;
             if (stats) {
                 double mean = a.obj_mean[(size_t)p * M + m], var = a.obj_var[(size_t)p * M + m];
-                double s = acc[m];
-                for (int n = 1; n < N; ++n) s = __dadd_rn(s, acc[(size_t)n * M + m]);
-                const double bmean = __ddiv_rn(s, dN);
-                double d0 = __dsub_rn(acc[m], bmean);
-                double v = __dmul_rn(d0, d0);
-                for (int n = 1; n < N; ++n) {
-                    const double d = __dsub_rn(acc[(size_t)n * M + m], bmean);
-                    v = __dadd_rn(v, __dmul_rn(d, d));
-                }
-                rms_update(mean, var, count, bmean, __ddiv_rn(v, dN), dN);
+                double bmean, bvar;
+                np_col_moments(acc, N, M, m, bmean, bvar);
+                rms_update(mean, var, count, bmean, bvar, dN);
                 a.obj_mean[(size_t)p * M + m] = mean; a.obj_var[(size_t)p * M + m] = var;
                 sd = sqrt(__dadd_rn(var, a.epsilon));
             }
@@ -172,8 +170,8 @@ __global__ void __launch_bounds__(128) k6_vecnorm_kernel(K6Args a) {
         for (int n = 0; n < N; ++n) ret[n] = __dadd_rn(__dmul_rn(ret[n], a.gamma), rw[n]);
         if (a.ret_stat) {
             double *st = a.ret_stat + (size_t)p * 3;
-            const double bmean = __ddiv_rn(np_sum1d([&](int i) { return ret[i]; }, N), dN);
-            const double bvar = __ddiv_rn(np_sum1d([&](int i) { const double d = __dsub_rn(ret[i], bmean); return __dmul_rn(d, d); }, N), dN);
+            const double bmean = __ddiv_rn(np_add_reduce([&](int i) { return ret[i]; }, N, false), dN);
+            const double bvar = __ddiv_rn(np_add_reduce([&](int i) { const double d = __dsub_rn(ret[i], bmean); return __dmul_rn(d, d); }, N, false), dN);
             double mean = st[0], var = st[1];
             rms_update(mean, var, st[2], bmean, bvar, dN);
             st[0] = mean; st[1] = var; st[2] = __dadd_rn(st[2], dN);

@@ -107,7 +107,9 @@ class DeviceVecNormalize:
             out['ret_rms'] = r
         if self.has_obj:
             r = RunningMeanStd()
-            if not self._obj_scalar[p]:
+            if self._obj_scalar[p]:                            # as loaded: shape () until the first update
+                r.mean, r.var = self.obj_mean[p, 0].cpu().numpy(), self.obj_var[p, 0].cpu().numpy()
+            else:
                 r.mean, r.var = self.obj_mean[p].cpu().numpy(), self.obj_var[p].cpu().numpy()
             r.count = float(self.obj_count[p])
             out['obj_rms'] = r

@@ -95,6 +95,39 @@ def test_minibatch_split_the_reference_would_run_differently_is_rejected(library
     assert rc == 1 and b"33 minibatches" in library.pgm_last_error()
 
 
+def _vecnorm_args(buf, **kw):
+    """Arguments of pgm_vecnorm_step_f64 for P = 2, N = 4, O = 3, M = 2, every pointer set (host memory: each case below
+    is refused before anything is launched, so nothing reads it); kw replaces single arguments by name."""
+    a = dict(raw_obs=buf, raw_rew=buf, raw_obj=buf, done=buf, ob_mean=buf, ob_var=buf, ob_count=buf, ret_acc=buf,
+             ret_stat=buf, obj_acc=buf, obj_started=buf, obj_mean=buf, obj_var=buf, obj_count=buf, obs_out=buf, obs_ts=12,
+             obj_out=buf, obj_ts=8, mask_out=buf, mask_ts=4, gamma=0.99, clipob=10.0, cliprew=10.0, epsilon=1e-8,
+             update=1, reset=0, P=2, N=4, O=3, M=2, stream=None)
+    a.update(kw)
+    return list(a.values())
+
+
+@pytest.mark.parametrize("kw,msg", [(dict(N=0), b"bad sizes"), (dict(N=129), b"N=129"), (dict(O=0), b"O=0"),
+                                    (dict(ob_count=None), b"ob_mean / ob_var / ob_count go together"),
+                                    (dict(obj_var=None), b"obj_mean / obj_var / obj_count go together"),
+                                    (dict(done=None), b"done flags are required")])
+def test_vecnorm_refusals_without_a_gpu(library, kw, msg):
+    """K6 refuses sizes outside 1 <= N <= 128, O >= 1, a running-moment triple with a missing member and a step without
+    done flags: rc 1 (argument error, not a CUDA error) and a message naming the problem."""
+    import ctypes
+    buf = ctypes.cast((ctypes.c_double * 64)(), ctypes.c_void_p)
+    assert library.pgm_vecnorm_step_f64(*_vecnorm_args(buf, **kw)) == 1
+    assert msg in library.pgm_last_error()
+
+
+def test_vecnorm_rollout_refuses_no_objectives(library):
+    """Rollout-slot mode writes reward vectors into the rollout buffer: M = 0 is refused (rc 1) before any launch."""
+    import ctypes
+    buf = ctypes.cast((ctypes.c_double * 64)(), ctypes.c_void_p)
+    rc = library.pgm_vecnorm_rollout_step_f64(buf, buf, buf, buf, buf, buf, buf, buf, buf, buf, buf, buf, buf, buf, buf, buf,
+                                              buf, 12, buf, 8, buf, 4, buf, 4, 0.99, 10.0, 10.0, 1e-8, 1, 2, 4, 3, 0, None)
+    assert rc == 1 and b"M=0" in library.pgm_last_error()
+
+
 def test_missing_library_fails_loudly(monkeypatch, tmp_path):
     from pgmorl_b200 import _lib
     monkeypatch.setattr(_lib, "_lib", None)
